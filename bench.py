@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # product arm (CUDA kernels)
     python bench.py --impl reference --gpus N --steps K --warmup W   # CPU reference arm
+    python bench.py ... --dump-outputs DIR     # also write the last timed step's outputs as DIR/*.npy (either arm)
 
 Workload at every N (weak scaling, one process per GPU): BASELINE.json configs[1] --
 "SLCL prototype path at 256x256 full-res 128-d embeddings, batch 32, 5 classes" (cfg2 of
@@ -44,6 +45,7 @@ CFG = dict(B=32, C=128, H=256, W=256, K=5, temperature=0.1, base_temperature=1.0
 WORKLOAD = ("cfg2: SLCL prototype path (mpcl_loss_calc+MPCL fwd+bwd, target variant with pixel_sel_loc), "
             "B32 C128 256x256 K5 fp32 NCHW per GPU")
 FALLBACK_HBM_GBS = 6650.0        # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+DUMP_SAMPLE = 1 << 21            # dL/dF elements --dump-outputs writes (8 MB of the 1.07 GB map, + 16 MB of positions)
 
 
 def base_config(world: int):
@@ -66,7 +68,13 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the per-kernel table of the other path kernels")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (rank 0; "
+                         "either arm, same names): loss.npy and a fixed, seeded sample of dL/dF (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def hbm_peak():
@@ -101,6 +109,23 @@ def make_inputs(n_images: int, seed: int, pin: bool):
     sel.copy_((torch.rand(n_images * h * w, generator=gen) > 0.5).float())
     centres = torch.randn(k, c, generator=gen)
     return feats, labels, sel, centres
+
+
+def dump_outputs(out_dir: str, dfeat: torch.Tensor, **arrays: torch.Tensor):
+    """--dump-outputs: what one step hands its caller, so that two builds -- or the two arms, whose inputs are the same
+    with the default --cpu-sample-images -- can be compared output for output on the same seeded inputs.  Each of
+    `arrays` goes to <name>.npy as fp32 (both arms write loss.npy; the product arm adds scal.npy, the forward's four
+    scalars: loss, coefficient, weight sum, weighted row-loss sum); dfeat_sample.npy: dL/dF at DUMP_SAMPLE flat NCHW
+    positions drawn with a fixed seed, which dfeat_sample_index.npy lists (float64, exact below 2**53)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    flat = dfeat.detach().reshape(-1)
+    idx = torch.randint(0, flat.numel(), (min(DUMP_SAMPLE, flat.numel()),),
+                        generator=torch.Generator().manual_seed(CFG["seed"])).sort().values
+    for name, value in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), value.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "dfeat_sample.npy"), flat[idx.to(flat.device)].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "dfeat_sample_index.npy"), idx.double().numpy())
 
 
 # ----------------------------------------------------------------------------
@@ -189,7 +214,7 @@ def cpu_step_fn(n_images: int):
         feats.grad = None
         loss = O.mpcl_loss_calc(feats, labels, centres, spec, pixel_sel_loc=sel, tag="target")
         loss.backward()
-        return float(loss.detach())
+        return loss.detach(), feats.grad
     return step, n_images * CFG["H"] * CFG["W"]
 
 
@@ -202,9 +227,9 @@ def time_cpu(n_images: int, warmup: int, steps: int):
     times = []
     for _ in range(steps):
         t0 = time.perf_counter()
-        step()
+        out = step()
         times.append(time.perf_counter() - t0)
-    return pixels, times, cores
+    return pixels, times, cores, out           # out: (loss, dL/dF) of the last timed step
 
 
 def time_torch_eager_gpu(dev, feats, labels, sel, centres, iters: int = 5):
@@ -242,7 +267,9 @@ def run_reference(args):
     if rank != 0:
         return
     n_img = args.cpu_sample_images
-    pixels, times, cores = time_cpu(n_img, max(args.warmup, 1), args.steps)
+    pixels, times, cores, (loss, dfeat) = time_cpu(n_img, max(args.warmup, 1), args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dfeat, loss=loss.reshape(1))
     total = sum(times)
     value = pixels * len(times) / total
     sample = (("the full cfg2 batch per step" if n_img == CFG["B"] else f"{n_img} of the 32 images of the cfg2 batch per step")
@@ -253,8 +280,8 @@ def run_reference(args):
         "warmup": args.warmup, "ms_per_step": 1e3 * total / len(times), "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": base_config(args.gpus),
-        "note": "CPU arm: the reference's op sequence (oracle port; /root/reference is pure Python and not on the GPU box) on "
-                "the box's host cores, rank 0 only",
+        "note": "CPU arm: the reference's op sequence (oracle port: the original project is a script collection, not an "
+                "installable package) on the box's host cores, rank 0 only",
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
@@ -402,6 +429,8 @@ def run_slcl(args):
         elapsed_ms = float(t.item())
     ms_per_step = elapsed_ms / args.steps
     value = world * n_px * args.steps / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dfeat, loss=scal[:1], scal=scal)   # the last timed step's, before e2e frees the plan
     fwd_ms = statistics.mean(m[0].elapsed_time(m[1]) for m in marks)
     xch_ms = statistics.mean(m[1].elapsed_time(m[2]) for m in marks)
     bwd_ms = statistics.mean(m[2].elapsed_time(m[3]) for m in marks)
@@ -581,7 +610,7 @@ def run_slcl(args):
         except Exception as exc:  # noqa: BLE001 - a comparator must never take the bench line down
             out["torch_eager_gpu"] = {"unavailable": repr(exc)[:200]}
         n_img = args.cpu_sample_images
-        pixels, times, cores = time_cpu(n_img, 1, 3)
+        pixels, times, cores, _ = time_cpu(n_img, 1, 3)
         out["cpu_baseline"] = {
             "value": pixels / min(times), "unit": UNIT, "cores": cores, "kind": "port",
             "sample": f"{n_img} of the 32 cfg2 images per step ({pixels} px), oracle port of the reference call sequence, "

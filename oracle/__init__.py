@@ -11,12 +11,13 @@ Pinning status (see DESIGN.md "Oracle"):
   * prototype path, EMA class centres, pseudo labels, hard centroids,
     ContrastiveLoss, SupCon/LocalCon/BlockCon: PINNED -- the restatement in
     ``slcl_oracle.py`` is checked against outputs of the reference's own
-    functions (``tests/golden/*.npz``, produced by ``oracle/make_golden.py``
-    which imports ``/root/reference`` in the build container) and against
-    the nine known-answer values of SURVEY.md section 8(c); where the
-    reference tree is mounted, ``tests/test_oracle_live_reference.py`` also runs
-    the reference's callables and the restatement side by side on randomised
-    inputs (losses and gradients, 30 cases; seg losses and ISCL included).
+    functions (``tests/golden/reference_*outputs.npz``, made by ``oracle/make_golden.py``
+    which imports a checkout of the original project, see ``ref_loader.py``) and against
+    the nine known-answer values of SURVEY.md section 8(c);
+    ``tests/test_oracle_live_reference.py`` checks it on randomised inputs
+    (losses and gradients, 33 cases; seg losses and ISCL included) against the
+    stored ``tests/golden/reference_live_cases.npz`` and, where a checkout of
+    the original is present, against the reference's callables run live.
   * soft-label centroid path: pinned against the reference function with the
     one-line repair described in SURVEY.md section 0 (the shipped function
     raises NameError).

@@ -1,12 +1,13 @@
-"""Generate tests/golden/*.npz by running the REAL reference functions
-(TEST INFRASTRUCTURE; run in the build container where /root/reference exists):
+"""Generate tests/golden/reference_outputs.npz and reference_seg_outputs.npz by running the REAL reference functions
+(TEST INFRASTRUCTURE; needs a checkout of the original project, see oracle/ref_loader.py):
 
     python -m oracle.make_golden
 
 Each fixture stores the outputs (loss, gradients, labels, centres) of the
 reference's own code on the seeded inputs of oracle/cases.py.  The committed
 fixtures are what the oracle restatement and the CUDA path are compared with
-on the GPU box, where the reference tree does not exist.
+wherever the original project is absent.  (tests/golden/reference_live_cases.npz
+is recorded by tests/test_oracle_live_reference.py itself; see its docstring.)
 """
 from __future__ import annotations
 

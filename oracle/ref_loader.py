@@ -1,10 +1,11 @@
-"""Import the *real* reference loss functions (TEST INFRASTRUCTURE, build
-container only).
+"""Import the *real* reference loss functions (TEST INFRASTRUCTURE).
 
-``/root/reference`` exists only in the build container, never on the GPU box,
-so this loader is used by ``oracle/make_golden.py`` (to produce the committed
-fixtures under ``tests/golden/``) and by CPU tests that are skipped when the
-reference tree is absent.  Recipe: SURVEY.md appendix B -- stub the four
+The reference is a checkout of the original Soft-Labeled-Contrastive-Learning
+project at ``oracle/_ref`` (git-ignored: it is not part of this repository) or
+wherever ``SLCL_REFERENCE_ROOT`` points.  This loader is used by
+``oracle/make_golden.py`` (to produce the committed fixtures under
+``tests/golden/``) and by CPU tests that are skipped when the reference tree is
+absent.  Recipe: SURVEY.md appendix B -- stub the four
 missing third-party modules that ``utils/utils_.py`` imports but the hot path
 never uses, and keep tensors on the host by making ``Tensor.cuda`` the
 identity while the reference functions run.
@@ -19,7 +20,7 @@ import types
 
 import torch
 
-REFERENCE_ROOT = os.environ.get("SLCL_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("SLCL_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available() -> bool:
