@@ -431,6 +431,39 @@ int slcl_p2p_bwd(const void* a_bf16, const void* b_bf16, int64_t n_anchor, int64
                  float temperature, const float* stats, const void* bwd_state, const float* grad_out, float* d_a, float* d_b,
                  void* workspace, size_t workspace_bytes, slcl_stream_t stream);
 
+/* ---------------------------------------------------------------------------
+ * Pixel <-> pixel losses over the GLOBAL batch of data-parallel ranks (SURVEY.md 8(e); the `group=` argument of
+ * SupConLoss / LocalConLoss / sampled_supcon_loss).  Each rank sweeps its own anchors against the contrast rows of all
+ * ranks (slcl_p2p_fwd, d_a of slcl_p2p_bwd), and the anchors of all ranks against its own contrast rows (d_b of
+ * slcl_p2p_bwd), so per-rank tensor work is 8 A_local M_global d flop and nothing is computed twice.
+ *
+ * slcl_peer_allgather: every rank contributes a record of n_bytes (multiple of 16, <= slot_bytes) and receives all ranks'
+ * records in rank order in out [world * n_bytes] -- a private buffer no later call touches.  Replaces the NCCL
+ * all_gather_into_tensor of the same records.  regions_dev: device array of `world` pointers to the ranks' row regions of
+ * slcl_peer_rows_region_bytes(slot_bytes) bytes each (zero-initialised, mapped by every rank like the mailboxes); the call
+ * is one exchange of the mailbox sequence of `peer` (same epochs, same time-out).  The first 16 bytes of a record are its
+ * key (sizes / shapes) and must be equal on every rank.  status [1] int32, in/out: bit 0 = a peer timed out (mailbox word 1
+ * counts it), bit 1 = a peer's key differs (mailbox word 5 counts it).  With a non-zero status on entry (an earlier
+ * exchange of the same result failed) or after a time-out waiting for a free slot, the call publishes nothing and waits
+ * for nobody, so the peers time out too and every rank's result is NaN; it still reads the peers' slots and acks them.
+ * Out is then undefined but never read past a slot.  The calls may interleave with the other exchanges of the mailbox in
+ * any order.
+ * ------------------------------------------------------------------------- */
+size_t slcl_peer_rows_region_bytes(int64_t slot_bytes);
+int slcl_peer_allgather(const void* record, int64_t n_bytes, void* out, int32_t* status, const slcl_peer_t* peer,
+                        const void* regions_dev, int64_t slot_bytes, slcl_stream_t stream);
+/* Byte offsets inside the analytic backward state of slcl_p2p_state_bytes(n_anchor, dim_padded):
+ * offsets_host[7] = {U partials, Bsum, ABsum [K][d+1] fp32, colshift [pad64(A)] fp32, alpha~ [A] fp32, beta~ [A] fp32, total}.
+ * Lets a data-parallel caller read a rank's per-anchor constants and ABsum table out of its forward state. */
+int slcl_p2p_state_layout(int64_t n_anchor, int64_t dim_padded, int64_t* offsets_host);
+/* Backward state for slcl_p2p_bwd(d_b only) over the anchors of all ranks, built from what each rank's forward left:
+ * alpha / beta / colshift [n_anchor] fp32 = the ranks' per-anchor constants concatenated in rank order, absum_parts
+ * [n_parts][n_class][dim_padded + 1] fp32 = the ranks' ABsum tables (summed in rank order).  Replaces the state a forward
+ * over all anchors would have left (U, Bsum: not read by the d_b backward, left unset). */
+int slcl_p2p_state_assemble(void* bwd_state, int64_t n_anchor, int64_t dim_padded, int n_class, const float* alpha,
+                            const float* beta, const float* colshift, const float* absum_parts, int n_parts,
+                            slcl_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

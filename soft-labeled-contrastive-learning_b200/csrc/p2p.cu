@@ -1769,6 +1769,53 @@ extern "C" size_t slcl_p2p_state_bytes(int64_t n_anchor, int64_t dim_padded) {
   return carve_state(nullptr, n_anchor, (int)dim_padded).total;
 }
 
+extern "C" int slcl_p2p_state_layout(int64_t n_anchor, int64_t dim_padded, int64_t* offsets_host) {
+  if (n_anchor <= 0 || dim_padded <= 0 || dim_padded > kMaxD || dim_padded % KCH || !offsets_host) return SLCL_ERR_INVALID_ARGUMENT;
+  const P2PState s = carve_state(nullptr, n_anchor, (int)dim_padded);
+  const float* f[6] = {s.u, s.bsum, s.absum, s.colshift, s.alpha, s.beta};
+  for (int i = 0; i < 6; ++i) offsets_host[i] = (int64_t)reinterpret_cast<uintptr_t>(f[i]);
+  offsets_host[6] = (int64_t)s.total;
+  return SLCL_OK;
+}
+
+namespace slcl {
+namespace {
+// Backward state of the dB sweep over the anchors of all ranks: per-anchor constants concatenated (colshift padded with the
+// switch-off shift), ABsum = sum of the ranks' tables in rank order (identical bits on every rank).
+__global__ void __launch_bounds__(256) p2p_state_assemble_kernel(int n_anchor, int n_padded, int n_tab, const float* alpha,
+                                                                 const float* beta, const float* colshift, const float* absum_parts,
+                                                                 int n_parts, float* st_alpha, float* st_beta,
+                                                                 float* st_colshift, float* st_absum) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_padded || i < n_tab; i += gridDim.x * blockDim.x) {
+    if (i < n_anchor) { st_alpha[i] = alpha[i]; st_beta[i] = beta[i]; }
+    if (i < n_padded) st_colshift[i] = i < n_anchor ? colshift[i] : kShiftOff;
+    if (i < n_tab) {
+      float t = 0.f;
+      for (int p = 0; p < n_parts; ++p) t += absum_parts[(size_t)p * n_tab + i];
+      st_absum[i] = t;
+    }
+  }
+}
+}  // namespace
+}  // namespace slcl
+
+extern "C" int slcl_p2p_state_assemble(void* bwd_state, int64_t n_anchor, int64_t dim_padded, int n_class, const float* alpha,
+                                       const float* beta, const float* colshift, const float* absum_parts, int n_parts,
+                                       slcl_stream_t stream_) {
+  if (!bwd_state || !aligned16(bwd_state) || !alpha || !beta || !colshift || !absum_parts || n_anchor <= 0 ||
+      n_anchor >= (int64_t)kMaxFinishBlocks * 256 || dim_padded <= 0 || dim_padded > kMaxD || dim_padded % KCH || n_class < 1 ||
+      n_class > kMaxLabelClasses || n_parts < 1)
+    return SLCL_ERR_INVALID_ARGUMENT;
+  const int d = (int)dim_padded;
+  P2PState s = carve_state(bwd_state, n_anchor, d);
+  const int n_padded = (int)align_up((size_t)n_anchor, BN), n_tab = n_class * (d + 1);
+  const int n = n_padded > n_tab ? n_padded : n_tab;
+  p2p_state_assemble_kernel<<<ceil_div(n, 256), 256, 0, (cudaStream_t)stream_>>>((int)n_anchor, n_padded, n_tab, alpha, beta,
+                                                                                   colshift, absum_parts, n_parts, s.alpha,
+                                                                                   s.beta, s.colshift, s.absum);
+  return check_launch("slcl_p2p_state_assemble");
+}
+
 extern "C" int slcl_p2p_fwd(const void* a_bf16, const void* b_bf16, int64_t n_anchor, int64_t n_contrast, int64_t dim_padded,
                             const int32_t* a_meta, const int32_t* b_meta, const int32_t* a_selfcol, int n_class, int n_batch,
                             const float* shift, const float* weight, float temperature, float* stats, float* loss,

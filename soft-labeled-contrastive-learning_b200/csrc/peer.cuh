@@ -9,7 +9,8 @@
 //   word 2  ticket   : block counter of a multi-block exchange kernel (self-resetting)
 //   word 3  ready    : split-phase exchanges: the epoch whose result this rank has published to its own blocks
 //   word 4  pending  : split-phase exchanges: the epoch a sender kernel has put on the wire and a later kernel completes
-//   word 5..7        : reserved
+//   word 5   mismatch: number of bulk all-gathers (peer_rows.cu) whose records disagreed in size between ranks
+//   word 6..7        : reserved
 //   word 8 + (q * world + r) * capacity + s : payload word s of sender r for epoch parity q
 // A payload word is {epoch : 32 | data : 32}: an aligned 8-byte store is single-copy atomic, so flag and data arrive
 // together and no fence is needed (the protocol NCCL calls LL).  A call with epoch e writes its words into every

@@ -109,6 +109,10 @@ SIGNATURES = {
                                _P]),
     "slcl_p2p_bwd": (C.c_int, [_P, _P, _I64, _I64, _I64, _I64, _P, _P, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, _P, _P, _P,
                                _P, _P, _P, _SZ, _P]),
+    "slcl_peer_rows_region_bytes": (_SZ, [_I64]),
+    "slcl_peer_allgather": (C.c_int, [_P, _I64, _P, _P, C.POINTER(PeerT), _P, _I64, _P]),
+    "slcl_p2p_state_layout": (C.c_int, [_I64, _I64, _P]),
+    "slcl_p2p_state_assemble": (C.c_int, [_P, _I64, _I64, C.c_int, _P, _P, _P, _P, C.c_int, _P]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -254,6 +254,37 @@ def peer_allreduce_f64(buf: Tensor, peer_ptrs: int, rank: int, world: int, capac
     check(st, "slcl_peer_allreduce_f64")
 
 
+@torch.library.custom_op("slcl::peer_allgather", mutates_args=("status",), device_types="cuda")
+def peer_allgather(record: Tensor, status: Tensor, peer_ptrs: int, rank: int, world: int, capacity_words: int, timeout_s: float,
+                   regions_ptr: int, slot_bytes: int) -> Tensor:
+    """All ranks' uint8 records [n] (n % 16 == 0, equal first 16 bytes) -> [world, n] in rank order, over NVLink peer memory
+    (slcl.peer.PeerMailbox built with rows_bytes).  ``status`` int32 [1], in/out: non-zero = a peer timed out (bit 0) or sent
+    a record of another size (bit 1); the caller turns it into NaN."""
+    dev = require_cuda(record, status)
+    rec = record.contiguous()
+    n = rec.numel()
+    if rec.dtype != torch.uint8 or n % 16 or n < 16:
+        raise ValueError("record must be uint8 with a multiple of 16 bytes")
+    if status.dtype != torch.int32 or status.numel() != 1:
+        raise ValueError("status must be int32 [1]")
+    if not regions_ptr or slot_bytes <= 0:
+        raise ValueError("this mailbox has no row region: build it with rows_bytes > 0")
+    if n > slot_bytes:
+        raise ValueError(f"record of {n} bytes exceeds the mailbox's row slot of {slot_bytes} bytes (rows_bytes)")
+    out = torch.empty((world, n), dtype=torch.uint8, device=dev)
+    peer = PeerT(peer_ptrs, rank, world, capacity_words, timeout_s)
+    with _guard(dev):
+        st = _lib.load().slcl_peer_allgather(ptr(rec), n, ptr(out), ptr(status), C.byref(peer), regions_ptr, slot_bytes,
+                                             stream_ptr(dev))
+    check(st, "slcl_peer_allgather")
+    return out
+
+
+@peer_allgather.register_fake
+def _(record, status, peer_ptrs, rank, world, capacity_words, timeout_s, regions_ptr, slot_bytes):
+    return record.new_empty((world, record.numel()))
+
+
 @torch.library.custom_op("slcl::proto_bwd", mutates_args=(), device_types="cuda")
 def proto_bwd(feat: Tensor, stash: Tensor, cstate: Tensor, scal: Tensor, grad_out: Tensor, rows_layout: bool,
               n_class: int, normalize: bool) -> Tensor:
@@ -992,6 +1023,43 @@ def p2p_bwd(a: Tensor, b: Tensor, dim: int, a_meta: Tensor, b_meta: Tensor, shif
 def _(a, b, dim, a_meta, b_meta, shift, weight, temperature, stats, grad_out, need_a, need_b, n_class=0, a_selfcol=None,
       b_selfrow=None, state=None, n_batch=1):
     return (shift.new_empty((a.shape[0] if need_a else 0, dim)), shift.new_empty((b.shape[0] if need_b else 0, dim)))
+
+
+P2P_STATE_FIELDS = ("u", "bsum", "absum", "colshift", "alpha", "beta")
+
+
+def p2p_state_layout(n_anchor: int, dim_padded: int) -> dict:
+    """Byte offsets of the fields of the analytic backward state (slcl_p2p_state_layout) plus its ``total`` size."""
+    off = (C.c_int64 * 7)()
+    check(_lib.load().slcl_p2p_state_layout(int(n_anchor), int(dim_padded), off), "slcl_p2p_state_layout")
+    return dict(zip(P2P_STATE_FIELDS + ("total",), list(off)))
+
+
+@torch.library.custom_op("slcl::p2p_state_assemble", mutates_args=(), device_types="cuda")
+def p2p_state_assemble(alpha: Tensor, beta: Tensor, colshift: Tensor, absum_parts: Tensor, dim_padded: int,
+                       n_class: int) -> Tensor:
+    """Backward state for p2p_bwd(need_b only) over the anchors of all ranks (slcl_p2p_state_assemble): per-anchor constants
+    [A] concatenated in rank order, ABsum tables [parts, n_class * (dim_padded + 1)] summed in rank order."""
+    dev = require_cuda(alpha, beta, colshift, absum_parts)
+    lib = _lib.load()
+    na = alpha.numel()
+    for t in (alpha, beta, colshift, absum_parts):
+        if t.dtype != _F32 or not t.is_contiguous():
+            raise ValueError("state pieces must be contiguous float32")
+    if beta.numel() != na or colshift.numel() != na or absum_parts.dim() != 2 or \
+            absum_parts.shape[1] != n_class * (dim_padded + 1):
+        raise ValueError("alpha / beta / colshift [A] and absum_parts [parts, n_class * (dim_padded + 1)]")
+    state = torch.empty(lib.slcl_p2p_state_bytes(na, dim_padded), dtype=torch.uint8, device=dev)
+    with _guard(dev):
+        st = lib.slcl_p2p_state_assemble(ptr(state), na, dim_padded, n_class, ptr(alpha), ptr(beta), ptr(colshift),
+                                         ptr(absum_parts), absum_parts.shape[0], stream_ptr(dev))
+    check(st, "slcl_p2p_state_assemble")
+    return state
+
+
+@p2p_state_assemble.register_fake
+def _(alpha, beta, colshift, absum_parts, dim_padded, n_class):
+    return torch.empty(_lib.load().slcl_p2p_state_bytes(alpha.numel(), dim_padded), dtype=torch.uint8, device=alpha.device)
 
 
 # ----------------------------------------------------------------------------

@@ -35,14 +35,18 @@ class _AutoClasses:
         self.fixed = n_class            # None = auto
         self.auto = None                # decided at the first labelled call
 
-    def resolve(self, labels):
-        """-> (n_class for the sweeps, device flag `labels in range` or None -- None since the kernels' own NaN covers it)"""
+    def resolve(self, labels, exchange=None):
+        """-> (n_class for the sweeps, device flag `labels in range` or None -- None since the kernels' own NaN covers it).
+        With an ``exchange`` (``group=``) the range is reduced over the ranks, so every rank takes the same sweeps."""
         if self.fixed is not None:
             return int(self.fixed), None
         if labels is None:
             return 0, None
         if self.auto is None:
-            lo, hi = int(labels.min()), int(labels.max())        # once per module
+            if exchange is None:
+                lo, hi = int(labels.min()), int(labels.max())        # once per module
+            else:
+                lo, hi = exchange.label_range(labels)
             self.auto = AUTO_N_CLASS if (lo >= 0 and hi < AUTO_N_CLASS) else 0
         if self.auto == 0:
             return 0, None
@@ -103,6 +107,221 @@ class _P2PLoss(torch.autograd.Function):
             _ops.scatter_rows_bwd(fm, idx_a, normalize, d_a, inv_a, dfeat)
             _ops.scatter_rows_bwd(fm, idx_b, normalize, d_b, inv_b, dfeat)
         return (dfeat,) + (None,) * 13
+
+
+_INT_MIN = -2 ** 31
+
+
+class _Exchange:
+    """The ``group=`` argument of the pixel <-> pixel losses: all-gather of byte records over NVLink peer memory
+    (``slcl.peer.PeerMailbox`` built with ``rows_bytes``; ``slcl_peer_allgather``) or NCCL (``True`` / a ProcessGroup)."""
+
+    def __init__(self, group):
+        from .peer import PeerMailbox
+        if isinstance(group, PeerMailbox):
+            self.box, self.pg = group, None
+            self.world, self.rank = group.world, group.rank
+        else:
+            import torch.distributed as dist
+            self.box, self.pg = None, (None if group is True else group)
+            self.world, self.rank = dist.get_world_size(self.pg), dist.get_rank(self.pg)
+
+    def allgather(self, record, status):
+        """uint8 record [n] -> [world, n] in rank order.  ``status`` (int32 [1]) turns non-zero when a peer timed out or
+        sent a record whose 16-byte key differs (peer route: the caller's result is then NaN)."""
+        if self.box is not None:
+            return _ops.peer_allgather(record, status, *self.box.args(), *self.box.rows_args())
+        import torch.distributed as dist
+        # NCCL cannot gather records of different sizes: compare the keys first and refuse on the host
+        keys = torch.empty((self.world, 16), dtype=torch.uint8, device=record.device)
+        dist.all_gather_into_tensor(keys, record[:16].contiguous(), group=self.pg)
+        if not bool((keys == record[:16]).all()):
+            raise ValueError("group= pixel<->pixel loss: the ranks passed row sets of different sizes")
+        out = torch.empty((self.world, record.numel()), dtype=torch.uint8, device=record.device)
+        dist.all_gather_into_tensor(out, record, group=self.pg)
+        return out
+
+    def label_range(self, labels):
+        """(min, max) of the labels over all ranks: one exchange and one host synchronisation."""
+        lohi = torch.stack([labels.min(), -labels.max()]).long()
+        rec, _ = _pack([_key(labels.device, 0, 0, 0, 3), lohi])
+        status = torch.zeros(1, dtype=torch.int32, device=labels.device)
+        got = self.allgather(rec, status)[:, 16:32].contiguous().view(torch.int64)
+        if int(status[0]) != 0:
+            raise RuntimeError("group= pixel<->pixel loss: the label-range exchange failed (peer timed out or shapes differ)")
+        lo, nhi = got.amin(0).tolist()
+        return lo, -nhi
+
+
+def _exchange(group):
+    """None (today's single-rank path) for no group or a world of one."""
+    if group is None:
+        return None
+    x = _Exchange(group)
+    return x if x.world > 1 else None
+
+
+def _key(dev, a, m, dp, flags):
+    """16-byte record key (int32 {A, M, dp, flags}): equal on every rank iff the records have the same layout."""
+    def build():          # filled on the device: a host copy would synchronise the stream in the middle of the exchanges
+        k = torch.zeros(4, dtype=torch.int32, device=dev)
+        for i, v in enumerate((a, m, dp, flags)):
+            k[i] = v
+        return k
+    return _cached(("key", a, m, dp, flags, str(dev)), build)
+
+
+def _pack(parts):
+    """tensors -> (uint8 record, layout); every part starts on a 16-byte boundary."""
+    chunks, layout, off = [], [], 0
+    for t in parts:
+        b = t.contiguous().view(-1).view(torch.uint8)
+        n = b.numel()
+        chunks.append(b)
+        if n % 16:
+            chunks.append(b.new_zeros(16 - n % 16))
+        layout.append((off, n, t.dtype, tuple(t.shape)))
+        off += n + (-n) % 16
+    return torch.cat(chunks), layout
+
+
+def _unpack(gathered, layout, i):
+    """Part i of every rank's record, concatenated in rank order along the first dimension (a private copy)."""
+    off, n, dtype, shape = layout[i]
+    return gathered[:, off:off + n].contiguous().view(dtype).reshape((-1,) + shape[1:])
+
+
+def _pad_meta_rows(meta):
+    out = torch.full(((meta.shape[0] + 63) // 64 * 64, 2), _INT_MIN, dtype=torch.int32, device=meta.device)
+    out[:meta.shape[0]] = meta
+    return out
+
+
+def global_record_bytes(n_anchor: int, n_contrast: int, channels: int, same_rows: bool = False) -> int:
+    """Send-slot size (``rows_bytes`` of ``PeerMailbox`` / ``LoopbackMailboxes``) that a ``group=`` pixel <-> pixel loss with
+    this many anchors / contrast rows per rank and ``channels`` feature channels needs."""
+    p16 = lambda n: (n + 15) // 16 * 16
+    dp = (channels + 63) // 64 * 64
+    rows = lambda r: r * dp * 2 + p16(r * 8) + p16(r * 4)
+    first = 16 + 16 + rows(n_contrast) + (0 if same_rows else rows(n_anchor))
+    second = 16 + 16 + max(3 * p16(n_anchor * 4) + p16(AUTO_N_CLASS * (dp + 1) * 4), p16(n_anchor * 12))
+    return max(first, second)
+
+
+class _P2PGlobal(torch.autograd.Function):
+    """loss(feat) of the pixel <-> pixel problem over the GLOBAL batch of ``x.world`` ranks (INTEGRATION.md section 4).
+
+    Anchors and contrast rows are the union of every rank's rows in rank order; ``meta_*`` carry ids that are unique across
+    ranks.  Forward: all-gather {rows, meta, norms, short flag} -> weights / shifts of the global problem -> this rank's
+    anchors x all contrast rows (slcl_p2p_fwd) -> all-gather {loss partial, per-anchor backward constants}.  Backward, no
+    exchange: d_a = this rank's anchors x all contrast rows, d_b = all anchors x this rank's contrast rows (slcl_p2p_bwd with
+    a state assembled from the gathered constants), so this rank gets exactly its shard of the global gradient."""
+
+    @staticmethod
+    def forward(ctx, feat, idx_a, idx_b, meta_a, meta_b, short, temperature, normalize, same_rows, n_class, selfcol, selfrow,
+                uniform_weight, zero_if_empty, x, rowmaps):
+        fm = feat.detach().contiguous()
+        c = fm.shape[1]
+        dev = fm.device
+        W, r = x.world, x.rank
+        b_l, _, inv_b = _ops.gather_unit_rows(fm, idx_b, normalize, True, False)
+        if same_rows:
+            a_l, inv_a = b_l, inv_b
+        else:
+            a_l, _, inv_a = _ops.gather_unit_rows(fm, idx_a, normalize, True, False)
+        na, m, dp = a_l.shape[0], b_l.shape[0], b_l.shape[1]
+        flags = int(same_rows) | int(normalize) << 1 | n_class << 2
+        parts = [_key(dev, na, m, dp, flags), short.reshape(1).to(torch.int32), b_l, meta_b[:m], inv_b]
+        if not same_rows:
+            parts += [a_l, meta_a[:na], inv_a]
+        rec, lay = _pack(parts)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        g1 = x.allgather(rec, status)
+        b_g, meta_b_g, inv_b_g = _unpack(g1, lay, 2), _pad_meta_rows(_unpack(g1, lay, 3)), _unpack(g1, lay, 4)
+        if same_rows:
+            a_g, meta_a_g, inv_a_g = b_g, meta_b_g, inv_b_g
+        else:
+            a_g, meta_a_g, inv_a_g = _unpack(g1, lay, 5), _pad_meta_rows(_unpack(g1, lay, 6)), _unpack(g1, lay, 7)
+        short_any = (_unpack(g1, lay, 1) != 0).any()
+        na_g, m_g = na * W, m * W
+        if uniform_weight:
+            w_g = torch.full((na_g,), 1.0 / na_g, device=dev)
+        else:         # fg_i / sum fg over the anchors of all ranks
+            w_g, _ = _ops.tile_weights(meta_a_g, na_g, 1, bool(zero_if_empty))
+        mine = slice(na * r, na * (r + 1))
+        w_l = w_g[mine]
+        if normalize:
+            shift_g = torch.full((na_g,), 1.0 / temperature, device=dev)
+        else:         # |a_i| max_j |b_j| / T over the contrast rows of all ranks
+            shift_g = _ops.p2p_shift(inv_a_g, inv_b_g, temperature)
+        shift_l = shift_g[mine]
+        analytic = n_class > 0
+        selfcol_f = selfrow_g = a_selfcol_g = b_selfrow_l = None
+        if selfcol is not None:        # the local self maps, offset into the global row index spaces
+            selfcol_f = torch.where(selfcol >= 0, selfcol + m * r, selfcol).to(torch.int32)
+            selfrow_g = torch.full((m_g,), -1, dtype=torch.int32, device=dev)
+            selfrow_g[m * r:m * (r + 1)] = selfrow
+            a_selfcol_g = torch.full((na_g,), -1, dtype=torch.int32, device=dev)
+            a_selfcol_g[mine] = selfcol
+            b_selfrow_l = torch.where(selfrow >= 0, selfrow + na * r, selfrow).to(torch.int32)
+        loss_l, stats_l, state_l = _ops.p2p_fwd(a_l, b_g, meta_a, meta_b_g, shift_l, w_l, temperature, n_class, selfcol_f,
+                                                analytic, 1)
+        parts2 = [_key(dev, na, m, dp, flags), loss_l]
+        if analytic:
+            off = ops.p2p_state_layout(na, dp)
+            f32 = lambda name, n: state_l[off[name]:off[name] + 4 * n].view(torch.float32)
+            parts2 += [f32("alpha", na), f32("beta", na), f32("colshift", na), f32("absum", n_class * (dp + 1))]
+        else:
+            parts2 += [stats_l]
+        rec2, lay2 = _pack(parts2)
+        g2 = x.allgather(rec2, status)
+        partials = _unpack(g2, lay2, 1)
+        loss = partials[0]
+        for q in range(1, W):          # rank order: identical bits on every rank
+            loss = loss + partials[q]
+        loss = torch.where((status[0] != 0) | short_any, torch.full_like(loss, float("nan")), loss)
+        if analytic:
+            state_g = _ops.p2p_state_assemble(_unpack(g2, lay2, 2), _unpack(g2, lay2, 3), _unpack(g2, lay2, 4),
+                                              _unpack(g2, lay2, 5).reshape(W, -1), dp, n_class)
+            stats_g = stats_l          # (not read by the analytic backward with a state)
+        else:
+            state_g, stats_g = None, _unpack(g2, lay2, 2).reshape(na_g, 3)
+        ctx.save_for_backward(fm, idx_a, idx_b, a_l, b_l, a_g, b_g, meta_a, meta_b, meta_a_g, meta_b_g, inv_a, inv_b, shift_l,
+                              shift_g, w_l, w_g, stats_l, stats_g, state_l, state_g, selfcol_f, selfrow_g, a_selfcol_g,
+                              b_selfrow_l, rowmaps)
+        ctx.cfg = (temperature, normalize, same_rows, c, n_class)
+        return loss
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (fm, idx_a, idx_b, a_l, b_l, a_g, b_g, meta_a, meta_b, meta_a_g, meta_b_g, inv_a, inv_b, shift_l, shift_g, w_l, w_g,
+         stats_l, stats_g, state_l, state_g, selfcol_f, selfrow_g, a_selfcol_g, b_selfrow_l, rowmaps) = ctx.saved_tensors
+        temperature, normalize, same_rows, c, n_class = ctx.cfg
+        none = (None,) * 15
+        if not ctx.needs_input_grad[0]:
+            return (None,) + none
+        g = grad_out.reshape(1)
+        d_a, _ = _ops.p2p_bwd(a_l, b_g, c, meta_a, meta_b_g, shift_l, w_l, temperature, stats_l, g, True, False, n_class,
+                              selfcol_f, selfrow_g, state_l if n_class > 0 else None)
+        _, d_b = _ops.p2p_bwd(a_g, b_l, c, meta_a_g, meta_b, shift_g, w_g, temperature, stats_g, g, False, True, n_class,
+                              a_selfcol_g, b_selfrow_l, state_g)
+        if rowmaps is not None and not same_rows:
+            return (_ops.scatter_rows_by_map(fm, normalize, rowmaps[0], d_a.contiguous(), inv_a, rowmaps[1], d_b.contiguous(),
+                                             inv_b),) + none
+        dfeat = torch.zeros_like(fm)
+        if same_rows:
+            _ops.scatter_rows_bwd(fm, idx_b, normalize, d_a + d_b, inv_b, dfeat)
+        else:
+            _ops.scatter_rows_bwd(fm, idx_a, normalize, d_a, inv_a, dfeat)
+            _ops.scatter_rows_bwd(fm, idx_b, normalize, d_b, inv_b, dfeat)
+        return (dfeat,) + none
+
+
+def _offset_ids(meta, n, offset):
+    """{label, id} rows with the ids of the first n rows moved by `offset` (ids unique across ranks)."""
+    if offset:
+        meta[:n, 1] += offset
+    return meta
 
 
 def p2p_loss(feat, idx_a, idx_b, lab_a, lab_b, id_a, id_b, weight, temperature, normalize, same_rows=False, n_class=0,
@@ -172,7 +391,7 @@ def _view_major_rows(b: int, v: int, h: int, w: int, ys: torch.Tensor, xs: torch
     return (img.view(-1, 1) * (h * w) + grid.view(1, -1)).reshape(-1)             # (v, b, y, x) order
 
 
-def _supcon(features, labels, temperature, ys, xs, zero_if_no_foreground=False, n_class=0, geom=None):
+def _supcon(features, labels, temperature, ys, xs, zero_if_no_foreground=False, n_class=0, geom=None, x=None):
     if features.ndim <= 3:                                                          # :334-336
         raise ValueError('`features` needs to be [bsz, n_views, ...],'
                          'at least 4 dimensions are required')
@@ -189,6 +408,8 @@ def _supcon(features, labels, temperature, ys, xs, zero_if_no_foreground=False, 
         idx = _view_major_rows(b, v, h, w, ys, xs, dev)
         ids = torch.arange(idx.numel(), device=dev, dtype=torch.int32)
     m = idx.numel()
+    if x is not None:
+        return _supcon_global(fmap, labels, idx, ids, m, v, temperature, zero_if_no_foreground, n_class, x)
     if labels is not None:
         # {label, pixel index} rows and the foreground weights fg / sum fg (:352-358, :382-384) in three launches;
         # zero_if_no_foreground: LocalConLoss / BlockConLoss early-out (:405-407, :439-440), without a host sync
@@ -204,11 +425,29 @@ def _supcon(features, labels, temperature, ys, xs, zero_if_no_foreground=False, 
     return p2p_loss(fmap, idx, idx, lab, lab, ids, ids, weight, temperature, normalize=False, same_rows=True, n_class=0)
 
 
+def _supcon_global(fmap, labels, idx, ids, m, v, temperature, zero_if_no_foreground, n_class, x):
+    """SupCon over the union of every rank's rows (rank-major): ids are pixel indices offset by the rank's pixel count
+    (labelled), or row indices offset by the rank's row count with "same pixel, other view" labels offset likewise."""
+    n_pix = fmap.shape[0] * fmap.shape[2] * fmap.shape[3]
+    if max(n_pix, m) * x.world >= 2 ** 31:
+        raise ValueError("group=: the global row / pixel ids must fit in int32")
+    no_short = torch.zeros((), dtype=torch.bool, device=fmap.device)
+    if labels is not None:
+        meta = _offset_ids(_ops.rows_meta(labels.reshape(-1).long(), idx), m, x.rank * n_pix)
+        selfcol = torch.arange(m, device=fmap.device, dtype=torch.int32) if n_class > 0 else None
+        return _P2PGlobal.apply(fmap, idx, idx, meta, meta, no_short, float(temperature), False, True, int(n_class), selfcol,
+                                selfcol, False, bool(zero_if_no_foreground), x, None)
+    per = m // v
+    meta = ops.pad_meta(ids % per + x.rank * per, ids + x.rank * m)
+    return _P2PGlobal.apply(fmap, idx, idx, meta, meta, no_short, float(temperature), False, True, 0, None, None, True, False,
+                            x, None)
+
+
 class SupConLoss(nn.Module):
     """Reference utils/loss.py:315-387.  ``contrast_mode`` / ``base_temperature`` are stored and
     unused there too."""
 
-    def __init__(self, temperature=0.07, contrast_mode='all', base_temperature=0.07, n_class=None):
+    def __init__(self, temperature=0.07, contrast_mode='all', base_temperature=0.07, n_class=None, group=None):
         super().__init__()
         self.temperature = temperature
         self.contrast_mode = contrast_mode
@@ -217,6 +456,15 @@ class SupConLoss(nn.Module):
         # (any integer labels); None (default) = decided from the labels themselves (_AutoClasses)
         self.n_class = n_class
         self._classes = _AutoClasses(n_class)
+        # extension (INTEGRATION.md section 4): None = this batch only.  True / a ProcessGroup (NCCL) or a
+        # slcl.peer.PeerMailbox built with rows_bytes (NVLink peer memory): every forward gets this rank's shard of a
+        # data-parallel batch and returns SupCon over the GLOBAL batch -- every rank's rows are anchors and contrast rows,
+        # in rank order; every rank returns the same loss and gets its shard of the gradient.  All ranks pass equal
+        # shapes, make the same sequence of group= calls and back-propagate the same grad_out.  A constructor argument
+        # here because SupConLoss.forward is a drop-in whose parameter list stays exactly the reference's (features,
+        # labels); LocalConLoss, which has no such constraint, also takes it per call.  Without n_class, the sweeps are
+        # chosen once, at the first labelled call, from the label range over all ranks of that call's group.
+        self.group = group
 
     def forward(self, features, labels=None):
         if features.ndim <= 3:
@@ -224,28 +472,36 @@ class SupConLoss(nn.Module):
                              'at least 4 dimensions are required')
         h, w = features.shape[-2:]
         dev = features.device
-        n_class, in_range = self._classes.resolve(labels)
+        x = _exchange(self.group)
+        n_class, in_range = self._classes.resolve(labels, x)
         return _guard(_supcon(features, labels, self.temperature, lambda: torch.arange(h, device=dev),
-                              lambda: torch.arange(w, device=dev), n_class=n_class, geom=("all",)), in_range)
+                              lambda: torch.arange(w, device=dev), n_class=n_class, geom=("all",), x=x), in_range)
 
 
 class LocalConLoss(nn.Module):
     """Reference utils/loss.py:390-413: stride-subsampled SupCon."""
 
-    def __init__(self, temperature=0.7, stride=4, n_class=None):
+    def __init__(self, temperature=0.7, stride=4, n_class=None, group=None):
         super().__init__()
         self.temp = temperature
-        self.supconloss = SupConLoss(temperature=self.temp, n_class=n_class)
+        # group: as SupConLoss's (the default of forward's group)
+        self.supconloss = SupConLoss(temperature=self.temp, n_class=n_class, group=group)
         self.stride = stride
 
-    def forward(self, features, labels=None):
+    def forward(self, features, labels=None, group=None):
+        """``group`` (extension; INTEGRATION.md section 4): the data-parallel group of this call -- None = the one given to
+        the constructor (None there too: this batch only); True / a ProcessGroup (NCCL) or a ``slcl.peer.PeerMailbox``
+        built with ``rows_bytes``: the loss of the GLOBAL batch, as ``SupConLoss(group=)``.  The "no foreground -> 0"
+        early-out then holds only when no rank has foreground.  Without ``n_class`` the sweeps are chosen once per module,
+        at its first labelled call, from the label range over all ranks of that call's group."""
         h, w = features.shape[-2:]
         dev = features.device
         st = self.stride
-        n_class, in_range = self.supconloss._classes.resolve(labels)
+        x = _exchange(self.supconloss.group if group is None else group)
+        n_class, in_range = self.supconloss._classes.resolve(labels, x)
         return _guard(_supcon(features, labels, self.temp, lambda: torch.arange(0, h, st, device=dev),
                               lambda: torch.arange(0, w, st, device=dev), zero_if_no_foreground=True, n_class=n_class,
-                              geom=("stride", st)), in_range)
+                              geom=("stride", st), x=x), in_range)
 
 
 class BlockConLoss(nn.Module):
@@ -345,11 +601,19 @@ def sample_class_balanced(labels: torch.Tensor, n_anchor: int, n_contrast: int, 
 def sampled_supcon_loss(feat: torch.Tensor, labels: torch.Tensor, n_anchor: int, n_contrast: int, n_class: int,
                         temperature: float = 0.7, generator: Optional[torch.Generator] = None,
                         anchor_idx: Optional[torch.Tensor] = None, contrast_idx: Optional[torch.Tensor] = None,
-                        analytic: bool = True):
+                        analytic: bool = True, group=None):
     """Sampled rectangular pixel <-> pixel loss (BASELINE.json configs[2]): anchors x contrast rows
     drawn class-balanced from an NCHW map, L2-normalised, bf16 tensor-core similarities.  The whole call -- draw,
     compaction, gather, sweeps -- runs without a host synchronisation; if the map holds fewer labelled pixels than the
-    sample needs, the loss is NaN (decided on the device)."""
+    sample needs, the loss is NaN (decided on the device).
+
+    ``group`` (extension; INTEGRATION.md section 4): ``feat`` / ``labels`` are this rank's shard of a data-parallel batch.
+    Each rank draws its rows from its own shard with its own generator, exactly as without a group; the loss is the one of
+    the union of all ranks' draws (anchors and contrast rows in rank order, weights fg_i / sum fg over all anchors), the same
+    on every rank, and the gradient is this rank's shard of its gradient.  NaN on every rank if any rank is short of
+    labelled pixels.  ``True`` / a ProcessGroup: NCCL; a ``slcl.peer.PeerMailbox`` built with ``rows_bytes >=
+    global_record_bytes(...)``: NVLink peer memory.  All ranks pass equal shapes, make the same sequence of ``group=``
+    calls and back-propagate the same grad_out."""
     short = None
     if anchor_idx is None or contrast_idx is None:
         anchor_idx, contrast_idx, a_fill, c_fill = sample_class_balanced(labels, n_anchor, n_contrast, n_class, generator,
@@ -357,6 +621,9 @@ def sampled_supcon_loss(feat: torch.Tensor, labels: torch.Tensor, n_anchor: int,
         short = (a_fill < anchor_idx.numel()) | (c_fill < contrast_idx.numel())
     lab = labels.reshape(-1).long()
     anchor_idx, contrast_idx = anchor_idx.reshape(-1).long(), contrast_idx.reshape(-1).long()
+    x = _exchange(group)
+    if x is not None:
+        return _sampled_global(feat, lab, anchor_idx, contrast_idx, short, n_class, temperature, analytic, x)
     meta_a, meta_b = _ops.rows_meta(lab, anchor_idx), _ops.rows_meta(lab, contrast_idx)          # {label, pixel index}
     weight, _ = _ops.tile_weights(meta_a, anchor_idx.numel(), 1, False)          # fg / sum fg over the anchors
     # analytic sweeps need class-index labels (true here) and unique picks (distinct pixels of one permutation are)
@@ -365,6 +632,25 @@ def sampled_supcon_loss(feat: torch.Tensor, labels: torch.Tensor, n_anchor: int,
     if short is not None:
         loss = torch.where(short, torch.full_like(loss, float("nan")), loss)
     return loss
+
+
+def _sampled_global(feat, lab, anchor_idx, contrast_idx, short, n_class, temperature, analytic, x):
+    n_pix = lab.numel()
+    if n_pix * x.world >= 2 ** 31:
+        raise ValueError("group=: the global pixel ids must fit in int32")
+    off = x.rank * n_pix                 # ids: pixel index in the rank-major global map
+    meta_a = _offset_ids(_ops.rows_meta(lab, anchor_idx), anchor_idx.numel(), off)
+    meta_b = _offset_ids(_ops.rows_meta(lab, contrast_idx), contrast_idx.numel(), off)
+    n_cls = n_class if (analytic and n_class <= 8) else 0
+    selfcol = selfrow = rowmaps = None
+    if n_cls > 0:                         # self pairs live on one rank: the local maps, offset inside _P2PGlobal
+        selfcol, selfrow, tables = _ops.self_maps_bounded(anchor_idx, contrast_idx, n_pix)
+        if (anchor_idx.numel() + contrast_idx.numel()) * 4 >= n_pix:
+            rowmaps = tables
+    if short is None:
+        short = torch.zeros((), dtype=torch.bool, device=feat.device)
+    return _P2PGlobal.apply(feat, anchor_idx, contrast_idx, meta_a, meta_b, short, float(temperature), True, False, n_cls,
+                            selfcol, selfrow, False, False, x, rowmaps)
 
 
 class InterpolatedSupervisedContrastiveLoss(nn.Module):

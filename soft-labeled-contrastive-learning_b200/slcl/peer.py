@@ -12,6 +12,11 @@ The mailboxes live in ``torch.distributed._symmetric_memory`` (one process per G
 the ``group=`` argument of ``mpcl_loss_calc`` / ``mpcl_target_step`` / ``update_class_center_iter`` / ``cal_centroid``.
 Rules: every rank makes the same sequence of ``group=mailbox`` calls, all on one CUDA stream per mailbox.  When
 symmetric memory cannot be set up, pass ``group=True`` (or a ProcessGroup) and the same calls use NCCL all-reduces.
+
+The pixel <-> pixel losses over the global batch (``SupConLoss`` / ``LocalConLoss`` / ``sampled_supcon_loss`` with
+``group=mailbox``) exchange whole row sets (megabytes per rank).  Those go through a second, bulk region per rank
+(``rows_bytes`` at construction; ``slcl_peer_allgather``): each rank copies its record into its own send slot and its
+peers read it with 16-byte NVLink loads into private tensors, with the mailbox epoch as the flag.
 """
 from __future__ import annotations
 
@@ -26,14 +31,22 @@ DEFAULT_CAPACITY_WORDS = 8192        # 4096 doubles per message: [16, 255+1] cla
 DEFAULT_TIMEOUT_S = 600.0            # a rank that checkpoints / evaluates for minutes must not poison the step
 
 
+def _slot_bytes(rows_bytes: int) -> int:
+    if rows_bytes < 16:
+        raise ValueError("rows_bytes must be at least 16")
+    return (int(rows_bytes) + 255) // 256 * 256
+
+
 class PeerMailbox:
     """One mailbox per rank of ``group``.  Construction is a collective call.
 
     ``capacity_words``: payload words per message (two per float64).  ``timeout_s``: how long a kernel waits for a
     peer before it gives up and returns NaN (0 = for ever, like an NCCL collective); ``timeouts()`` reads the count of
-    such events and ``check()`` raises if there were any."""
+    such events and ``check()`` raises if there were any.  ``rows_bytes``: size of the send slot of the bulk row exchange
+    (0 = none; ``slcl.p2p.global_record_bytes`` gives what a pixel <-> pixel loss needs); it must be equal on every rank."""
 
-    def __init__(self, device, group=None, capacity_words: int = DEFAULT_CAPACITY_WORDS, timeout_s: float = DEFAULT_TIMEOUT_S):
+    def __init__(self, device, group=None, capacity_words: int = DEFAULT_CAPACITY_WORDS, timeout_s: float = DEFAULT_TIMEOUT_S,
+                 rows_bytes: int = 0):
         import torch.distributed._symmetric_memory as symm
         if not dist.is_initialized():
             raise RuntimeError("PeerMailbox needs an initialised torch.distributed process group")
@@ -53,6 +66,19 @@ class PeerMailbox:
         torch.cuda.synchronize(self.dev)
         self.handle = symm.rendezvous(self.buf, pg)
         self.ptrs_dev = int(self.handle.buffer_ptrs_dev)
+        self.rows_slot_bytes, self.rows_ptrs_dev, self.rows_buf = 0, 0, None
+        if rows_bytes:
+            slot = _slot_bytes(rows_bytes)
+            agree = torch.tensor([slot, -slot], dtype=torch.int64, device=self.dev)
+            dist.all_reduce(agree, op=dist.ReduceOp.MAX, group=pg)
+            if int(agree[0]) != -int(agree[1]):
+                raise ValueError(f"rows_bytes must be equal on every rank (rank {self.rank}: {rows_bytes})")
+            self.rows_buf = symm.empty(self.lib.slcl_peer_rows_region_bytes(slot), dtype=torch.uint8, device=self.dev)
+            self.rows_buf.zero_()
+            torch.cuda.synchronize(self.dev)
+            self.rows_handle = symm.rendezvous(self.rows_buf, pg)
+            self.rows_ptrs_dev = int(self.rows_handle.buffer_ptrs_dev)
+            self.rows_slot_bytes = slot
         dist.barrier(pg)                      # every mailbox is zeroed and mapped before the first store can arrive
         torch.cuda.synchronize(self.dev)
 
@@ -63,18 +89,31 @@ class PeerMailbox:
         """(ptrs_dev, rank, world, capacity_words, timeout_s): the flat form the torch custom ops take."""
         return self.ptrs_dev, self.rank, self.world, self.capacity_words, self.timeout_s
 
+    def rows_args(self):
+        """(regions_ptr, slot_bytes) of the bulk row exchange (0, 0 without ``rows_bytes``)."""
+        return self.rows_ptrs_dev, self.rows_slot_bytes
+
     def epoch(self) -> int:
         return int(self.buf[0].item())
 
     def timeouts(self) -> int:
         return int(self.buf[1].item())
 
+    def mismatches(self) -> int:
+        """Bulk row exchanges whose records differed in size between ranks (the affected results are NaN)."""
+        return int(self.buf[5].item())
+
     def check(self) -> None:
-        """Host-side check (synchronises): raise if any exchange kernel gave up waiting for a peer."""
+        """Host-side check (synchronises): raise if any exchange kernel gave up waiting for a peer, or if ranks exchanged
+        row sets of different sizes."""
         n = self.timeouts()
         if n:
             raise RuntimeError(f"slcl peer exchange: {n} poll(s) timed out after {self.timeout_s} s on rank {self.rank}; "
                                "the affected results are NaN")
+        n = self.mismatches()
+        if n:
+            raise RuntimeError(f"slcl peer exchange: {n} row exchange(s) on rank {self.rank} got records of another size "
+                               "from a peer (ranks with different shapes); the affected results are NaN")
 
 
 class _LoopbackBox(PeerMailbox):
@@ -89,6 +128,8 @@ class _LoopbackBox(PeerMailbox):
         self.timeout_s = owner.timeout_s
         self.buf = owner.bufs[rank]
         self.ptrs_dev = owner.table.data_ptr()
+        self.rows_slot_bytes = owner.rows_slot_bytes
+        self.rows_ptrs_dev = owner.rows_table.data_ptr() if owner.rows_table is not None else 0
 
 
 class LoopbackMailboxes:
@@ -96,7 +137,8 @@ class LoopbackMailboxes:
     Several "ranks" can then run on different CUDA streams of one GPU and really exchange through the protocol --
     how the single-GPU test box exercises the multi-rank kernels."""
 
-    def __init__(self, world: int, device, capacity_words: int = DEFAULT_CAPACITY_WORDS, timeout_s: float = 20.0):
+    def __init__(self, world: int, device, capacity_words: int = DEFAULT_CAPACITY_WORDS, timeout_s: float = 20.0,
+                 rows_bytes: int = 0):
         self.lib = _lib.load()
         self.dev = torch.device(device)
         self.world = int(world)
@@ -107,5 +149,11 @@ class LoopbackMailboxes:
             raise ValueError("peer exchange supports 1..16 ranks and capacity >= 2 words")
         self.bufs: List[torch.Tensor] = [torch.zeros(n_bytes // 8, dtype=torch.int64, device=self.dev) for _ in range(world)]
         self.table = torch.tensor([b.data_ptr() for b in self.bufs], dtype=torch.int64, device=self.dev)
+        self.rows_slot_bytes, self.rows_table = 0, None
+        if rows_bytes:                        # the bulk row regions, in plain device memory
+            self.rows_slot_bytes = _slot_bytes(rows_bytes)
+            n = self.lib.slcl_peer_rows_region_bytes(self.rows_slot_bytes)
+            self.rows_bufs = [torch.zeros(n, dtype=torch.uint8, device=self.dev) for _ in range(world)]
+            self.rows_table = torch.tensor([b.data_ptr() for b in self.rows_bufs], dtype=torch.int64, device=self.dev)
         torch.cuda.synchronize(self.dev)
         self.boxes = [_LoopbackBox(self, r) for r in range(world)]
