@@ -414,6 +414,9 @@ int slcl_entropy_map(const float* prob, int64_t n_elems, int n_class, float* out
  *     per-class sums per batch): anchors [z A/n, (z+1) A/n) are
  *     contrasted with contrast rows [z M/n, (z+1) M/n) only -- BlockConLoss (utils/loss.py:416-466) as ONE launch per
  *     sweep instead of div_num^2 separate problems.  A/n and M/n must be multiples of 128.
+ * Sizes: A and M below INT_MAX - 128 in either mode (row indices are 32-bit); every finishing and reduction stage
+ * grid-strides or sizes its partials from A, so no other row bound applies.  The workspace and the kept state grow
+ * linearly with A (U partials and dA split partials: about 4 A dp bytes each per column split).
  * forward : stats [A,3] = {sum_j exp(S_ij - shift_i), sum_pos S_ij * T, #pos},
  *           loss [1] = sum_i w_i (shift_i + log stats_i0 - stats_i1/(T stats_i2)).
  * backward: d_a [A, dim] and/or d_b [M, dim] fp32 = dL/da, dL/db for dL/dloss = *grad_out
@@ -463,6 +466,13 @@ int slcl_p2p_state_layout(int64_t n_anchor, int64_t dim_padded, int64_t* offsets
 int slcl_p2p_state_assemble(void* bwd_state, int64_t n_anchor, int64_t dim_padded, int n_class, const float* alpha,
                             const float* beta, const float* colshift, const float* absum_parts, int n_parts,
                             slcl_stream_t stream);
+/* The same for n_batch block-diagonal batches (the d_b backward of a block-diagonal problem, BlockConLoss(group=)):
+ * alpha / beta / colshift [n_anchor] are already in the global batch-major order the d_b sweep reads, and absum_parts is
+ * [n_parts][n_batch][n_class][dim_padded + 1] (one ABsum table per batch and rank, summed in rank order).  n_batch > 1
+ * needs n_anchor / n_batch a multiple of 128, as slcl_p2p_bwd does.  slcl_p2p_state_assemble is the n_batch = 1 case. */
+int slcl_p2p_state_assemble_batched(void* bwd_state, int64_t n_anchor, int64_t dim_padded, int n_class, int n_batch,
+                                    const float* alpha, const float* beta, const float* colshift, const float* absum_parts,
+                                    int n_parts, slcl_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -1780,8 +1780,9 @@ extern "C" int slcl_p2p_state_layout(int64_t n_anchor, int64_t dim_padded, int64
 
 namespace slcl {
 namespace {
-// Backward state of the dB sweep over the anchors of all ranks: per-anchor constants concatenated (colshift padded with the
-// switch-off shift), ABsum = sum of the ranks' tables in rank order (identical bits on every rank).
+// Backward state of the dB sweep over the anchors of all ranks: per-anchor constants as gathered (colshift padded with the
+// switch-off shift), ABsum = sum of the ranks' tables in rank order (identical bits on every rank).  n_tab covers the
+// tables of every block-diagonal batch ([n_batch][K][d+1], contiguous in the parts and in the state alike).
 __global__ void __launch_bounds__(256) p2p_state_assemble_kernel(int n_anchor, int n_padded, int n_tab, const float* alpha,
                                                                  const float* beta, const float* colshift, const float* absum_parts,
                                                                  int n_parts, float* st_alpha, float* st_beta,
@@ -1799,21 +1800,31 @@ __global__ void __launch_bounds__(256) p2p_state_assemble_kernel(int n_anchor, i
 }  // namespace
 }  // namespace slcl
 
+extern "C" int slcl_p2p_state_assemble_batched(void* bwd_state, int64_t n_anchor, int64_t dim_padded, int n_class, int n_batch,
+                                               const float* alpha, const float* beta, const float* colshift,
+                                               const float* absum_parts, int n_parts, slcl_stream_t stream_) {
+  if (!bwd_state || !aligned16(bwd_state) || !alpha || !beta || !colshift || !absum_parts || n_anchor <= 0 ||
+      n_anchor >= (int64_t)INT_MAX - BM || dim_padded <= 0 || dim_padded > kMaxD || dim_padded % KCH || n_class < 1 ||
+      n_class > kMaxLabelClasses || n_parts < 1 || n_batch < 1)
+    return SLCL_ERR_INVALID_ARGUMENT;
+  // the state holds one table per possible batch of whole 128-row tiles (carve_state)
+  if (n_batch > 1 && (n_anchor % n_batch || (n_anchor / n_batch) % BM)) return SLCL_ERR_INVALID_ARGUMENT;
+  const int d = (int)dim_padded;
+  P2PState s = carve_state(bwd_state, n_anchor, d);
+  const int64_t n_padded = (int64_t)align_up((size_t)n_anchor, BN), n_tab = (int64_t)n_batch * n_class * (d + 1);
+  const int64_t n = n_padded > n_tab ? n_padded : n_tab;
+  if (n >= (int64_t)INT_MAX - 256) return SLCL_ERR_INVALID_ARGUMENT;
+  p2p_state_assemble_kernel<<<(unsigned)ceil_div<int64_t>(n, 256), 256, 0, (cudaStream_t)stream_>>>(
+      (int)n_anchor, (int)n_padded, (int)n_tab, alpha, beta, colshift, absum_parts, n_parts, s.alpha, s.beta, s.colshift,
+      s.absum);
+  return check_launch("slcl_p2p_state_assemble");
+}
+
 extern "C" int slcl_p2p_state_assemble(void* bwd_state, int64_t n_anchor, int64_t dim_padded, int n_class, const float* alpha,
                                        const float* beta, const float* colshift, const float* absum_parts, int n_parts,
                                        slcl_stream_t stream_) {
-  if (!bwd_state || !aligned16(bwd_state) || !alpha || !beta || !colshift || !absum_parts || n_anchor <= 0 ||
-      n_anchor >= (int64_t)kMaxFinishBlocks * 256 || dim_padded <= 0 || dim_padded > kMaxD || dim_padded % KCH || n_class < 1 ||
-      n_class > kMaxLabelClasses || n_parts < 1)
-    return SLCL_ERR_INVALID_ARGUMENT;
-  const int d = (int)dim_padded;
-  P2PState s = carve_state(bwd_state, n_anchor, d);
-  const int n_padded = (int)align_up((size_t)n_anchor, BN), n_tab = n_class * (d + 1);
-  const int n = n_padded > n_tab ? n_padded : n_tab;
-  p2p_state_assemble_kernel<<<ceil_div(n, 256), 256, 0, (cudaStream_t)stream_>>>((int)n_anchor, n_padded, n_tab, alpha, beta,
-                                                                                   colshift, absum_parts, n_parts, s.alpha,
-                                                                                   s.beta, s.colshift, s.absum);
-  return check_launch("slcl_p2p_state_assemble");
+  return slcl_p2p_state_assemble_batched(bwd_state, n_anchor, dim_padded, n_class, 1, alpha, beta, colshift, absum_parts,
+                                         n_parts, stream_);
 }
 
 extern "C" int slcl_p2p_fwd(const void* a_bf16, const void* b_bf16, int64_t n_anchor, int64_t n_contrast, int64_t dim_padded,
@@ -1829,7 +1840,6 @@ extern "C" int slcl_p2p_fwd(const void* a_bf16, const void* b_bf16, int64_t n_an
   const int d = (int)dim_padded;
   if (workspace_bytes < slcl_p2p_workspace_bytes(n_anchor, n_contrast, dim_padded) || !aligned16(workspace))
     return SLCL_ERR_WORKSPACE;
-  if (n_anchor >= (int64_t)kMaxFinishBlocks * 256) return SLCL_ERR_UNSUPPORTED;
   cudaStream_t stream = (cudaStream_t)stream_;
   P2PWs w = carve(workspace, n_anchor, n_contrast, d);
   const float inv_t = 1.0f / temperature;
@@ -1880,7 +1890,6 @@ extern "C" int slcl_p2p_bwd(const void* a_bf16, const void* b_bf16, int64_t n_an
   const int d = (int)dim_padded;
   if (workspace_bytes < slcl_p2p_workspace_bytes(n_anchor, n_contrast, dim_padded) || !aligned16(workspace))
     return SLCL_ERR_WORKSPACE;
-  if (n_anchor >= (int64_t)kMaxFinishBlocks * 256) return SLCL_ERR_UNSUPPORTED;
   cudaStream_t stream = (cudaStream_t)stream_;
   P2PWs w = carve(workspace, n_anchor, n_contrast, d);
   const float inv_t = 1.0f / temperature;

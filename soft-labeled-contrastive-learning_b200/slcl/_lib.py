@@ -113,6 +113,7 @@ SIGNATURES = {
     "slcl_peer_allgather": (C.c_int, [_P, _I64, _P, _P, C.POINTER(PeerT), _P, _I64, _P]),
     "slcl_p2p_state_layout": (C.c_int, [_I64, _I64, _P]),
     "slcl_p2p_state_assemble": (C.c_int, [_P, _I64, _I64, C.c_int, _P, _P, _P, _P, C.c_int, _P]),
+    "slcl_p2p_state_assemble_batched": (C.c_int, [_P, _I64, _I64, C.c_int, C.c_int, _P, _P, _P, _P, C.c_int, _P]),
 }
 
 _lib: Optional[C.CDLL] = None

@@ -1037,9 +1037,10 @@ def p2p_state_layout(n_anchor: int, dim_padded: int) -> dict:
 
 @torch.library.custom_op("slcl::p2p_state_assemble", mutates_args=(), device_types="cuda")
 def p2p_state_assemble(alpha: Tensor, beta: Tensor, colshift: Tensor, absum_parts: Tensor, dim_padded: int,
-                       n_class: int) -> Tensor:
-    """Backward state for p2p_bwd(need_b only) over the anchors of all ranks (slcl_p2p_state_assemble): per-anchor constants
-    [A] concatenated in rank order, ABsum tables [parts, n_class * (dim_padded + 1)] summed in rank order."""
+                       n_class: int, n_batch: int = 1) -> Tensor:
+    """Backward state for p2p_bwd(need_b only) over the anchors of all ranks (slcl_p2p_state_assemble_batched): per-anchor
+    constants [A] in the order the d_b sweep reads them (rank-major; batch-major for ``n_batch`` block-diagonal batches),
+    ABsum tables [parts, n_batch * n_class * (dim_padded + 1)] summed in rank order."""
     dev = require_cuda(alpha, beta, colshift, absum_parts)
     lib = _lib.load()
     na = alpha.numel()
@@ -1047,18 +1048,18 @@ def p2p_state_assemble(alpha: Tensor, beta: Tensor, colshift: Tensor, absum_part
         if t.dtype != _F32 or not t.is_contiguous():
             raise ValueError("state pieces must be contiguous float32")
     if beta.numel() != na or colshift.numel() != na or absum_parts.dim() != 2 or \
-            absum_parts.shape[1] != n_class * (dim_padded + 1):
-        raise ValueError("alpha / beta / colshift [A] and absum_parts [parts, n_class * (dim_padded + 1)]")
+            absum_parts.shape[1] != n_batch * n_class * (dim_padded + 1):
+        raise ValueError("alpha / beta / colshift [A] and absum_parts [parts, n_batch * n_class * (dim_padded + 1)]")
     state = torch.empty(lib.slcl_p2p_state_bytes(na, dim_padded), dtype=torch.uint8, device=dev)
     with _guard(dev):
-        st = lib.slcl_p2p_state_assemble(ptr(state), na, dim_padded, n_class, ptr(alpha), ptr(beta), ptr(colshift),
-                                         ptr(absum_parts), absum_parts.shape[0], stream_ptr(dev))
-    check(st, "slcl_p2p_state_assemble")
+        st = lib.slcl_p2p_state_assemble_batched(ptr(state), na, dim_padded, n_class, int(n_batch), ptr(alpha), ptr(beta),
+                                                 ptr(colshift), ptr(absum_parts), absum_parts.shape[0], stream_ptr(dev))
+    check(st, "slcl_p2p_state_assemble_batched")
     return state
 
 
 @p2p_state_assemble.register_fake
-def _(alpha, beta, colshift, absum_parts, dim_padded, n_class):
+def _(alpha, beta, colshift, absum_parts, dim_padded, n_class, n_batch=1):
     return torch.empty(_lib.load().slcl_p2p_state_bytes(alpha.numel(), dim_padded), dtype=torch.uint8, device=alpha.device)
 
 

@@ -185,10 +185,15 @@ def _pack(parts):
     return torch.cat(chunks), layout
 
 
-def _unpack(gathered, layout, i):
-    """Part i of every rank's record, concatenated in rank order along the first dimension (a private copy)."""
+def _unpack(gathered, layout, i, n_batch=1):
+    """Part i of every rank's record, concatenated along the first dimension (a private copy): in rank order, or, for a
+    part whose rows fall into ``n_batch`` equal block-diagonal batches, batch-major -- [batch][rank][rows of the batch] --
+    so that every batch's rows of all ranks are contiguous.  The reordering is a strided view in front of the one copy."""
     off, n, dtype, shape = layout[i]
-    return gathered[:, off:off + n].contiguous().view(dtype).reshape((-1,) + shape[1:])
+    part = gathered[:, off:off + n]
+    if n_batch > 1:
+        part = part.view(gathered.shape[0], n_batch, n // n_batch).transpose(0, 1)
+    return part.contiguous().view(dtype).reshape((-1,) + shape[1:])
 
 
 def _pad_meta_rows(meta):
@@ -197,80 +202,99 @@ def _pad_meta_rows(meta):
     return out
 
 
-def global_record_bytes(n_anchor: int, n_contrast: int, channels: int, same_rows: bool = False) -> int:
+def global_record_bytes(n_anchor: int, n_contrast: int, channels: int, same_rows: bool = False, n_batch: int = 1) -> int:
     """Send-slot size (``rows_bytes`` of ``PeerMailbox`` / ``LoopbackMailboxes``) that a ``group=`` pixel <-> pixel loss with
-    this many anchors / contrast rows per rank and ``channels`` feature channels needs."""
+    this many anchors / contrast rows per rank and ``channels`` feature channels needs.  ``n_batch``: block-diagonal
+    batches (``BlockConLoss``: div^2 tiles), each of which carries its own table of per-class sums."""
     p16 = lambda n: (n + 15) // 16 * 16
     dp = (channels + 63) // 64 * 64
     rows = lambda r: r * dp * 2 + p16(r * 8) + p16(r * 4)
     first = 16 + 16 + rows(n_contrast) + (0 if same_rows else rows(n_anchor))
-    second = 16 + 16 + max(3 * p16(n_anchor * 4) + p16(AUTO_N_CLASS * (dp + 1) * 4), p16(n_anchor * 12))
+    second = 16 + 16 + max(3 * p16(n_anchor * 4) + p16(n_batch * AUTO_N_CLASS * (dp + 1) * 4), p16(n_anchor * 12))
     return max(first, second)
+
+
+def _global_self_maps(selfcol, selfrow, na, m, world, rank, n_batch):
+    """The local self maps carried into the global row index spaces, whose order is [batch][rank][row of the batch]
+    (rank-major for n_batch = 1): -> (local anchors -> global contrast rows [na], global contrast rows -> local anchors
+    [m world], global anchors -> local contrast rows [na world], local contrast rows -> global anchors [m]); -1 = no self
+    pair (a self pair never crosses ranks)."""
+    ra, rb = na // n_batch, m // n_batch
+
+    def to_global(i, rows):          # local (batch t, row k) -> global t world rows + rank rows + k
+        i = i.long()
+        return torch.where(i >= 0, (i // rows) * (world * rows) + rank * rows + i % rows, i).to(torch.int32)
+
+    selfrow_g = torch.full((n_batch, world, rb), -1, dtype=torch.int32, device=selfcol.device)
+    selfrow_g[:, rank] = selfrow.view(n_batch, rb)
+    a_selfcol_g = torch.full((n_batch, world, ra), -1, dtype=torch.int32, device=selfcol.device)
+    a_selfcol_g[:, rank] = selfcol.view(n_batch, ra)
+    return to_global(selfcol, rb), selfrow_g.view(-1), a_selfcol_g.view(-1), to_global(selfrow, ra)
 
 
 class _P2PGlobal(torch.autograd.Function):
     """loss(feat) of the pixel <-> pixel problem over the GLOBAL batch of ``x.world`` ranks (INTEGRATION.md section 4).
 
     Anchors and contrast rows are the union of every rank's rows in rank order; ``meta_*`` carry ids that are unique across
-    ranks.  Forward: all-gather {rows, meta, norms, short flag} -> weights / shifts of the global problem -> this rank's
+    ranks.  With ``n_batch`` > 1 block-diagonal batches (BlockConLoss's tiles) each rank's rows are batch-major, and the
+    union is ordered [batch][rank][row of the batch]: batch z of the global problem is batch z of every rank.
+    Forward: all-gather {rows, meta, norms, short flag} -> weights / shifts of the global problem -> this rank's
     anchors x all contrast rows (slcl_p2p_fwd) -> all-gather {loss partial, per-anchor backward constants}.  Backward, no
     exchange: d_a = this rank's anchors x all contrast rows, d_b = all anchors x this rank's contrast rows (slcl_p2p_bwd with
     a state assembled from the gathered constants), so this rank gets exactly its shard of the global gradient."""
 
     @staticmethod
     def forward(ctx, feat, idx_a, idx_b, meta_a, meta_b, short, temperature, normalize, same_rows, n_class, selfcol, selfrow,
-                uniform_weight, zero_if_empty, x, rowmaps):
+                uniform_weight, zero_if_empty, x, rowmaps, n_batch, maps_key):
         fm = feat.detach().contiguous()
         c = fm.shape[1]
         dev = fm.device
-        W, r = x.world, x.rank
+        W, r, T = x.world, x.rank, n_batch
         b_l, _, inv_b = _ops.gather_unit_rows(fm, idx_b, normalize, True, False)
         if same_rows:
             a_l, inv_a = b_l, inv_b
         else:
             a_l, _, inv_a = _ops.gather_unit_rows(fm, idx_a, normalize, True, False)
         na, m, dp = a_l.shape[0], b_l.shape[0], b_l.shape[1]
-        flags = int(same_rows) | int(normalize) << 1 | n_class << 2
+        flags = int(same_rows) | int(normalize) << 1 | n_class << 2 | (T - 1) << 6
         parts = [_key(dev, na, m, dp, flags), short.reshape(1).to(torch.int32), b_l, meta_b[:m], inv_b]
         if not same_rows:
             parts += [a_l, meta_a[:na], inv_a]
         rec, lay = _pack(parts)
         status = torch.zeros(1, dtype=torch.int32, device=dev)
         g1 = x.allgather(rec, status)
-        b_g, meta_b_g, inv_b_g = _unpack(g1, lay, 2), _pad_meta_rows(_unpack(g1, lay, 3)), _unpack(g1, lay, 4)
+        b_g, meta_b_g, inv_b_g = _unpack(g1, lay, 2, T), _pad_meta_rows(_unpack(g1, lay, 3, T)), _unpack(g1, lay, 4, T)
         if same_rows:
             a_g, meta_a_g, inv_a_g = b_g, meta_b_g, inv_b_g
         else:
-            a_g, meta_a_g, inv_a_g = _unpack(g1, lay, 5), _pad_meta_rows(_unpack(g1, lay, 6)), _unpack(g1, lay, 7)
+            a_g, meta_a_g, inv_a_g = _unpack(g1, lay, 5, T), _pad_meta_rows(_unpack(g1, lay, 6, T)), _unpack(g1, lay, 7, T)
         short_any = (_unpack(g1, lay, 1) != 0).any()
         na_g, m_g = na * W, m * W
         if uniform_weight:
             w_g = torch.full((na_g,), 1.0 / na_g, device=dev)
-        else:         # fg_i / sum fg over the anchors of all ranks
-            w_g, _ = _ops.tile_weights(meta_a_g, na_g, 1, bool(zero_if_empty))
-        mine = slice(na * r, na * (r + 1))
-        w_l = w_g[mine]
+        else:         # fg_i / sum fg over the anchors of all ranks (per batch, averaged over the batches with foreground)
+            w_g, _ = _ops.tile_weights(meta_a_g, na_g, T, bool(zero_if_empty))
+        mine = lambda t: t.view(T, W, -1)[:, r].reshape(-1)          # this rank's rows of every batch
+        w_l = mine(w_g)
         if normalize:
             shift_g = torch.full((na_g,), 1.0 / temperature, device=dev)
         else:         # |a_i| max_j |b_j| / T over the contrast rows of all ranks
             shift_g = _ops.p2p_shift(inv_a_g, inv_b_g, temperature)
-        shift_l = shift_g[mine]
+        shift_l = mine(shift_g)
         analytic = n_class > 0
         selfcol_f = selfrow_g = a_selfcol_g = b_selfrow_l = None
-        if selfcol is not None:        # the local self maps, offset into the global row index spaces
-            selfcol_f = torch.where(selfcol >= 0, selfcol + m * r, selfcol).to(torch.int32)
-            selfrow_g = torch.full((m_g,), -1, dtype=torch.int32, device=dev)
-            selfrow_g[m * r:m * (r + 1)] = selfrow
-            a_selfcol_g = torch.full((na_g,), -1, dtype=torch.int32, device=dev)
-            a_selfcol_g[mine] = selfcol
-            b_selfrow_l = torch.where(selfrow >= 0, selfrow + na * r, selfrow).to(torch.int32)
+        if selfcol is not None:        # the local self maps, moved into the global row index spaces
+            build = lambda: _global_self_maps(selfcol, selfrow, na, m, W, r, T)
+            # maps_key: the self maps are a pure function of the geometry it names (cached like the row indices)
+            selfcol_f, selfrow_g, a_selfcol_g, b_selfrow_l = (build() if maps_key is None else
+                                                              _cached(("global_self_maps", maps_key, W, r, T), build))
         loss_l, stats_l, state_l = _ops.p2p_fwd(a_l, b_g, meta_a, meta_b_g, shift_l, w_l, temperature, n_class, selfcol_f,
-                                                analytic, 1)
+                                                analytic, T)
         parts2 = [_key(dev, na, m, dp, flags), loss_l]
         if analytic:
             off = ops.p2p_state_layout(na, dp)
             f32 = lambda name, n: state_l[off[name]:off[name] + 4 * n].view(torch.float32)
-            parts2 += [f32("alpha", na), f32("beta", na), f32("colshift", na), f32("absum", n_class * (dp + 1))]
+            parts2 += [f32("alpha", na), f32("beta", na), f32("colshift", na), f32("absum", T * n_class * (dp + 1))]
         else:
             parts2 += [stats_l]
         rec2, lay2 = _pack(parts2)
@@ -281,30 +305,31 @@ class _P2PGlobal(torch.autograd.Function):
             loss = loss + partials[q]
         loss = torch.where((status[0] != 0) | short_any, torch.full_like(loss, float("nan")), loss)
         if analytic:
-            state_g = _ops.p2p_state_assemble(_unpack(g2, lay2, 2), _unpack(g2, lay2, 3), _unpack(g2, lay2, 4),
-                                              _unpack(g2, lay2, 5).reshape(W, -1), dp, n_class)
+            # per-anchor constants batch-major like the anchors; the ABsum tables stay rank-major (summed in rank order)
+            state_g = _ops.p2p_state_assemble(_unpack(g2, lay2, 2, T), _unpack(g2, lay2, 3, T), _unpack(g2, lay2, 4, T),
+                                              _unpack(g2, lay2, 5).reshape(W, -1), dp, n_class, T)
             stats_g = stats_l          # (not read by the analytic backward with a state)
         else:
-            state_g, stats_g = None, _unpack(g2, lay2, 2).reshape(na_g, 3)
+            state_g, stats_g = None, _unpack(g2, lay2, 2, T).reshape(na_g, 3)
         ctx.save_for_backward(fm, idx_a, idx_b, a_l, b_l, a_g, b_g, meta_a, meta_b, meta_a_g, meta_b_g, inv_a, inv_b, shift_l,
                               shift_g, w_l, w_g, stats_l, stats_g, state_l, state_g, selfcol_f, selfrow_g, a_selfcol_g,
                               b_selfrow_l, rowmaps)
-        ctx.cfg = (temperature, normalize, same_rows, c, n_class)
+        ctx.cfg = (temperature, normalize, same_rows, c, n_class, T)
         return loss
 
     @staticmethod
     def backward(ctx, grad_out):
         (fm, idx_a, idx_b, a_l, b_l, a_g, b_g, meta_a, meta_b, meta_a_g, meta_b_g, inv_a, inv_b, shift_l, shift_g, w_l, w_g,
          stats_l, stats_g, state_l, state_g, selfcol_f, selfrow_g, a_selfcol_g, b_selfrow_l, rowmaps) = ctx.saved_tensors
-        temperature, normalize, same_rows, c, n_class = ctx.cfg
-        none = (None,) * 15
+        temperature, normalize, same_rows, c, n_class, T = ctx.cfg
+        none = (None,) * 17
         if not ctx.needs_input_grad[0]:
             return (None,) + none
         g = grad_out.reshape(1)
         d_a, _ = _ops.p2p_bwd(a_l, b_g, c, meta_a, meta_b_g, shift_l, w_l, temperature, stats_l, g, True, False, n_class,
-                              selfcol_f, selfrow_g, state_l if n_class > 0 else None)
+                              selfcol_f, selfrow_g, state_l if n_class > 0 else None, T)
         _, d_b = _ops.p2p_bwd(a_g, b_l, c, meta_a_g, meta_b, shift_g, w_g, temperature, stats_g, g, False, True, n_class,
-                              a_selfcol_g, b_selfrow_l, state_g)
+                              a_selfcol_g, b_selfrow_l, state_g, T)
         if rowmaps is not None and not same_rows:
             return (_ops.scatter_rows_by_map(fm, normalize, rowmaps[0], d_a.contiguous(), inv_a, rowmaps[1], d_b.contiguous(),
                                              inv_b),) + none
@@ -425,22 +450,25 @@ def _supcon(features, labels, temperature, ys, xs, zero_if_no_foreground=False, 
     return p2p_loss(fmap, idx, idx, lab, lab, ids, ids, weight, temperature, normalize=False, same_rows=True, n_class=0)
 
 
-def _supcon_global(fmap, labels, idx, ids, m, v, temperature, zero_if_no_foreground, n_class, x):
+def _supcon_global(fmap, labels, idx, ids, m, v, temperature, zero_if_no_foreground, n_class, x, n_batch=1, geom=None):
     """SupCon over the union of every rank's rows (rank-major): ids are pixel indices offset by the rank's pixel count
-    (labelled), or row indices offset by the rank's row count with "same pixel, other view" labels offset likewise."""
+    (labelled), or row indices offset by the rank's row count with "same pixel, other view" labels offset likewise.
+    ``n_batch`` > 1: BlockConLoss's block-diagonal tiles -- tile z of the global problem holds tile z's rows of every rank
+    (global order [tile][rank][view, image, y, x], see _unpack), so the ids above are unique within every tile across
+    ranks; ``geom`` names the row geometry, of which the self maps are then a pure function (cached)."""
     n_pix = fmap.shape[0] * fmap.shape[2] * fmap.shape[3]
     if max(n_pix, m) * x.world >= 2 ** 31:
         raise ValueError("group=: the global row / pixel ids must fit in int32")
     no_short = torch.zeros((), dtype=torch.bool, device=fmap.device)
     if labels is not None:
         meta = _offset_ids(_ops.rows_meta(labels.reshape(-1).long(), idx), m, x.rank * n_pix)
-        selfcol = torch.arange(m, device=fmap.device, dtype=torch.int32) if n_class > 0 else None
+        selfcol = ids if n_class > 0 else None          # ids = arange(m): row i is its own contrast row
         return _P2PGlobal.apply(fmap, idx, idx, meta, meta, no_short, float(temperature), False, True, int(n_class), selfcol,
-                                selfcol, False, bool(zero_if_no_foreground), x, None)
-    per = m // v
+                                selfcol, False, bool(zero_if_no_foreground), x, None, n_batch, geom)
+    per = m // (v * n_batch)
     meta = ops.pad_meta(ids % per + x.rank * per, ids + x.rank * m)
     return _P2PGlobal.apply(fmap, idx, idx, meta, meta, no_short, float(temperature), False, True, 0, None, None, True, False,
-                            x, None)
+                            x, None, n_batch, None)
 
 
 class SupConLoss(nn.Module):
@@ -508,24 +536,35 @@ class BlockConLoss(nn.Module):
     """Reference utils/loss.py:416-466: mean of SupCon over block_size x block_size tiles; tiles whose
     labels are all background are skipped (decided on the device, no per-tile host sync)."""
 
-    def __init__(self, temperature=0.7, block_size=32, n_class=None):
+    def __init__(self, temperature=0.7, block_size=32, n_class=None, group=None):
         super().__init__()
         self.block_size = block_size
-        self.supconloss = SupConLoss(temperature=temperature, n_class=n_class)
+        # group: as SupConLoss's (the default of forward's group)
+        self.supconloss = SupConLoss(temperature=temperature, n_class=n_class, group=group)
         self.batched = True             # all tiles as one block-diagonal problem where the shape allows (False: per-tile loop)
 
-    def forward(self, features, labels=None):
+    def forward(self, features, labels=None, group=None):
+        """``group`` (extension; INTEGRATION.md section 4): the data-parallel group of this call -- None = the one given to
+        the constructor (None there too: this batch only); True / a ProcessGroup (NCCL) or a ``slcl.peer.PeerMailbox``
+        built with ``rows_bytes``: the loss of the GLOBAL batch, i.e. BlockConLoss of the ranks' batches concatenated.
+        Every tile's problem is then the union of that tile's rows on all ranks, tile weights and the average over tiles
+        with foreground are decided over that union, and "no foreground -> 0" holds only when no rank has foreground.
+        The global form needs the block-diagonal layout (b v block_size^2 a multiple of 128, ``batched``): other shapes
+        raise ValueError on every rank before anything is exchanged."""
         dev = features.device
         bs = self.block_size
         div = features.shape[-1] // bs                                               # :426-428
         t = self.supconloss.temperature
         if div == 0:
             return torch.zeros((), device=dev)
-        n_class, in_range = self.supconloss._classes.resolve(labels)
-        if self.batched and features.ndim == 5:
-            b, v = features.shape[:2]
-            if (b * v * bs * bs) % 128 == 0:
-                return _guard(self._forward_batched(features, labels, div, t, n_class), in_range)
+        x = _exchange(self.supconloss.group if group is None else group)
+        batched = self.batched and features.ndim == 5 and (features.shape[0] * features.shape[1] * bs * bs) % 128 == 0
+        if x is not None and not batched:
+            raise ValueError("BlockConLoss(group=) needs [b, v, c, h, w] features with b * v * block_size^2 a multiple of "
+                             "128 and batched = True (the per-tile loop would need div^2 exchanges)")
+        n_class, in_range = self.supconloss._classes.resolve(labels, x)
+        if batched:
+            return _guard(self._forward_batched(features, labels, div, t, n_class, x), in_range)
         losses, flags = [], []
         for i in range(div):
             for j in range(div):
@@ -540,7 +579,7 @@ class BlockConLoss(nn.Module):
         keep = torch.stack(flags).float()
         return _guard((stacked * keep).sum() / keep.sum().clamp_min(1.0), in_range)   # :445-448 (0 when every tile is skipped)
 
-    def _forward_batched(self, features, labels, div, t, n_class=0):
+    def _forward_batched(self, features, labels, div, t, n_class=0, x=None):
         """All div x div tiles as ONE block-diagonal problem (one launch per tensor-core sweep instead of div^2
         separate SupCon calls): rows are ordered (tile, view, image, y, x); the per-tile weighting of :445-448 /
         :465 -- fg_i / sum_tile fg, averaged over the tiles that have foreground -- is folded into the row weights.
@@ -558,8 +597,11 @@ class BlockConLoss(nn.Module):
             img = (torch.arange(b, device=dev).view(1, -1) * v + torch.arange(v, device=dev).view(-1, 1)).reshape(-1)   # (v, b)
             i = (img.view(1, -1, 1) * (h * w) + grid.view(div * div, 1, bs * bs)).reshape(-1)           # (tile, v, b, y, x)
             return i, torch.arange(i.numel(), device=dev, dtype=torch.int32)
-        idx, ids = _cached(("blocks", b, v, h, w, bs, div, str(dev)), build)
+        geom = ("blocks", b, v, h, w, bs, div, str(dev))
+        idx, ids = _cached(geom, build)
         n_tiles, m_tile = div * div, b * v * bs * bs
+        if x is not None:
+            return _supcon_global(fmap, labels, idx, ids, idx.numel(), v, t, True, n_class, x, n_tiles, geom)
         if labels is not None:
             meta = _ops.rows_meta(labels.reshape(-1).long(), idx)
             weight, _ = _ops.tile_weights(meta, idx.numel(), n_tiles, True)
@@ -650,7 +692,7 @@ def _sampled_global(feat, lab, anchor_idx, contrast_idx, short, n_class, tempera
     if short is None:
         short = torch.zeros((), dtype=torch.bool, device=feat.device)
     return _P2PGlobal.apply(feat, anchor_idx, contrast_idx, meta_a, meta_b, short, float(temperature), True, False, n_cls,
-                            selfcol, selfrow, False, False, x, rowmaps)
+                            selfcol, selfrow, False, False, x, rowmaps, 1, None)
 
 
 class InterpolatedSupervisedContrastiveLoss(nn.Module):
