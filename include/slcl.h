@@ -371,6 +371,23 @@ int slcl_seg_fwd(const float* logits, const int64_t* labels, int64_t batch, int 
                  float* stats, float* losses, void* workspace, size_t workspace_bytes, slcl_stream_t stream);
 int slcl_seg_bwd(const float* logits, const int64_t* labels, int64_t batch, int n_class, int64_t pixels,
                  const float* stats, const float* grad_losses, float* dlogits, slcl_stream_t stream);
+/* The same losses over the global batch of data-parallel ranks (utils/loss.py:11-103 on the ranks' batches
+ * concatenated in rank order; ranks may hold different B, H W and K must agree).  Each rank reduces its batch into
+ *   vec [2K+4] fp64 = {inter_k (K), card_k (K), n_valid, sum ce, sum dice_bk over its images, n_images}
+ * which is a sum over ranks.  slcl_seg_fwd_peer all-reduces it inside its finaliser through the peer mailboxes (rank
+ * order: identical bits on every rank; capacity_words >= 2 (2K+4)) and writes the GLOBAL vec and losses; a peer that
+ * times out makes both NaN.  slcl_seg_fwd_local writes this rank's vec (the caller sums it over the ranks, e.g. NCCL)
+ * and slcl_seg_finish turns a summed vec into losses with the same arithmetic.  stats stays per local image.
+ * slcl_seg_bwd_global: this rank's dlogits of the global losses, from its stats and the global vec (no exchange). */
+int slcl_seg_fwd_peer(const float* logits, const int64_t* labels, int64_t batch, int n_class, int64_t pixels,
+                      float* stats, double* vec, float* losses, const slcl_peer_t* peer,
+                      void* workspace, size_t workspace_bytes, slcl_stream_t stream);
+int slcl_seg_fwd_local(const float* logits, const int64_t* labels, int64_t batch, int n_class, int64_t pixels,
+                       float* stats, double* vec, void* workspace, size_t workspace_bytes, slcl_stream_t stream);
+int slcl_seg_finish(const double* vec, int n_class, float* losses, slcl_stream_t stream);
+int slcl_seg_bwd_global(const float* logits, const int64_t* labels, int64_t batch, int n_class, int64_t pixels,
+                        const float* stats, const double* vec, const float* grad_losses, float* dlogits,
+                        slcl_stream_t stream);
 int slcl_entropy_map(const float* prob, int64_t n_elems, int n_class, float* out, const float* grad_out,
                      float* dprob, slcl_stream_t stream);
 

@@ -102,6 +102,11 @@ SIGNATURES = {
     "slcl_seg_workspace_bytes": (_SZ, [_I64, _I64, C.c_int]),
     "slcl_seg_fwd": (C.c_int, [_P, _P, _I64, C.c_int, _I64, _P, _P, _P, _SZ, _P]),
     "slcl_seg_bwd": (C.c_int, [_P, _P, _I64, C.c_int, _I64, _P, _P, _P, _P]),
+    # segmentation losses over the global batch of data-parallel ranks (utils/loss.py:11-103)
+    "slcl_seg_fwd_peer": (C.c_int, [_P, _P, _I64, C.c_int, _I64, _P, _P, _P, C.POINTER(PeerT), _P, _SZ, _P]),
+    "slcl_seg_fwd_local": (C.c_int, [_P, _P, _I64, C.c_int, _I64, _P, _P, _P, _SZ, _P]),
+    "slcl_seg_finish": (C.c_int, [_P, C.c_int, _P, _P]),
+    "slcl_seg_bwd_global": (C.c_int, [_P, _P, _I64, C.c_int, _I64, _P, _P, _P, _P, _P]),
     "slcl_entropy_map": (C.c_int, [_P, _I64, C.c_int, _P, _P, _P, _P]),
     "slcl_p2p_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
     "slcl_p2p_state_bytes": (_SZ, [_I64, _I64]),

@@ -1114,6 +1114,118 @@ def _(logits, labels, stats, grad_losses):
     return torch.empty_like(logits)
 
 
+def seg_vec_len(n_class: int) -> int:
+    """Length of the data-parallel vector {inter_k, card_k, n_valid, sum ce, sum dice_bk, n_images} (fp64)."""
+    return 2 * int(n_class) + 4
+
+
+def _seg_inputs(logits: Tensor, labels: Tensor):
+    if logits.dim() != 4 or logits.dtype != _F32:
+        raise ValueError("logits must be float32 [B, K, H, W]")
+    logits = logits.contiguous()
+    b, k, h, w = logits.shape
+    labels = labels.reshape(b, -1).long().contiguous()
+    if labels.shape[1] != h * w:
+        raise ValueError("labels must be [B, H, W] at the resolution of the logits")
+    return logits, labels
+
+
+@torch.library.custom_op("slcl::seg_fwd_peer", mutates_args=(), device_types="cuda")
+def seg_fwd_peer(logits: Tensor, labels: Tensor, peer_ptrs: int, rank: int, world: int, capacity_words: int,
+                 timeout_s: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """Segmentation losses of the ranks' concatenated batches, exchanged through the peer mailboxes inside the
+    finaliser (slcl.peer.PeerMailbox.args()).  -> (GLOBAL losses[3], local stats[B,K,4], GLOBAL vec[2K+4] fp64)."""
+    dev = require_cuda(logits, labels)
+    lib = _lib.load()
+    logits, labels = _seg_inputs(logits, labels)
+    b, k, h, w = logits.shape
+    if capacity_words < 2 * seg_vec_len(k):
+        raise ValueError(f"seg losses over {k} classes exchange {seg_vec_len(k)} doubles: the mailbox needs "
+                         f"capacity_words >= {2 * seg_vec_len(k)}, it has {capacity_words}")
+    stats = torch.empty((b, k, 4), dtype=_F32, device=dev)
+    vec = torch.empty(seg_vec_len(k), dtype=torch.float64, device=dev)
+    losses = torch.empty(3, dtype=_F32, device=dev)
+    ws = _ws(lib.slcl_seg_workspace_bytes(b, h * w, k), dev)
+    peer = PeerT(peer_ptrs, rank, world, capacity_words, timeout_s)
+    with _guard(dev):
+        st = lib.slcl_seg_fwd_peer(ptr(logits), ptr(labels), b, k, h * w, ptr(stats), ptr(vec), ptr(losses), C.byref(peer),
+                                   ptr(ws), ws.numel(), stream_ptr(dev))
+    check(st, "slcl_seg_fwd_peer")
+    return losses, stats, vec
+
+
+@seg_fwd_peer.register_fake
+def _(logits, labels, peer_ptrs, rank, world, capacity_words, timeout_s):
+    b, k = logits.shape[0], logits.shape[1]
+    return logits.new_empty(3), logits.new_empty((b, k, 4)), logits.new_empty(seg_vec_len(k), dtype=torch.float64)
+
+
+@torch.library.custom_op("slcl::seg_fwd_local", mutates_args=(), device_types="cuda")
+def seg_fwd_local(logits: Tensor, labels: Tensor) -> Tuple[Tensor, Tensor]:
+    """-> (stats[B,K,4], this rank's vec[2K+4] fp64); sum vec over the ranks, then seg_finish."""
+    dev = require_cuda(logits, labels)
+    lib = _lib.load()
+    logits, labels = _seg_inputs(logits, labels)
+    b, k, h, w = logits.shape
+    stats = torch.empty((b, k, 4), dtype=_F32, device=dev)
+    vec = torch.empty(seg_vec_len(k), dtype=torch.float64, device=dev)
+    ws = _ws(lib.slcl_seg_workspace_bytes(b, h * w, k), dev)
+    with _guard(dev):
+        st = lib.slcl_seg_fwd_local(ptr(logits), ptr(labels), b, k, h * w, ptr(stats), ptr(vec), ptr(ws), ws.numel(),
+                                    stream_ptr(dev))
+    check(st, "slcl_seg_fwd_local")
+    return stats, vec
+
+
+@seg_fwd_local.register_fake
+def _(logits, labels):
+    b, k = logits.shape[0], logits.shape[1]
+    return logits.new_empty((b, k, 4)), logits.new_empty(seg_vec_len(k), dtype=torch.float64)
+
+
+@torch.library.custom_op("slcl::seg_finish", mutates_args=(), device_types="cuda")
+def seg_finish(vec: Tensor, n_class: int) -> Tensor:
+    """losses[3] = {ce, dice, jaccard} from a vector summed over the ranks (the peer finaliser's arithmetic)."""
+    dev = require_cuda(vec)
+    if vec.dtype != torch.float64 or vec.numel() != seg_vec_len(n_class):
+        raise ValueError(f"vec must be float64 [{seg_vec_len(n_class)}]")
+    v = vec.contiguous()
+    losses = torch.empty(3, dtype=_F32, device=dev)
+    with _guard(dev):
+        st = _lib.load().slcl_seg_finish(ptr(v), int(n_class), ptr(losses), stream_ptr(dev))
+    check(st, "slcl_seg_finish")
+    return losses
+
+
+@seg_finish.register_fake
+def _(vec, n_class):
+    return vec.new_empty(3, dtype=_F32)
+
+
+@torch.library.custom_op("slcl::seg_bwd_global", mutates_args=(), device_types="cuda")
+def seg_bwd_global(logits: Tensor, labels: Tensor, stats: Tensor, vec: Tensor, grad_losses: Tensor) -> Tensor:
+    """This rank's dlogits of the global losses: local stats, global vec (seg_fwd_peer / summed seg_fwd_local)."""
+    dev = require_cuda(logits, labels, stats, vec, grad_losses)
+    lib = _lib.load()
+    logits = logits.contiguous()
+    b, k, h, w = logits.shape
+    if vec.dtype != torch.float64 or vec.numel() != seg_vec_len(k):
+        raise ValueError(f"vec must be float64 [{seg_vec_len(k)}]")
+    labels = labels.reshape(b, -1).long().contiguous()
+    g = grad_losses.to(_F32).reshape(3).contiguous()
+    dlogits = torch.empty_like(logits)
+    with _guard(dev):
+        st = lib.slcl_seg_bwd_global(ptr(logits), ptr(labels), b, k, h * w, ptr(stats.contiguous()), ptr(vec.contiguous()),
+                                     ptr(g), ptr(dlogits), stream_ptr(dev))
+    check(st, "slcl_seg_bwd_global")
+    return dlogits
+
+
+@seg_bwd_global.register_fake
+def _(logits, labels, stats, vec, grad_losses):
+    return torch.empty_like(logits)
+
+
 @torch.library.custom_op("slcl::entropy_map", mutates_args=(), device_types="cuda")
 def entropy_map(prob: Tensor) -> Tensor:
     dev = require_cuda(prob)
