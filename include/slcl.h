@@ -206,14 +206,20 @@ int slcl_pseudo_label(const float* feat, const slcl_map_t* map, const float* cen
  * (utils/utils_.py:580-590) and cal_centroid (utils/utils_.py:509-540).
  *
  * Weights:  hard   w_ik = [label_i == k]                              (labels != null)
- *           soft   w_ik = probs[b,k,p] * cert_i      (weighted != 0)  (probs  != null)
+ *           soft   w_ik = probs[b,k,p] * cert_i      (weighted & SLCL_SOFT_WEIGHTED)  (probs  != null)
  *           argmax w_ik = [argmax_k probs == k] * cert_i (weighted == 0)
  *           cert_i = [max_k probs >= threshold] if 0 < threshold < 1 else 1
  *           and, when part_id != null, times [part_id_i == partition].
+ * `weighted` is a flags word.  SLCL_SOFT_LOGITS: `probs` holds the logits z [B,K,HW] and the kernels use
+ * probs = softmax_k(z) (per pixel: zmax = max_k z_k, arg-max = its first index, s = sum_k expf(z_k - zmax),
+ * p_k = expf(z_k - zmax) / s, max_k p_k = 1/s), the same weights as above from one read of z.  Soft labels only:
+ * the flag with `labels`, or any other bit, returns SLCL_ERR_INVALID_ARGUMENT.
  * Output sums [P*K, C+1] fp64 row-major: columns 0..C-1 = weighted feature
  * sums, column C = weight sum (exact integer counts for hard labels).  This is
  * the buffer a multi-GPU caller all-reduces (SURVEY.md section 8(e)).
  * ------------------------------------------------------------------------- */
+#define SLCL_SOFT_WEIGHTED 1          /* soft weights p_k * cert (else the arg-max one-hot) */
+#define SLCL_SOFT_LOGITS   2          /* `probs` are logits; dprobs of slcl_centroid_bwd receives dL/dlogits */
 size_t slcl_class_sums_workspace_bytes(int64_t batch, int64_t channels, int64_t pixels, int n_cols);
 int slcl_class_sums(const float* feat, int64_t batch, int64_t channels, int64_t pixels,
                     const int64_t* labels, const float* probs, int weighted, float threshold,
@@ -257,6 +263,8 @@ int slcl_centroids_fwd(const float* feat, int64_t batch, int64_t channels, int64
  * (S, W from `sums`, the same -- possibly all-reduced -- buffer the forward used):
  *   dfeat[b,c,p]  = sum_j w_ij * gc[j,c]
  *   dprobs[b,k,p] = cert_i * [part_i] * ( x_i . gc_j - mu_j . gc_j ),  j = part_i*K + k   (soft weighted only)
+ * With SLCL_SOFT_LOGITS (`probs` = logits z, p = softmax_k(z) as in slcl_class_sums), with g_ik the value above:
+ *   dprobs[b,k,p] = dL/dz_ik = p_ik * ( g_ik - sum_m p_im g_im )
  * ema_scale = 1 - momentum when the forward applied the EMA, else 1.
  * dprobs may be null (hard labels / arg-max weights: no gradient to the labels). */
 size_t slcl_centroid_bwd_workspace_bytes(int64_t channels, int n_cols);

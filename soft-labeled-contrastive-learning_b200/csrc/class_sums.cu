@@ -73,10 +73,30 @@ __device__ __forceinline__ void st_vec(float* p, const float (&v)[VEC]) {
   else st_stream1(p, v[0]);
 }
 
+// Logits mode (SLCL_SOFT_LOGITS): the K values z[0..K) of one pixel become softmax(z) in place.  `arg` = first index of
+// the largest logit (torch.argmax), `pmax` = 1/s = the largest probability.  Full-precision expf and an IEEE division,
+// the arithmetic of torch.softmax, so certainty and arg-max decisions agree with softmax-then-probabilities except
+// within the last bits of a tie.
+__device__ __forceinline__ void softmax_inplace(float (&z)[SLCL_MAX_CLASSES], int K, float& pmax, int& arg) {
+  float zmax = -INFINITY;
+  arg = 0;
+#pragma unroll
+  for (int k = 0; k < SLCL_MAX_CLASSES; ++k)
+    if (k < K && z[k] > zmax) { zmax = z[k]; arg = k; }
+  float s = 0.f;
+#pragma unroll
+  for (int k = 0; k < SLCL_MAX_CLASSES; ++k)
+    if (k < K) { z[k] = expf(z[k] - zmax); s += z[k]; }
+#pragma unroll
+  for (int k = 0; k < SLCL_MAX_CLASSES; ++k)
+    if (k < K) z[k] = z[k] / s;
+  pmax = 1.f / s;
+}
+
 // Weight row(s) of VEC pixels starting at image b, pixel p (flat index pix).
 // Hard labels: utils_.py:581 / :535.  Soft: :517-519 (weighted) or :524-525
-// (arg-max one-hot); certainty :511-514; partitions: SURVEY.md 8(c)-2.
-template <int KWT, int VEC>
+// (arg-max one-hot); certainty :511-514; partitions: SURVEY.md 8(c)-2.  LOGITS: `probs` holds logits, softmax first.
+template <int KWT, int VEC, bool LOGITS = false>
 __device__ __forceinline__ void build_weights(const SumArgs& a, int64_t b, int64_t p, int64_t pix, float (&w)[VEC][KWT]) {
 #pragma unroll
   for (int v = 0; v < VEC; ++v)
@@ -121,9 +141,18 @@ __device__ __forceinline__ void build_weights(const SumArgs& a, int64_t b, int64
   for (int v = 0; v < VEC; ++v) {
     float best = -INFINITY;
     int arg = 0;
+    if constexpr (LOGITS) {
+      float z[SLCL_MAX_CLASSES];
 #pragma unroll
-    for (int k = 0; k < SLCL_MAX_CLASSES; ++k) {
-      if (k < a.n_class && pr[k][v] > best) { best = pr[k][v]; arg = k; }
+      for (int k = 0; k < SLCL_MAX_CLASSES; ++k) z[k] = (k < a.n_class) ? pr[k][v] : 0.f;
+      softmax_inplace(z, a.n_class, best, arg);
+#pragma unroll
+      for (int k = 0; k < SLCL_MAX_CLASSES; ++k) pr[k][v] = z[k];
+    } else {
+#pragma unroll
+      for (int k = 0; k < SLCL_MAX_CLASSES; ++k) {
+        if (k < a.n_class && pr[k][v] > best) { best = pr[k][v]; arg = k; }
+      }
     }
     float cert = (a.threshold > 0.f && a.threshold < 1.f) ? ((best >= a.threshold) ? 1.f : 0.f) : 1.f;
     bool ok = part[v] >= 0 && part[v] < a.n_part;
@@ -145,7 +174,7 @@ __device__ __forceinline__ void build_weights(const SumArgs& a, int64_t b, int64
 // 128-bit shared loads.  The weights therefore cost registers only transiently, whatever P*K is.
 constexpr int kChunks = 8;
 
-template <int KWT, int CPW, int VEC>
+template <int KWT, int CPW, int VEC, bool LOGITS>
 __global__ void __launch_bounds__(kThreads, 2) class_sums_kernel(const SumArgs a) {
   constexpr bool kPipe = KWT <= 8;       // wide weight rows: keep one x buffer, the accumulators need the registers
   extern __shared__ __align__(16) float sW[];            // [KWT][TP]
@@ -180,7 +209,7 @@ __global__ void __launch_bounds__(kThreads, 2) class_sums_kernel(const SumArgs a
         const int pl = v * kThreads + threadIdx.x;
         const int64_t p = p_tile + pl;
         float w1[1][KWT];
-        if (p < a.pixels) build_weights<KWT, 1>(a, b, p, b * a.pixels + p, w1);
+        if (p < a.pixels) build_weights<KWT, 1, LOGITS>(a, b, p, b * a.pixels + p, w1);
         else {
 #pragma unroll
           for (int q = 0; q < KWT; ++q) w1[0][q] = 0.f;
@@ -449,7 +478,7 @@ struct __align__(8) V3Bars { uint64_t x_full[kV3MaxStages], r_full[kV3MaxStages]
 __host__ __device__ constexpr int v3_raw_rows(int kwt) { return kwt < 2 ? 2 : kwt; }
 
 // NCW = upper bound of the consumer warps (8 or 16), NBW = builder warps: together they set the register budget.
-template <int KWT, int CPW, int NCW, int NBW>
+template <int KWT, int CPW, int NCW, int NBW, bool LOGITS>
 __global__ void __launch_bounds__(32 * (3 + NBW + NCW), 1)
 class_sums_v3_kernel(const __grid_constant__ CUtensorMap map_feat, const __grid_constant__ CUtensorMap map_raw,
                      const SumArgs a) {
@@ -580,7 +609,11 @@ class_sums_v3_kernel(const __grid_constant__ CUtensorMap map_feat, const __grid_
           for (int k = 0; k < SLCL_MAX_CLASSES; ++k) pr[k] = (k < a.n_class) ? v3_lds32(raw + (uint32_t)((k * kV3Px + px) * 4)) : 0.f;
           float cert = 1.f;
           int arg = 0;
-          if (use_thr || !a.weighted) {
+          if constexpr (LOGITS) {          // logits -> probabilities (SLCL_SOFT_LOGITS); the largest one is 1/s
+            float pmax;
+            softmax_inplace(pr, a.n_class, pmax, arg);
+            if (use_thr) cert = pmax >= a.threshold ? 1.f : 0.f;
+          } else if (use_thr || !a.weighted) {
             float best = -INFINITY;
 #pragma unroll
             for (int k = 0; k < SLCL_MAX_CLASSES; ++k)
@@ -1087,7 +1120,7 @@ __global__ void __launch_bounds__(kThreads) centroid_bwd_prep_kernel(const float
 template <int KWT> constexpr int kwpad() { return (KWT + 3) / 4 * 4; }
 constexpr int kCenRing = 8;         // channels in flight per thread in the centroid backward (cp.async ring; a power of two)
 
-template <int KWT, int VEC, bool HAS_DP>
+template <int KWT, int VEC, bool HAS_DP, bool LOGITS>
 __global__ void __launch_bounds__(kThreads) centroid_bwd_kernel(const CenBwdArgs a) {
   constexpr int KP = kwpad<KWT>();
   extern __shared__ __align__(16) float sG[];        // [C][KP]
@@ -1104,7 +1137,7 @@ __global__ void __launch_bounds__(kThreads) centroid_bwd_kernel(const CenBwdArgs
   const int64_t p = (g - b * groups) * VEC;
   const int64_t pix = b * a.s.pixels + p;
   float w[VEC][KWT];
-  build_weights<KWT, VEC>(a.s, b, p, pix, w);
+  build_weights<KWT, VEC, LOGITS>(a.s, b, p, pix, w);
   const float* src = a.s.feat + b * a.s.sb + p * a.s.sp;
   float* dst = a.dfeat + b * a.s.sb + p * a.s.sp;
   float dot[HAS_DP ? KWT : 1][VEC];
@@ -1166,7 +1199,39 @@ __global__ void __launch_bounds__(kThreads) centroid_bwd_kernel(const CenBwdArgs
       }
     }
   }
-  if constexpr (HAS_DP) {
+  if constexpr (HAS_DP && LOGITS) {
+    // d z_ik = p_ik * (g_ik - sum_m p_im g_im),  g_ik = cert_i * (x_i.gc_j - mu_j.gc_j),  j = part_i*K + k.  The weight row
+    // holds p_ik * cert_i in the pixel's K columns and zeros elsewhere, so with S_i = sum_j w_ij (x_i.gc_j - mu_j.gc_j) over
+    // every column, column j of the pixel's partition gives w_ij (x_i.gc_j - mu_j.gc_j - S_i) = d z_ik, certainty included.
+    const int K = a.s.n_class;
+    int part[VEC];
+    float S[VEC];
+#pragma unroll
+    for (int v = 0; v < VEC; ++v) {
+      part[v] = a.s.part_id ? a.s.part_id[pix + v] : 0;
+      S[v] = 0.f;
+#pragma unroll
+      for (int j = 0; j < KWT; ++j) {
+        dot[j][v] -= (j < a.s.n_cols) ? a.mu_dot_gc[j] : 0.f;
+        S[v] = fmaf(w[v][j], dot[j][v], S[v]);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < SLCL_MAX_CLASSES; ++k) {
+      if (k < K) {
+        float o[VEC];
+#pragma unroll
+        for (int v = 0; v < VEC; ++v) {
+          const int col = part[v] * K + k;
+          float val = 0.f;
+#pragma unroll
+          for (int j = 0; j < KWT; ++j) val = (j == col) ? w[v][j] * (dot[j][v] - S[v]) : val;
+          o[v] = val;
+        }
+        st_vec<VEC>(a.dprobs + (b * K + k) * a.s.pixels + p, o);
+      }
+    }
+  } else if constexpr (HAS_DP) {
     // d w_ij / d p_ik = cert_i * [part_i == j / K]  (weighted soft labels only)
     const int K = a.s.n_class;
     const bool use_thr = a.s.threshold > 0.f && a.s.threshold < 1.f;
@@ -1240,7 +1305,7 @@ __device__ __forceinline__ float2 cb_unpack(unsigned long long v) {
   return r;
 }
 
-template <int KWT, bool HAS_DP>
+template <int KWT, bool HAS_DP, bool LOGITS>
 __global__ void __launch_bounds__(kThreads, 2) centroid_bwd4_kernel(const CenBwdArgs a) {
   constexpr int KP = (KWT + 1) / 2 * 2;               // gc pairs are fetched two columns (one LDS.128) at a time
   extern __shared__ __align__(16) float cb_smem[];    // sG2 [C][KP] {g, g} pairs | scratch [KWT][threads] float4 | x ring
@@ -1300,7 +1365,15 @@ __global__ void __launch_bounds__(kThreads, 2) centroid_bwd4_kernel(const CenBwd
 #pragma unroll
       for (int v = 0; v < 4; ++v) {
         int arg = 0;
-        if (use_thr || !a.s.weighted) {
+        if constexpr (LOGITS) {        // logits -> probabilities (SLCL_SOFT_LOGITS); the largest one is 1/s
+          float z[SLCL_MAX_CLASSES], pmax;
+#pragma unroll
+          for (int k = 0; k < SLCL_MAX_CLASSES; ++k) z[k] = (k < K) ? pr[k][v] : 0.f;
+          softmax_inplace(z, K, pmax, arg);
+#pragma unroll
+          for (int k = 0; k < SLCL_MAX_CLASSES; ++k) pr[k][v] = z[k];
+          if (use_thr && !(pmax >= a.s.threshold)) cert[v] = 0.f;
+        } else if (use_thr || !a.s.weighted) {
           float best = -INFINITY;
 #pragma unroll
           for (int k = 0; k < SLCL_MAX_CLASSES; ++k)
@@ -1349,7 +1422,42 @@ __global__ void __launch_bounds__(kThreads, 2) centroid_bwd4_kernel(const CenBwd
     const float2 oa = cb_unpack(o01), ob = cb_unpack(o23);
     st_stream4(dst + (int64_t)c * a.s.sc, make_float4(oa.x, oa.y, ob.x, ob.y));
   }
-  if constexpr (HAS_DP) {
+  if constexpr (HAS_DP && LOGITS) {
+    // d z[b,k,p] = p_k * (g_k - sum_m p_m g_m), g_k = cert * (x . gc_j - mu_j . gc_j), j = part*K + k.  The weight row
+    // (still in the scratch) holds p_k * cert in the pixel's K columns and zeros elsewhere: with S = sum_j w_j (x . gc_j -
+    // mu_j . gc_j) over every column, replace w_j by w_j (x . gc_j - mu_j . gc_j - S) and gather columns part*K + k by
+    // address as below.  The weights come back from shared memory, so w01 / w23 need not live past the channel loop.
+    float S[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int j = 0; j < KWT; ++j) {
+      const float m = (j < a.s.n_cols) ? a.mu_dot_gc[j] : 0.f;
+      const float2 da = cb_unpack(d01[j]), db = cb_unpack(d23[j]);
+      unsigned long long wlo, whi;
+      cb_lds2x64(scratch + (uint32_t)(j * kThreads * 16), wlo, whi);
+      const float2 wa = cb_unpack(wlo), wb = cb_unpack(whi);
+      S[0] = fmaf(wa.x, da.x - m, S[0]); S[1] = fmaf(wa.y, da.y - m, S[1]);
+      S[2] = fmaf(wb.x, db.x - m, S[2]); S[3] = fmaf(wb.y, db.y - m, S[3]);
+    }
+#pragma unroll
+    for (int j = 0; j < KWT; ++j) {
+      const float m = (j < a.s.n_cols) ? a.mu_dot_gc[j] : 0.f;
+      const float2 da = cb_unpack(d01[j]), db = cb_unpack(d23[j]);
+      unsigned long long wlo, whi;
+      cb_lds2x64(scratch + (uint32_t)(j * kThreads * 16), wlo, whi);
+      const float2 wa = cb_unpack(wlo), wb = cb_unpack(whi);
+      cb_sts128(scratch + (uint32_t)(j * kThreads * 16), make_float4(wa.x * (da.x - m - S[0]), wa.y * (da.y - m - S[1]),
+                                                                     wb.x * (db.x - m - S[2]), wb.y * (db.y - m - S[3])));
+    }
+#pragma unroll
+    for (int k = 0; k < SLCL_MAX_CLASSES; ++k) {
+      if (k < K) {
+        float o[4];
+#pragma unroll
+        for (int v = 0; v < 4; ++v) o[v] = base[v] >= 0 ? cb_lds32(scratch + (uint32_t)((base[v] + k) * kThreads * 16 + v * 4)) : 0.f;
+        st_stream4(a.dprobs + (b * K + k) * a.s.pixels + p, make_float4(o[0], o[1], o[2], o[3]));
+      }
+    }
+  } else if constexpr (HAS_DP) {
     // d probs[b,k,p] = cert * (x . gc_j - mu_j . gc_j), j = part*K + k: park the KWT dot rows in the scratch, gather by address
 #pragma unroll
     for (int j = 0; j < KWT; ++j) {
@@ -1405,14 +1513,15 @@ size_t partial_bytes(const SumPlan& p, int64_t C) {
   return align_up((size_t)p.grid.x * p.kwt * (C + 1) * sizeof(float), 256);
 }
 
-template <int KWT, int CPW>
+template <int KWT, int CPW, bool LOGITS>
 void launch_sums(const SumArgs& a, const SumPlan& p, cudaStream_t stream) {
   const size_t smem = (size_t)KWT * kChunks * 32 * p.vec * sizeof(float);
   if (p.vec == 4) {
-    if (smem > 32 * 1024) cudaFuncSetAttribute(class_sums_kernel<KWT, CPW, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    class_sums_kernel<KWT, CPW, 4><<<p.grid, kThreads, smem, stream>>>(a);
+    if (smem > 32 * 1024)
+      cudaFuncSetAttribute(class_sums_kernel<KWT, CPW, 4, LOGITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    class_sums_kernel<KWT, CPW, 4, LOGITS><<<p.grid, kThreads, smem, stream>>>(a);
   } else {
-    class_sums_kernel<KWT, CPW, 1><<<p.grid, kThreads, smem, stream>>>(a);
+    class_sums_kernel<KWT, CPW, 1, LOGITS><<<p.grid, kThreads, smem, stream>>>(a);
   }
 }
 
@@ -1496,7 +1605,7 @@ int v3_encode(CUtensorMap* map, const void* base, const cuuint64_t (&dims)[3], c
   return SLCL_OK;
 }
 
-template <int KWT, int CPW, int NCW, int NBW>
+template <int KWT, int CPW, int NCW, int NBW, bool LOGITS>
 int launch_v3(const SumArgs& a, const V3Plan& p, cudaStream_t stream) {
   ensure_context_on_this_thread();
   CUtensorMap map, map_raw;
@@ -1508,7 +1617,7 @@ int launch_v3(const SumArgs& a, const V3Plan& p, cudaStream_t stream) {
     if (st != SLCL_OK) return st;
   }
   map_raw = map;
-  if (a.mode == kSoft) {              // probs [B, K, HW]: box = all K probability rows of 128 pixels of one image
+  if (a.mode == kSoft) {              // probs (or logits) [B, K, HW]: box = all K rows of 128 pixels of one image
     const cuuint64_t dims[3] = {(cuuint64_t)a.pixels, (cuuint64_t)a.n_class, (cuuint64_t)a.batch};
     const cuuint64_t strides[2] = {(cuuint64_t)a.pixels * 4, (cuuint64_t)a.pixels * a.n_class * 4};
     const cuuint32_t box[3] = {(cuuint32_t)kV3Px, (cuuint32_t)a.n_class, 1};
@@ -1525,7 +1634,7 @@ int launch_v3(const SumArgs& a, const V3Plan& p, cudaStream_t stream) {
   static bool attr_set_dev[64] = {};          // function attributes are per device
   bool& attr_set = attr_set_dev[current_device_slot()];
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(class_sums_v3_kernel<KWT, CPW, NCW, NBW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(class_sums_v3_kernel<KWT, CPW, NCW, NBW, LOGITS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          220 * 1024);
     if (e != cudaSuccess) { set_cuda_error(e, "cudaFuncSetAttribute(class_sums_v3_kernel)"); return SLCL_ERR_CUDA; }
     attr_set = true;
@@ -1534,17 +1643,17 @@ int launch_v3(const SumArgs& a, const V3Plan& p, cudaStream_t stream) {
   av.n_cw = p.n_cw;
   av.n_stages = v3_stages(KWT, CPW, p.n_cw, NBW / 2);
   if (smem > 220 * 1024) return SLCL_ERR_UNSUPPORTED;
-  class_sums_v3_kernel<KWT, CPW, NCW, NBW><<<p.grid, 32 * (3 + NBW + p.n_cw), smem, stream>>>(map, map_raw, av);
+  class_sums_v3_kernel<KWT, CPW, NCW, NBW, LOGITS><<<p.grid, 32 * (3 + NBW + p.n_cw), smem, stream>>>(map, map_raw, av);
   return SLCL_OK;
 }
 
-template <int KWT>
+template <int KWT, bool LOGITS>
 int launch_v3_cpw(const SumArgs& a, const V3Plan& p, cudaStream_t stream) {
   constexpr int CPW = v3_cpw(KWT);
   if constexpr (v3_ncw(KWT) > 8) {
-    if (p.n_cw > 8) return launch_v3<KWT, CPW, 16, v3_nbw(16, KWT)>(a, p, stream);
+    if (p.n_cw > 8) return launch_v3<KWT, CPW, 16, v3_nbw(16, KWT), LOGITS>(a, p, stream);
   }
-  return launch_v3<KWT, CPW, 8, v3_nbw(8, KWT)>(a, p, stream);
+  return launch_v3<KWT, CPW, 8, v3_nbw(8, KWT), LOGITS>(a, p, stream);
 }
 
 void launch_reduce(const SumArgs& a, int n_blocks, int kwt, double* sums, const slcl_peer_t* peer, const FinArgs& fin,
@@ -1559,9 +1668,10 @@ void launch_reduce(const SumArgs& a, int n_blocks, int kwt, double* sums, const 
                                                                     PeerCtx{}, fin, a.ticket);
 }
 
-// sweep + reduce (+ cross-rank exchange through `peer`, + finaliser `fin` in the reduce kernel's last block)
+// sweep + reduce (+ cross-rank exchange through `peer`, + finaliser `fin` in the reduce kernel's last block).
+// logits: soft mode with logits in a.probs (the sweep applies the softmax).
 int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t workspace_bytes, cudaStream_t stream,
-                   const slcl_peer_t* peer = nullptr, FinArgs fin = FinArgs{}) {
+                   const slcl_peer_t* peer = nullptr, FinArgs fin = FinArgs{}, bool logits = false) {
   if (a.n_cols < 1 || a.n_cols > SLCL_MAX_WEIGHT_COLS) return SLCL_ERR_INVALID_ARGUMENT;
   if (peer != nullptr) {
     if (!peer_valid(peer)) return SLCL_ERR_INVALID_ARGUMENT;
@@ -1578,15 +1688,15 @@ int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t w
     a.partial = reinterpret_cast<float*>(workspace);
     int st;
     switch (v3.kwt) {
-      case 2: st = launch_v3_cpw<2>(a, v3, stream); break;
-      case 3: st = launch_v3_cpw<3>(a, v3, stream); break;
-      case 4: st = launch_v3_cpw<4>(a, v3, stream); break;
-      case 5: st = launch_v3_cpw<5>(a, v3, stream); break;
-      case 6: st = launch_v3_cpw<6>(a, v3, stream); break;
-      case 8: st = launch_v3_cpw<8>(a, v3, stream); break;
-      case 10: st = launch_v3_cpw<10>(a, v3, stream); break;
-      case 12: st = launch_v3_cpw<12>(a, v3, stream); break;
-      case 16: st = launch_v3_cpw<16>(a, v3, stream); break;
+      case 2: st = logits ? launch_v3_cpw<2, true>(a, v3, stream) : launch_v3_cpw<2, false>(a, v3, stream); break;
+      case 3: st = logits ? launch_v3_cpw<3, true>(a, v3, stream) : launch_v3_cpw<3, false>(a, v3, stream); break;
+      case 4: st = logits ? launch_v3_cpw<4, true>(a, v3, stream) : launch_v3_cpw<4, false>(a, v3, stream); break;
+      case 5: st = logits ? launch_v3_cpw<5, true>(a, v3, stream) : launch_v3_cpw<5, false>(a, v3, stream); break;
+      case 6: st = logits ? launch_v3_cpw<6, true>(a, v3, stream) : launch_v3_cpw<6, false>(a, v3, stream); break;
+      case 8: st = logits ? launch_v3_cpw<8, true>(a, v3, stream) : launch_v3_cpw<8, false>(a, v3, stream); break;
+      case 10: st = logits ? launch_v3_cpw<10, true>(a, v3, stream) : launch_v3_cpw<10, false>(a, v3, stream); break;
+      case 12: st = logits ? launch_v3_cpw<12, true>(a, v3, stream) : launch_v3_cpw<12, false>(a, v3, stream); break;
+      case 16: st = logits ? launch_v3_cpw<16, true>(a, v3, stream) : launch_v3_cpw<16, false>(a, v3, stream); break;
       default: return SLCL_ERR_INVALID_ARGUMENT;
     }
     if (st != SLCL_OK) return st;
@@ -1597,15 +1707,15 @@ int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t w
   a.cg_per_block = p.cg_per_block; a.pt_per_block = p.pt_per_block;
   a.partial = reinterpret_cast<float*>(workspace);
   switch (p.kwt) {
-    case 2: launch_sums<2, 8>(a, p, stream); break;
-    case 3: launch_sums<3, 8>(a, p, stream); break;
-    case 4: launch_sums<4, 4>(a, p, stream); break;
-    case 5: launch_sums<5, 4>(a, p, stream); break;
-    case 6: launch_sums<6, 4>(a, p, stream); break;
-    case 8: launch_sums<8, 4>(a, p, stream); break;
-    case 10: launch_sums<10, 4>(a, p, stream); break;
-    case 12: launch_sums<12, 4>(a, p, stream); break;
-    case 16: launch_sums<16, 4>(a, p, stream); break;
+    case 2: logits ? launch_sums<2, 8, true>(a, p, stream) : launch_sums<2, 8, false>(a, p, stream); break;
+    case 3: logits ? launch_sums<3, 8, true>(a, p, stream) : launch_sums<3, 8, false>(a, p, stream); break;
+    case 4: logits ? launch_sums<4, 4, true>(a, p, stream) : launch_sums<4, 4, false>(a, p, stream); break;
+    case 5: logits ? launch_sums<5, 4, true>(a, p, stream) : launch_sums<5, 4, false>(a, p, stream); break;
+    case 6: logits ? launch_sums<6, 4, true>(a, p, stream) : launch_sums<6, 4, false>(a, p, stream); break;
+    case 8: logits ? launch_sums<8, 4, true>(a, p, stream) : launch_sums<8, 4, false>(a, p, stream); break;
+    case 10: logits ? launch_sums<10, 4, true>(a, p, stream) : launch_sums<10, 4, false>(a, p, stream); break;
+    case 12: logits ? launch_sums<12, 4, true>(a, p, stream) : launch_sums<12, 4, false>(a, p, stream); break;
+    case 16: logits ? launch_sums<16, 4, true>(a, p, stream) : launch_sums<16, 4, false>(a, p, stream); break;
     default: return SLCL_ERR_INVALID_ARGUMENT;
   }
   launch_reduce(a, (int)p.grid.x, p.kwt, sums, peer, fin, stream);
@@ -1617,6 +1727,13 @@ bool nchw_vec4(const float* feat, int64_t C, int64_t HW, std::initializer_list<c
   for (const void* q : ptrs) ok = ok && (q == nullptr || aligned16(q));
   (void)feat; (void)C;
   return ok;
+}
+
+// `weighted` of the soft-label entry points is a flags word: SLCL_SOFT_WEIGHTED | SLCL_SOFT_LOGITS, the latter for soft
+// labels only.
+bool soft_flags_ok(int flags, const int64_t* labels) {
+  if (flags & ~(SLCL_SOFT_WEIGHTED | SLCL_SOFT_LOGITS)) return false;
+  return !((flags & SLCL_SOFT_LOGITS) && labels != nullptr);
 }
 
 }  // namespace
@@ -1655,7 +1772,7 @@ extern "C" int slcl_class_sums(const float* feat, int64_t batch, int64_t channel
                                const int32_t* part_id, int n_partitions, int n_class, double* sums, void* workspace,
                                size_t workspace_bytes, slcl_stream_t stream_) {
   if (!feat || batch <= 0 || channels <= 0 || pixels <= 0 || !sums || !workspace) return SLCL_ERR_INVALID_ARGUMENT;
-  if ((labels == nullptr) == (probs == nullptr)) return SLCL_ERR_INVALID_ARGUMENT;
+  if ((labels == nullptr) == (probs == nullptr) || !soft_flags_ok(weighted, labels)) return SLCL_ERR_INVALID_ARGUMENT;
   if (n_class < 1 || n_class > kMaxK || n_partitions < 1 || n_partitions * n_class > SLCL_MAX_WEIGHT_COLS)
     return SLCL_ERR_INVALID_ARGUMENT;
   if (n_partitions > 1 && part_id == nullptr) return SLCL_ERR_INVALID_ARGUMENT;
@@ -1664,11 +1781,12 @@ extern "C" int slcl_class_sums(const float* feat, int64_t batch, int64_t channel
   a.batch = batch; a.channels = channels; a.pixels = pixels;
   a.sb = channels * pixels; a.sc = pixels; a.sp = 1;
   a.mode = labels ? kHard : kSoft;
-  a.labels = labels; a.probs = probs; a.weighted = weighted; a.threshold = threshold;
+  a.labels = labels; a.probs = probs; a.weighted = weighted & SLCL_SOFT_WEIGHTED; a.threshold = threshold;
   a.part_id = part_id; a.n_part = n_partitions; a.n_class = n_class;
   a.n_cols = n_partitions * n_class;
   bool vec4 = nchw_vec4(feat, channels, pixels, {feat, labels, probs, part_id});
-  return run_class_sums(a, vec4, sums, workspace, workspace_bytes, (cudaStream_t)stream_);
+  return run_class_sums(a, vec4, sums, workspace, workspace_bytes, (cudaStream_t)stream_, nullptr, FinArgs{},
+                        (weighted & SLCL_SOFT_LOGITS) != 0);
 }
 
 extern "C" int slcl_class_centres_update(const float* feat, int64_t batch, int64_t channels, int64_t pixels,
@@ -1696,7 +1814,7 @@ extern "C" int slcl_centroids_fwd(const float* feat, int64_t batch, int64_t chan
                                   slcl_stream_t stream_) {
   if (!feat || batch <= 0 || channels <= 0 || pixels <= 0 || !centroids || !inv_weight || !sums || !workspace)
     return SLCL_ERR_INVALID_ARGUMENT;
-  if ((labels == nullptr) == (probs == nullptr)) return SLCL_ERR_INVALID_ARGUMENT;
+  if ((labels == nullptr) == (probs == nullptr) || !soft_flags_ok(weighted, labels)) return SLCL_ERR_INVALID_ARGUMENT;
   if (n_class < 1 || n_class > kMaxK || n_partitions < 1 || n_partitions * n_class > SLCL_MAX_WEIGHT_COLS)
     return SLCL_ERR_INVALID_ARGUMENT;
   if (n_partitions > 1 && part_id == nullptr) return SLCL_ERR_INVALID_ARGUMENT;
@@ -1705,12 +1823,13 @@ extern "C" int slcl_centroids_fwd(const float* feat, int64_t batch, int64_t chan
   a.batch = batch; a.channels = channels; a.pixels = pixels;
   a.sb = channels * pixels; a.sc = pixels; a.sp = 1;
   a.mode = labels ? kHard : kSoft;
-  a.labels = labels; a.probs = probs; a.weighted = weighted; a.threshold = threshold;
+  a.labels = labels; a.probs = probs; a.weighted = weighted & SLCL_SOFT_WEIGHTED; a.threshold = threshold;
   a.part_id = part_id; a.n_part = n_partitions; a.n_class = n_class;
   a.n_cols = n_partitions * n_class;
   const bool vec4 = nchw_vec4(feat, channels, pixels, {feat, labels, probs, part_id});
   FinArgs fin{kFinCentroid, previous, momentum, n_class, centroids, inv_weight};
-  return run_class_sums(a, vec4, sums, workspace, workspace_bytes, (cudaStream_t)stream_, peer, fin);
+  return run_class_sums(a, vec4, sums, workspace, workspace_bytes, (cudaStream_t)stream_, peer, fin,
+                        (weighted & SLCL_SOFT_LOGITS) != 0);
 }
 
 namespace slcl {
@@ -1870,11 +1989,12 @@ extern "C" int slcl_centroid_bwd(const float* feat, int64_t batch, int64_t chann
                                  size_t workspace_bytes, slcl_stream_t stream_) {
   if (!feat || batch <= 0 || channels <= 0 || pixels <= 0 || !grad_centroids || !sums || !dfeat || !workspace)
     return SLCL_ERR_INVALID_ARGUMENT;
-  if ((labels == nullptr) == (probs == nullptr)) return SLCL_ERR_INVALID_ARGUMENT;
+  if ((labels == nullptr) == (probs == nullptr) || !soft_flags_ok(weighted, labels)) return SLCL_ERR_INVALID_ARGUMENT;
   if (n_class < 1 || n_class > kMaxK || n_partitions < 1 || n_partitions * n_class > SLCL_MAX_WEIGHT_COLS)
     return SLCL_ERR_INVALID_ARGUMENT;
   if (n_partitions > 1 && part_id == nullptr) return SLCL_ERR_INVALID_ARGUMENT;
-  if (dprobs != nullptr && (probs == nullptr || !weighted)) return SLCL_ERR_INVALID_ARGUMENT;
+  if (dprobs != nullptr && (probs == nullptr || !(weighted & SLCL_SOFT_WEIGHTED))) return SLCL_ERR_INVALID_ARGUMENT;
+  const bool logits = (weighted & SLCL_SOFT_LOGITS) != 0;
   const int n_cols = n_partitions * n_class;
   if (workspace_bytes < slcl_centroid_bwd_workspace_bytes(channels, n_cols) || !aligned16(workspace))
     return SLCL_ERR_WORKSPACE;
@@ -1887,7 +2007,7 @@ extern "C" int slcl_centroid_bwd(const float* feat, int64_t batch, int64_t chann
   a.s.batch = batch; a.s.channels = channels; a.s.pixels = pixels;
   a.s.sb = channels * pixels; a.s.sc = pixels; a.s.sp = 1;
   a.s.mode = labels ? kHard : kSoft;
-  a.s.labels = labels; a.s.probs = probs; a.s.weighted = weighted; a.s.threshold = threshold;
+  a.s.labels = labels; a.s.probs = probs; a.s.weighted = weighted & SLCL_SOFT_WEIGHTED; a.s.threshold = threshold;
   a.s.part_id = part_id; a.s.n_part = n_partitions; a.s.n_class = n_class;
   a.s.n_cols = n_partitions * n_class;
   a.gc = gc; a.mu_dot_gc = mu_dot_gc; a.dfeat = dfeat; a.dprobs = dprobs;
@@ -1913,8 +2033,14 @@ extern "C" int slcl_centroid_bwd(const float* feat, int64_t batch, int64_t chann
       return SLCL_OK;                                                                                         \
     };                                                                                                        \
     int st;                                                                                                   \
-    if (dprobs) st = vec4 ? launch(centroid_bwd4_kernel<KW_, true>) : launch(centroid_bwd_kernel<KW_, 1, true>);      \
-    else st = vec4 ? launch(centroid_bwd4_kernel<KW_, false>) : launch(centroid_bwd_kernel<KW_, 1, false>);           \
+    if (logits) {                                                                                             \
+      if (dprobs) st = vec4 ? launch(centroid_bwd4_kernel<KW_, true, true>) : launch(centroid_bwd_kernel<KW_, 1, true, true>); \
+      else st = vec4 ? launch(centroid_bwd4_kernel<KW_, false, true>) : launch(centroid_bwd_kernel<KW_, 1, false, true>); \
+    } else if (dprobs) {                                                                                      \
+      st = vec4 ? launch(centroid_bwd4_kernel<KW_, true, false>) : launch(centroid_bwd_kernel<KW_, 1, true, false>); \
+    } else {                                                                                                  \
+      st = vec4 ? launch(centroid_bwd4_kernel<KW_, false, false>) : launch(centroid_bwd_kernel<KW_, 1, false, false>); \
+    }                                                                                                         \
     if (st != SLCL_OK) return st;                                                                             \
   } break;
   switch (kwt) {

@@ -176,53 +176,57 @@ def proto_loss(feat: Tensor, labels: Optional[Tensor], soft_mask: Optional[Tenso
 class _Centroids(torch.autograd.Function):
     """cal_centroid (reference utils/utils_.py:479-565, repaired; partitions per
     SURVEY.md 8(c)-2).  Forward = class sums (+ optional cross-rank all-reduce)
-    + finalise; backward = appendix A.4."""
+    + finalise; backward = appendix A.4.  from_logits: ``probs`` holds logits, the kernels apply the softmax and the
+    backward returns dL/dlogits in its slot."""
 
     @staticmethod
-    def forward(ctx, feat, labels, probs, previous, weighted, threshold, part_id, n_partitions, n_class, momentum, group):
+    def forward(ctx, feat, labels, probs, previous, weighted, threshold, part_id, n_partitions, n_class, momentum, group,
+                from_logits):
         from .peer import PeerMailbox
         prev = None if previous is None else previous.detach()
         if group is None or isinstance(group, PeerMailbox):
             # two launches: sweep, then reduce [+ exchange over the NVLink peer mailboxes] + finalise
             peer = group.args() if group is not None else ()
             cen, _inv_w, sums = _ops.centroids_fwd(feat.detach(), labels, None if probs is None else probs.detach(), weighted,
-                                                   threshold, part_id, n_partitions, n_class, prev, momentum, *peer)
+                                                   threshold, part_id, n_partitions, n_class, prev, momentum, *peer,
+                                                   from_logits=from_logits)
         else:
             from .distributed import all_reduce_sums
             sums = _ops.class_sums(feat.detach(), labels, None if probs is None else probs.detach(), weighted, threshold,
-                                   part_id, n_partitions, n_class)
+                                   part_id, n_partitions, n_class, from_logits)
             sums = all_reduce_sums(sums, group)
             cen, _inv_w = _ops.centroid_finalize(sums, prev, momentum, n_partitions, n_class)
         ctx.save_for_backward(feat, labels, probs, part_id, sums)
-        ctx.cfg = (weighted, threshold, n_partitions, n_class, momentum, previous is not None)
+        ctx.cfg = (weighted, threshold, n_partitions, n_class, momentum, previous is not None, from_logits)
         return cen
 
     @staticmethod
     def backward(ctx, grad_cen):
         feat, labels, probs, part_id, sums = ctx.saved_tensors
-        weighted, threshold, n_partitions, n_class, momentum, has_prev = ctx.cfg
+        weighted, threshold, n_partitions, n_class, momentum, has_prev, from_logits = ctx.cfg
         ema_scale = (1.0 - momentum) if has_prev else 1.0
         dfeat = dprobs = dprev = None
         need_dp = probs is not None and ctx.needs_input_grad[2] and weighted
         if ctx.needs_input_grad[0] or need_dp:
             dfeat, dp = _ops.centroid_bwd(feat.detach(), labels, None if probs is None else probs.detach(), weighted,
                                           threshold, part_id, n_partitions, n_class, grad_cen.contiguous(), sums,
-                                          ema_scale, need_dp)
+                                          ema_scale, need_dp, from_logits)
             if need_dp:
                 dprobs = dp
             if not ctx.needs_input_grad[0]:
                 dfeat = None
         if has_prev and ctx.needs_input_grad[3]:
             dprev = momentum * grad_cen.reshape(n_partitions, n_class, -1).sum(0)
-        return dfeat, None, dprobs, dprev, None, None, None, None, None, None, None
+        return dfeat, None, dprobs, dprev, None, None, None, None, None, None, None, None
 
 
 def centroids(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor], previous: Optional[Tensor], *,
               weighted: bool, threshold: float, part_id: Optional[Tensor], n_partitions: int, n_class: int,
-              momentum: float, group=None) -> Tensor:
-    """-> [P*K, C] centroids (EMA'd with `previous` when given)."""
+              momentum: float, group=None, from_logits: bool = False) -> Tensor:
+    """-> [P*K, C] centroids (EMA'd with `previous` when given).  ``from_logits``: ``probs`` are the logits whose
+    softmax over dim 1 is the soft label; its gradient is dL/dlogits."""
     return _Centroids.apply(feat, labels, probs, previous, weighted, threshold, part_id, n_partitions, n_class, momentum,
-                            group)
+                            group, bool(from_logits))
 
 
 class _CentroidLoss(torch.autograd.Function):

@@ -399,10 +399,16 @@ def _nchw_contig(feat: Tensor) -> Tensor:
     return feat.contiguous()
 
 
+def _soft_flags(weighted: bool, from_logits: bool) -> int:
+    """The ``weighted`` flags word of the class-sum / centroid entry points (SLCL_SOFT_WEIGHTED, SLCL_SOFT_LOGITS)."""
+    return (1 if weighted else 0) | (2 if from_logits else 0)
+
+
 @torch.library.custom_op("slcl::class_sums", mutates_args=(), device_types="cuda")
 def class_sums(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor], weighted: bool, threshold: float,
-               part_id: Optional[Tensor], n_partitions: int, n_class: int) -> Tensor:
-    """-> sums [P*K, C+1] float64 (weighted feature sums | weight sums)."""
+               part_id: Optional[Tensor], n_partitions: int, n_class: int, from_logits: bool = False) -> Tensor:
+    """-> sums [P*K, C+1] float64 (weighted feature sums | weight sums).  ``from_logits``: ``probs`` holds logits and the
+    weights are built from ``softmax(probs, 1)`` inside the sweep."""
     dev = require_cuda(feat, labels, probs, part_id)
     lib = _lib.load()
     feat = _nchw_contig(feat)
@@ -423,14 +429,15 @@ def class_sums(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor], 
     sums = torch.empty((cols, c + 1), dtype=torch.float64, device=dev)
     ws = _ws(lib.slcl_class_sums_workspace_bytes(b, c, h * w, cols), dev)
     with _guard(dev):
-        st = lib.slcl_class_sums(ptr(feat), b, c, h * w, ptr(labels), ptr(probs), int(weighted), float(threshold),
+        st = lib.slcl_class_sums(ptr(feat), b, c, h * w, ptr(labels), ptr(probs), _soft_flags(weighted, from_logits),
+                                 float(threshold),
                                  ptr(part_id), n_partitions, n_class, ptr(sums), ptr(ws), ws.numel(), stream_ptr(dev))
     check(st, "slcl_class_sums")
     return sums
 
 
 @class_sums.register_fake
-def _(feat, labels, probs, weighted, threshold, part_id, n_partitions, n_class):
+def _(feat, labels, probs, weighted, threshold, part_id, n_partitions, n_class, from_logits=False):
     return torch.empty((n_partitions * n_class, feat.shape[1] + 1), dtype=torch.float64, device=feat.device)
 
 
@@ -471,9 +478,9 @@ def _(feat, labels, old_centres, m, peer_ptrs=0, rank=0, world=1, capacity_words
 def centroids_fwd(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor], weighted: bool, threshold: float,
                   part_id: Optional[Tensor], n_partitions: int, n_class: int, previous: Optional[Tensor], momentum: float,
                   peer_ptrs: int = 0, rank: int = 0, world: int = 1, capacity_words: int = 0,
-                  timeout_s: float = 0.0) -> Tuple[Tensor, Tensor, Tensor]:
+                  timeout_s: float = 0.0, from_logits: bool = False) -> Tuple[Tensor, Tensor, Tensor]:
     """cal_centroid forward as two launches: class sums, then reduce [+ peer all-reduce] + centroid finalise.
-    -> (centroids [P*K, C], inv_weight [P*K], sums [P*K, C+1] float64)."""
+    -> (centroids [P*K, C], inv_weight [P*K], sums [P*K, C+1] float64).  ``from_logits``: as for class_sums."""
     dev = require_cuda(feat, labels, probs, part_id, previous)
     lib = _lib.load()
     feat = _nchw_contig(feat)
@@ -501,7 +508,8 @@ def centroids_fwd(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor
     ws = _ws(lib.slcl_class_sums_workspace_bytes(b, c, h * w, cols), dev)
     peer = _peer(peer_ptrs, rank, world, capacity_words, timeout_s)
     with _guard(dev):
-        st = lib.slcl_centroids_fwd(ptr(feat), b, c, h * w, ptr(labels), ptr(probs), int(weighted), float(threshold),
+        st = lib.slcl_centroids_fwd(ptr(feat), b, c, h * w, ptr(labels), ptr(probs), _soft_flags(weighted, from_logits),
+                                    float(threshold),
                                     ptr(part_id), n_partitions, n_class, ptr(previous), float(momentum), ptr(cen), ptr(inv_w),
                                     ptr(sums), C.byref(peer) if peer is not None else None, ptr(ws), ws.numel(),
                                     stream_ptr(dev))
@@ -511,7 +519,7 @@ def centroids_fwd(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor
 
 @centroids_fwd.register_fake
 def _(feat, labels, probs, weighted, threshold, part_id, n_partitions, n_class, previous, momentum, peer_ptrs=0, rank=0,
-      world=1, capacity_words=0, timeout_s=0.0):
+      world=1, capacity_words=0, timeout_s=0.0, from_logits=False):
     rows, c = n_partitions * n_class, feat.shape[1]
     return (torch.empty((rows, c), dtype=_F32, device=feat.device), torch.empty(rows, dtype=_F32, device=feat.device),
             torch.empty((rows, c + 1), dtype=torch.float64, device=feat.device))
@@ -569,7 +577,9 @@ def _(sums, previous, momentum, n_sets, n_class):
 @torch.library.custom_op("slcl::centroid_bwd", mutates_args=(), device_types="cuda")
 def centroid_bwd(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor], weighted: bool, threshold: float,
                  part_id: Optional[Tensor], n_partitions: int, n_class: int, grad_centroids: Tensor, sums: Tensor,
-                 ema_scale: float, need_dprobs: bool) -> Tuple[Tensor, Tensor]:
+                 ema_scale: float, need_dprobs: bool, from_logits: bool = False) -> Tuple[Tensor, Tensor]:
+    """-> (dL/dfeat, dL/dprobs or an empty tensor).  ``from_logits``: ``probs`` holds logits, and the second output is
+    dL/dlogits through the softmax."""
     dev = require_cuda(feat, labels, probs, part_id, grad_centroids, sums)
     lib = _lib.load()
     feat = _nchw_contig(feat)
@@ -588,7 +598,8 @@ def centroid_bwd(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor]
     dprobs = torch.empty_like(probs) if (need_dprobs and probs is not None) else torch.empty(0, dtype=_F32, device=dev)
     ws = _ws(lib.slcl_centroid_bwd_workspace_bytes(c, cols), dev)
     with _guard(dev):
-        st = lib.slcl_centroid_bwd(ptr(feat), b, c, h * w, ptr(labels), ptr(probs), int(weighted), float(threshold),
+        st = lib.slcl_centroid_bwd(ptr(feat), b, c, h * w, ptr(labels), ptr(probs), _soft_flags(weighted, from_logits),
+                                   float(threshold),
                                    ptr(part_id), n_partitions, n_class, ptr(g), ptr(sums.contiguous()), float(ema_scale),
                                    ptr(dfeat), ptr(dprobs) if dprobs.numel() else None, ptr(ws), ws.numel(),
                                    stream_ptr(dev))
@@ -598,7 +609,7 @@ def centroid_bwd(feat: Tensor, labels: Optional[Tensor], probs: Optional[Tensor]
 
 @centroid_bwd.register_fake
 def _(feat, labels, probs, weighted, threshold, part_id, n_partitions, n_class, grad_centroids, sums, ema_scale,
-      need_dprobs):
+      need_dprobs, from_logits=False):
     dp = torch.empty_like(probs) if (need_dprobs and probs is not None) else feat.new_empty(0)
     return torch.empty_like(feat), dp
 

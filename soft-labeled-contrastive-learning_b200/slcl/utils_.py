@@ -66,7 +66,7 @@ def rmc_partition_ids(n_pixels: int, partition: int, generator: Optional[torch.G
 
 def cal_centroid(decoder_ft, label, previous_centroid=None, momentum=0.95, pseudo_label=False, n_class=4, partition=1,
                  threshold: int = None, thd_w: float = 0.0, weighted_ave=False, epoch=0, max_epoch=1000,
-                 low_thd=0, high_thd=0.99, stdmin=False, part_id=None, generator=None, group=None):
+                 low_thd=0, high_thd=0.99, stdmin=False, part_id=None, generator=None, group=None, from_logits=False):
     """Per-class (soft-label weighted) feature centroids (reference
     utils/utils_.py:479-565, with the repair of SURVEY.md section 0).
 
@@ -75,9 +75,21 @@ def cal_centroid(decoder_ft, label, previous_centroid=None, momentum=0.95, pseud
     too, :565).  ``partition > 1`` returns a list of P ``[K,C]`` tensors (what
     trainer/Trainer_MCCL.py:281-326 consumes); the partition of every pixel
     comes from ``part_id`` or is drawn with ``rmc_partition_ids(generator)``.
-    Extra keywords (``part_id``, ``generator``, ``group``) are additions.
+    Extra keywords (``part_id``, ``generator``, ``group``, ``from_logits``) are additions.
+
+    ``from_logits=True`` takes the segmentor's logits ``[B, K, h, w]`` at the feature map's resolution as ``label`` and
+    returns what ``cal_centroid(decoder_ft, softmax(label, 1), pseudo_label=True, ...)`` returns, gradients included
+    (into the logits), with the softmax done inside the class-sum and backward kernels.  It needs ``pseudo_label=True``.
+    Logits at another resolution: interpolating probabilities does not commute with the softmax, so call ``softmax``
+    and this function without ``from_logits``.
     """
     b, c, h, w = decoder_ft.shape
+    if from_logits:
+        if not pseudo_label:
+            raise ValueError("from_logits=True needs pseudo_label=True (logits are soft labels)")
+        if tuple(label.shape) != (b, n_class, h, w):
+            raise ValueError(f"from_logits=True needs logits [B, K, h, w] = {(b, n_class, h, w)} at the feature map's "
+                             f"resolution, got {tuple(label.shape)}")
     lab = label
     if not pseudo_label and (lab.shape[-1] != w or lab.shape[-2] != h):                 # :498-502
         if lab.ndim == 3:
@@ -109,7 +121,7 @@ def cal_centroid(decoder_ft, label, previous_centroid=None, momentum=0.95, pseud
     if pseudo_label:
         cen = SF.centroids(decoder_ft, None, lab, prev if isinstance(prev, torch.Tensor) else None,
                            weighted=bool(weighted_ave), threshold=thr, part_id=part_id, n_partitions=n_part,
-                           n_class=n_class, momentum=float(momentum), group=group)
+                           n_class=n_class, momentum=float(momentum), group=group, from_logits=bool(from_logits))
     else:
         cen = SF.centroids(decoder_ft, lab.reshape(-1).long(), None, prev if isinstance(prev, torch.Tensor) else None,
                            weighted=False, threshold=0.0, part_id=None, n_partitions=1, n_class=n_class,
