@@ -398,6 +398,12 @@ int slcl_seg_bwd_global(const float* logits, const int64_t* labels, int64_t batc
                         slcl_stream_t stream);
 int slcl_entropy_map(const float* prob, int64_t n_elems, int n_class, float* out, const float* grad_out,
                      float* dprob, slcl_stream_t stream);
+/* prob_2_entropy (utils/utils_.py:627-631) of softmax(logits, 1), the map of trainer/Trainer_MPSCL.py:171-172, from
+ * logits [B,K,HW] fp32 in one pass: p = softmax_k(z) (the seg losses' softmax), out = -p log2(p+1e-7)/log2(K) with
+ * slcl_entropy_map's arithmetic.  With grad_out and dlogits [B,K,HW] (= d/d out): dlogits = p (t - sum_m p_m t_m),
+ * t = grad_out * d out / d p, p recomputed from the logits.  out, the pair (grad_out, dlogits), or both; 2 <= K <= 8. */
+int slcl_entropy_map_logits(const float* logits, int64_t batch, int n_class, int64_t pixels, float* out,
+                            const float* grad_out, float* dlogits, slcl_stream_t stream);
 
 /* ---------------------------------------------------------------------------
  * Pixel <-> pixel supervised contrastive loss (SupConLoss.forward,

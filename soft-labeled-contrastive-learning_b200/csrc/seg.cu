@@ -6,7 +6,7 @@
 //   loss_calc        utils/loss.py:46-66    nn.CrossEntropyLoss (+ jaccard_loss when jaccard=True)
 //   jaccard_loss     utils/loss.py:11-43    softmax, one-hot, per-class intersection / union over (B,H,W)
 //   dice_loss        utils/loss.py:69-103   softmax, one-hot, per-(image,class) 2 p.g / (p.p + g.g + 1e-5)
-//   prob_2_entropy   utils/utils_.py:627-631   -p log2(p + 1e-7) / log2(C)
+//   prob_2_entropy   utils/utils_.py:627-631   -p log2(p + 1e-7) / log2(C), on probabilities or on logits (softmax fused)
 // Callers: trainer/Trainer_MPSCL.py:125,171-172, trainer/Trainer_MCCL.py:252.
 //
 // Roofline: HBM.  forward 4K + 8 B/px (logits + label), backward 8K + 8 B/px; the reference makes
@@ -328,6 +328,50 @@ __global__ void __launch_bounds__(kThreads) entropy_map_kernel(const float* prob
   if (dprob) dprob[i] = -gout[i] * inv_log2c * (l2 + p / ((p + 1e-7f) * 0.6931471805599453f));
 }
 
+// prob_2_entropy(softmax(z, 1)) straight from the logits (Trainer_MPSCL.py:171-172): p = softmax_k(z), then per class the
+// expressions of entropy_map_kernel.  BWD: dlogits = p (t - sum_m p_m t_m) with t = de/dp * gout, recomputed from z (nothing
+// is stashed); out is written too when non-null.  Grid and layout as seg_fwd_kernel.
+template <int K, int VEC, bool BWD>
+__global__ void __launch_bounds__(kThreads) entropy_logits_kernel(const float* logits, int64_t hw, float inv_log2c, float* out,
+                                                                  const float* gout, float* dlogits) {
+  const int64_t p = ((int64_t)blockIdx.x * kThreads + threadIdx.x) * VEC;
+  if (p >= hw) return;
+  const int64_t img = (int64_t)blockIdx.y * K * hw;
+  float prob[K][VEC], logp[K][VEC];
+  softmax_k<K, VEC>(logits + img, hw, p, prob, logp);
+  float e[K][VEC], t[K][VEC];
+  if constexpr (BWD) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) ldv<VEC>(gout + img + (int64_t)k * hw + p, t[k]);
+  }
+#pragma unroll
+  for (int v = 0; v < VEC; ++v) {
+    float dot = 0.f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const float pk = prob[k][v];
+      const float l2 = log2f(pk + 1e-7f);
+      e[k][v] = -pk * l2 * inv_log2c;
+      if constexpr (BWD) {
+        t[k][v] = -t[k][v] * inv_log2c * (l2 + pk / ((pk + 1e-7f) * 0.6931471805599453f));
+        dot = fmaf(pk, t[k][v], dot);
+      }
+    }
+    if constexpr (BWD) {
+#pragma unroll
+      for (int k = 0; k < K; ++k) t[k][v] = prob[k][v] * (t[k][v] - dot);          // softmax backward
+    }
+  }
+  if (!BWD || out) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) stv<VEC>(out + img + (int64_t)k * hw + p, e[k]);
+  }
+  if constexpr (BWD) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) stv<VEC>(dlogits + img + (int64_t)k * hw + p, t[k]);
+  }
+}
+
 }  // namespace
 }  // namespace slcl
 
@@ -462,4 +506,20 @@ extern "C" int slcl_entropy_map(const float* prob, int64_t n_elems, int n_class,
   entropy_map_kernel<<<(unsigned)ceil_div<int64_t>(n_elems, kThreads), kThreads, 0, (cudaStream_t)stream_>>>(
       prob, n_elems, inv_log2c, out, grad_out, dprob);
   return check_launch("slcl_entropy_map");
+}
+
+extern "C" int slcl_entropy_map_logits(const float* logits, int64_t batch, int n_class, int64_t pixels, float* out,
+                                       const float* grad_out, float* dlogits, slcl_stream_t stream_) {
+  if (!logits || batch <= 0 || pixels <= 0 || n_class < 2 || n_class > KM || (!out && !dlogits) || (dlogits && !grad_out))
+    return SLCL_ERR_INVALID_ARGUMENT;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const float inv_log2c = 1.0f / log2f((float)n_class);
+  const bool vec4 = (pixels % 4 == 0) && aligned16(logits) && aligned16(out) && aligned16(grad_out) && aligned16(dlogits);
+  const int bpi = (int)ceil_div<int64_t>(pixels, (int64_t)kThreads * (vec4 ? 4 : 1));
+  dim3 grid((unsigned)bpi, (unsigned)batch);
+  SLCL_SEG_DISPATCH(n_class, vec4, {
+    if (dlogits) entropy_logits_kernel<KK, VV, true><<<grid, kThreads, 0, stream>>>(logits, pixels, inv_log2c, out, grad_out, dlogits);
+    else entropy_logits_kernel<KK, VV, false><<<grid, kThreads, 0, stream>>>(logits, pixels, inv_log2c, out, nullptr, nullptr);
+  })
+  return check_launch("slcl_entropy_map_logits");
 }

@@ -108,6 +108,7 @@ SIGNATURES = {
     "slcl_seg_finish": (C.c_int, [_P, C.c_int, _P, _P]),
     "slcl_seg_bwd_global": (C.c_int, [_P, _P, _I64, C.c_int, _I64, _P, _P, _P, _P, _P]),
     "slcl_entropy_map": (C.c_int, [_P, _I64, C.c_int, _P, _P, _P, _P]),
+    "slcl_entropy_map_logits": (C.c_int, [_P, _I64, C.c_int, _I64, _P, _P, _P, _P]),
     "slcl_p2p_workspace_bytes": (_SZ, [_I64, _I64, _I64]),
     "slcl_p2p_state_bytes": (_SZ, [_I64, _I64]),
     "slcl_p2p_fwd": (C.c_int, [_P, _P, _I64, _I64, _I64, _P, _P, _P, C.c_int, C.c_int, _P, _P, C.c_float, _P, _P, _P, _P, _SZ,

@@ -1272,6 +1272,59 @@ def _(prob, grad_out):
     return torch.empty_like(prob)
 
 
+def check_entropy_logits(logits: Tensor) -> None:
+    """The logits entropy map's argument errors, raised before anything touches the device."""
+    if logits.dim() != 4 or logits.dtype != _F32:
+        raise ValueError(f"prob_2_entropy(from_logits=True): logits must be float32 [B, K, H, W], got "
+                         f"{logits.dtype} {tuple(logits.shape)}")
+    k = logits.shape[1]
+    if k < 2 or k > _lib.MAX_CLASSES:
+        raise ValueError(f"prob_2_entropy(from_logits=True) needs 2 <= K <= {_lib.MAX_CLASSES} classes, got {k}")
+
+
+@torch.library.custom_op("slcl::entropy_map_logits", mutates_args=(), device_types="cuda")
+def entropy_map_logits(logits: Tensor) -> Tensor:
+    """prob_2_entropy(softmax(logits, 1)) of [B, K, H, W] logits, one launch."""
+    check_entropy_logits(logits)
+    dev = require_cuda(logits)
+    lib = _lib.load()
+    z = logits.contiguous()
+    b, k, h, w = z.shape
+    out = torch.empty_like(z)
+    with _guard(dev):
+        st = lib.slcl_entropy_map_logits(ptr(z), b, k, h * w, ptr(out), None, None, stream_ptr(dev))
+    check(st, "slcl_entropy_map_logits")
+    return out
+
+
+@entropy_map_logits.register_fake
+def _(logits):
+    return logits.new_empty(logits.shape)
+
+
+@torch.library.custom_op("slcl::entropy_map_logits_bwd", mutates_args=(), device_types="cuda")
+def entropy_map_logits_bwd(logits: Tensor, grad_out: Tensor) -> Tensor:
+    """dL/dlogits of entropy_map_logits for grad_out = dL/d(map); the softmax is recomputed from the logits."""
+    check_entropy_logits(logits)
+    dev = require_cuda(logits, grad_out)
+    lib = _lib.load()
+    if grad_out.shape != logits.shape:
+        raise ValueError(f"grad_out must have the logits' shape {tuple(logits.shape)}, got {tuple(grad_out.shape)}")
+    z = logits.contiguous()
+    b, k, h, w = z.shape
+    g = grad_out.to(_F32).contiguous()
+    dz = torch.empty_like(z)
+    with _guard(dev):
+        st = lib.slcl_entropy_map_logits(ptr(z), b, k, h * w, None, ptr(g), ptr(dz), stream_ptr(dev))
+    check(st, "slcl_entropy_map_logits")
+    return dz
+
+
+@entropy_map_logits_bwd.register_fake
+def _(logits, grad_out):
+    return logits.new_empty(logits.shape)
+
+
 # ----------------------------------------------------------------------------
 # eager fast path
 # ----------------------------------------------------------------------------

@@ -120,6 +120,28 @@ class _EntropyMap(torch.autograd.Function):
         return _ops.entropy_map_bwd(prob.detach(), grad_out.contiguous())
 
 
-def prob_2_entropy(prob):
-    """utils/utils_.py:627-631: weighted self-information map -p log2(p + 1e-7) / log2(C) of [N,C,H,W] probabilities."""
-    return _EntropyMap.apply(prob)
+class _EntropyMapLogits(torch.autograd.Function):
+    """The map from logits; saves the logits only and recomputes the softmax in the backward."""
+    @staticmethod
+    def forward(ctx, logits):
+        ctx.save_for_backward(logits)
+        return _ops.entropy_map_logits(logits.detach())
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        (logits,) = ctx.saved_tensors
+        return _ops.entropy_map_logits_bwd(logits.detach(), grad_out)
+
+
+def prob_2_entropy(prob, from_logits=False):
+    """utils/utils_.py:627-631: weighted self-information map -p log2(p + 1e-7) / log2(C) of [N,C,H,W] probabilities.
+
+    ``from_logits`` (addition): ``prob`` holds float32 logits [B, K, H, W] (2 <= K <= 8) and the call returns
+    ``prob_2_entropy(torch.softmax(prob, 1))``, the gradient flowing into the logits; the softmax runs inside the map's
+    forward and backward kernels (Trainer_MPSCL.py:171-172 without the ``F.softmax``)."""
+    if not from_logits:
+        return _EntropyMap.apply(prob)
+    ops.check_entropy_logits(prob)
+    if torch.is_grad_enabled() and prob.requires_grad:
+        return _EntropyMapLogits.apply(prob)
+    return _ops.entropy_map_logits(prob)
