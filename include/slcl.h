@@ -300,6 +300,52 @@ int slcl_mccl_losses(const float* centroid_s, const float* centroid_t_parts, con
                      float inter_w, float intra_w, float cnr_w, float* losses, float* d_s, float* d_t_parts,
                      float* d_t_aug, void* workspace, size_t workspace_bytes, slcl_stream_t stream);
 
+/* The MCCL loss section from the decoder outputs to the loss with its gradients (trainer/Trainer_MCCL.py:275-326) in
+ * one forward and one backward call, defined as this composition:
+ *   S = slcl_centroids_fwd(feat_s, labels_s, previous_s, momentum)            hard labels; no gradient (:277)
+ *   T = slcl_centroids_fwd(feat_t, pred_t, part_id, n_partitions, flags, threshold)   soft labels
+ *   A = slcl_centroids_fwd(feat_a, pred_a, flags, threshold)                  P = 1; optional (feat_a = pred_a = null,
+ *                                                                             batch_a = 0: no intra term)
+ *   losses = slcl_mccl_losses(S, T, A, split, bg, norm, inter_w, intra_w, cnr_w)
+ * All maps are contiguous fp32 NCHW with the same channels and pixels (h * w); labels_s int64 [batch_s * pixels],
+ * pred_* [B, K, pixels] probabilities or, with flags & SLCL_SOFT_LOGITS, logits; 2 <= K <= 8, P * K <= 16.
+ * Outputs: sums [rows, C+1] fp64 and centroids [rows, C] with rows = (P + 1 + has_aug) K in the order S | T | A (sums
+ * bit-identical to the separate calls'), losses [4] = {total, inter, intra, cnr}, d_centroids [rows, C] = d total / d
+ * centroids (saved for the backward).
+ * slcl_mccl_step_fwd: one class-sum sweep per set, then one tail kernel (reduce of every set, with `peer` one exchange of
+ * the whole sums matrix -- capacity_words >= 2 rows (C+1) --, centroids, every centroid term); peer may be null.
+ * slcl_mccl_step_fwd_local writes this rank's sums only; the caller sums them over the ranks (e.g. NCCL) and
+ * slcl_mccl_step_finish computes the rest with the same arithmetic (its workspace:
+ * slcl_mccl_step_finish_workspace_bytes).
+ * slcl_mccl_step_bwd: dfeat_t / dfeat_a and, for SLCL_SOFT_WEIGHTED, dpred_t / dpred_a (each may be null; dL/dlogits
+ * with SLCL_SOFT_LOGITS) of grad_out[0] * total, from the forward's sums and d_centroids: three launches, no host sync.
+ * Workspace: slcl_centroid_bwd_workspace_bytes(channels, rows - K). */
+size_t slcl_mccl_step_workspace_bytes(int64_t batch_s, int64_t batch_t, int64_t batch_a, int64_t channels, int64_t pixels,
+                                      int n_partitions, int n_class);
+size_t slcl_mccl_step_finish_workspace_bytes(int has_aug, int64_t channels, int n_partitions, int n_class);
+int slcl_mccl_step_fwd(const float* feat_s, const int64_t* labels_s, int64_t batch_s, const float* feat_t,
+                       const float* pred_t, const int32_t* part_id, int64_t batch_t, const float* feat_a,
+                       const float* pred_a, int64_t batch_a, int64_t channels, int64_t pixels, int n_partitions,
+                       int n_class, int flags, float threshold, const float* previous_s, float momentum,
+                       int split, int bg, int norm, float inter_w, float intra_w, float cnr_w, double* sums,
+                       float* centroids, float* losses, float* d_centroids, const slcl_peer_t* peer,
+                       void* workspace, size_t workspace_bytes, slcl_stream_t stream);
+int slcl_mccl_step_fwd_local(const float* feat_s, const int64_t* labels_s, int64_t batch_s, const float* feat_t,
+                             const float* pred_t, const int32_t* part_id, int64_t batch_t, const float* feat_a,
+                             const float* pred_a, int64_t batch_a, int64_t channels, int64_t pixels,
+                             int n_partitions, int n_class, int flags, float threshold, double* sums,
+                             void* workspace, size_t workspace_bytes, slcl_stream_t stream);
+int slcl_mccl_step_finish(const double* sums, int has_aug, int64_t channels, int n_partitions, int n_class,
+                          const float* previous_s, float momentum, int split, int bg, int norm, float inter_w,
+                          float intra_w, float cnr_w, float* centroids, float* losses, float* d_centroids,
+                          void* workspace, size_t workspace_bytes, slcl_stream_t stream);
+int slcl_mccl_step_bwd(const float* feat_t, const float* pred_t, const int32_t* part_id, int64_t batch_t,
+                       const float* feat_a, const float* pred_a, int64_t batch_a, int64_t channels,
+                       int64_t pixels, int n_partitions, int n_class, int flags, float threshold,
+                       const double* sums, const float* d_centroids, const float* grad_out, float* dfeat_t,
+                       float* dpred_t, float* dfeat_a, float* dpred_a, void* workspace, size_t workspace_bytes,
+                       slcl_stream_t stream);
+
 /* ---------------------------------------------------------------------------
  * Sampler: per-class compaction + gather (north_star item 1).
  * slcl_compact_by_class: stable compaction of pixel indices by label, order

@@ -16,6 +16,7 @@
 // state is load + FMA only: 4C + 8 bytes per pixel, one pass, no atomics.
 // Per-block partials are summed in fp64 by a second tiny kernel in block
 // order (deterministic; exact integer counts beyond 2^24).
+#include "centroid_pair.cuh"
 #include "common.cuh"
 #include "peer.cuh"
 #include "proto_math.cuh"
@@ -1095,14 +1096,15 @@ struct CenBwdArgs {
 };
 
 // gc_j = dL/dcentroid_j * ema_scale / (W_j + 1e-7);  mu_dot_gc_j = mu_j . gc_j  with mu_j = S_j / (W_j + 1e-7)
-__global__ void __launch_bounds__(kThreads) centroid_bwd_prep_kernel(const float* grad_cen, const double* sums,
-                                                                     float ema_scale, int C, float* gc, float* mu_dot_gc) {
+// One block per row j; grad(i) is dL/dcentroid at flat index i = j * C + c.
+template <class Grad>
+__device__ __forceinline__ void centroid_bwd_prep_row(Grad grad, const double* sums, float ema_scale, int C, int j, float* gc,
+                                                      float* mu_dot_gc) {
   __shared__ float red[kWarps];
-  const int j = blockIdx.x;
   const float wsum = (float)sums[(int64_t)j * (C + 1) + C] + 1e-7f;
   float acc = 0.f;
   for (int c = threadIdx.x; c < C; c += kThreads) {
-    const float g = grad_cen[(int64_t)j * C + c] * ema_scale / wsum;
+    const float g = grad((int64_t)j * C + c) * ema_scale / wsum;
     const float mu = (float)sums[(int64_t)j * (C + 1) + c] / wsum;
     gc[(int64_t)j * C + c] = g;
     acc = fmaf(mu, g, acc);
@@ -1115,6 +1117,11 @@ __global__ void __launch_bounds__(kThreads) centroid_bwd_prep_kernel(const float
     for (int w = 0; w < kWarps; ++w) t += red[w];
     mu_dot_gc[j] = t;
   }
+}
+
+__global__ void __launch_bounds__(kThreads) centroid_bwd_prep_kernel(const float* grad_cen, const double* sums,
+                                                                     float ema_scale, int C, float* gc, float* mu_dot_gc) {
+  centroid_bwd_prep_row([=](int64_t i) { return grad_cen[i]; }, sums, ema_scale, C, blockIdx.x, gc, mu_dot_gc);
 }
 
 template <int KWT> constexpr int kwpad() { return (KWT + 3) / 4 * 4; }
@@ -1668,21 +1675,12 @@ void launch_reduce(const SumArgs& a, int n_blocks, int kwt, double* sums, const 
                                                                     PeerCtx{}, fin, a.ticket);
 }
 
-// sweep + reduce (+ cross-rank exchange through `peer`, + finaliser `fin` in the reduce kernel's last block).
-// logits: soft mode with logits in a.probs (the sweep applies the softmax).
-int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t workspace_bytes, cudaStream_t stream,
-                   const slcl_peer_t* peer = nullptr, FinArgs fin = FinArgs{}, bool logits = false) {
-  if (a.n_cols < 1 || a.n_cols > SLCL_MAX_WEIGHT_COLS) return SLCL_ERR_INVALID_ARGUMENT;
-  if (peer != nullptr) {
-    if (!peer_valid(peer)) return SLCL_ERR_INVALID_ARGUMENT;
-    if (2 * (int64_t)a.n_cols * (a.channels + 1) > peer->capacity_words) return SLCL_ERR_INVALID_ARGUMENT;
-  }
+// The sweep alone: per-block partials of `a` at `workspace` (`usable` bytes); the caller has set a.ticket.  On return
+// a.partial, n_blocks and kwt describe the partials for the reduce (launch_reduce or the MCCL step's tail).
+int launch_sweep(SumArgs& a, bool vec4, void* workspace, size_t usable, cudaStream_t stream, bool logits, int& n_blocks,
+                 int& kwt) {
   SumPlan p = plan_sums(a.batch, a.channels, a.pixels, a.n_cols, vec4);
   if (p.kwt < 0) return SLCL_ERR_INVALID_ARGUMENT;
-  if (workspace_bytes < partial_bytes(p, a.channels) + kTicketBytes || !aligned16(workspace)) return SLCL_ERR_WORKSPACE;
-  // the ticket lives in the last 256 bytes of the workspace the caller sized with class_sums_ws_bytes()
-  a.ticket = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(workspace) + (workspace_bytes - kTicketBytes) / 16 * 16);
-  const size_t usable = workspace_bytes - kTicketBytes;
   const V3Plan v3 = plan_v3(a, vec4);
   if (v3.ok && (size_t)v3.grid.x * v3.kwt * (a.channels + 1) * sizeof(float) <= usable) {
     a.partial = reinterpret_cast<float*>(workspace);
@@ -1699,10 +1697,11 @@ int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t w
       case 16: st = logits ? launch_v3_cpw<16, true>(a, v3, stream) : launch_v3_cpw<16, false>(a, v3, stream); break;
       default: return SLCL_ERR_INVALID_ARGUMENT;
     }
-    if (st != SLCL_OK) return st;
-    launch_reduce(a, (int)v3.grid.x, v3.kwt, sums, peer, fin, stream);
-    return check_launch("slcl_class_sums");
+    n_blocks = (int)v3.grid.x;
+    kwt = v3.kwt;
+    return st;
   }
+  if (partial_bytes(p, a.channels) > usable) return SLCL_ERR_WORKSPACE;
   a.tiles_per_image = p.tiles_per_image; a.n_tiles = p.n_tiles;
   a.cg_per_block = p.cg_per_block; a.pt_per_block = p.pt_per_block;
   a.partial = reinterpret_cast<float*>(workspace);
@@ -1718,7 +1717,29 @@ int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t w
     case 16: logits ? launch_sums<16, 4, true>(a, p, stream) : launch_sums<16, 4, false>(a, p, stream); break;
     default: return SLCL_ERR_INVALID_ARGUMENT;
   }
-  launch_reduce(a, (int)p.grid.x, p.kwt, sums, peer, fin, stream);
+  n_blocks = (int)p.grid.x;
+  kwt = p.kwt;
+  return SLCL_OK;
+}
+
+// sweep + reduce (+ cross-rank exchange through `peer`, + finaliser `fin` in the reduce kernel's last block).
+// logits: soft mode with logits in a.probs (the sweep applies the softmax).
+int run_class_sums(SumArgs a, bool vec4, double* sums, void* workspace, size_t workspace_bytes, cudaStream_t stream,
+                   const slcl_peer_t* peer = nullptr, FinArgs fin = FinArgs{}, bool logits = false) {
+  if (a.n_cols < 1 || a.n_cols > SLCL_MAX_WEIGHT_COLS) return SLCL_ERR_INVALID_ARGUMENT;
+  if (peer != nullptr) {
+    if (!peer_valid(peer)) return SLCL_ERR_INVALID_ARGUMENT;
+    if (2 * (int64_t)a.n_cols * (a.channels + 1) > peer->capacity_words) return SLCL_ERR_INVALID_ARGUMENT;
+  }
+  SumPlan p = plan_sums(a.batch, a.channels, a.pixels, a.n_cols, vec4);
+  if (p.kwt < 0) return SLCL_ERR_INVALID_ARGUMENT;
+  if (workspace_bytes < partial_bytes(p, a.channels) + kTicketBytes || !aligned16(workspace)) return SLCL_ERR_WORKSPACE;
+  // the ticket lives in the last 256 bytes of the workspace the caller sized with class_sums_ws_bytes()
+  a.ticket = reinterpret_cast<unsigned int*>(reinterpret_cast<char*>(workspace) + (workspace_bytes - kTicketBytes) / 16 * 16);
+  int n_blocks = 0, kwt = 0;
+  const int st = launch_sweep(a, vec4, workspace, workspace_bytes - kTicketBytes, stream, logits, n_blocks, kwt);
+  if (st != SLCL_OK) return st;
+  launch_reduce(a, n_blocks, kwt, sums, peer, fin, stream);
   return check_launch("slcl_class_sums");
 }
 
@@ -1977,6 +1998,53 @@ extern "C" int slcl_centroid_finalize(const double* sums, const float* previous,
   return check_launch("slcl_centroid_finalize");
 }
 
+namespace slcl {
+namespace {
+// The centroid backward sweep of `a` (a.gc / a.mu_dot_gc prepared): centroid_bwd4_kernel on 128-bit maps, else
+// centroid_bwd_kernel; a.dprobs may be null.
+int launch_centroid_bwd(const CenBwdArgs& a, bool vec4, bool logits, cudaStream_t stream) {
+  const int64_t channels = a.s.channels;
+  const float* dprobs = a.dprobs;
+  const int kwt = pick_kwt(a.s.n_cols);
+  const int vec = vec4 ? 4 : 1;
+  size_t smem = (size_t)channels * ((kwt + 3) / 4 * 4) * sizeof(float);
+  if (vec4) {      // centroid_bwd4_kernel: {g, g} pairs [C][KP] + per-thread scratch [KWT][threads] float4 (+ the cp.async ring)
+    smem = (size_t)channels * ((kwt + 1) / 2 * 2) * 8 + (size_t)kwt * kThreads * 16;
+    if (dprobs) smem += (size_t)kCenRing * kThreads * 16;
+  }
+  if (smem > 200 * 1024) return SLCL_ERR_UNSUPPORTED;
+  const int blocks = (int)ceil_div<int64_t>(a.s.batch * a.s.pixels / vec, kThreads);
+#define SLCL_CB(KW_)                                                                                          \
+  case KW_: {                                                                                                 \
+    auto launch = [&](auto kern) -> int {                                                                     \
+      if (smem > 48 * 1024) {                                                                                 \
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   \
+        if (e != cudaSuccess) { set_cuda_error(e, "cudaFuncSetAttribute"); return SLCL_ERR_CUDA; }            \
+      }                                                                                                       \
+      kern<<<blocks, kThreads, smem, stream>>>(a);                                                            \
+      return SLCL_OK;                                                                                         \
+    };                                                                                                        \
+    int st;                                                                                                   \
+    if (logits) {                                                                                             \
+      if (dprobs) st = vec4 ? launch(centroid_bwd4_kernel<KW_, true, true>) : launch(centroid_bwd_kernel<KW_, 1, true, true>); \
+      else st = vec4 ? launch(centroid_bwd4_kernel<KW_, false, true>) : launch(centroid_bwd_kernel<KW_, 1, false, true>); \
+    } else if (dprobs) {                                                                                      \
+      st = vec4 ? launch(centroid_bwd4_kernel<KW_, true, false>) : launch(centroid_bwd_kernel<KW_, 1, true, false>); \
+    } else {                                                                                                  \
+      st = vec4 ? launch(centroid_bwd4_kernel<KW_, false, false>) : launch(centroid_bwd_kernel<KW_, 1, false, false>); \
+    }                                                                                                         \
+    if (st != SLCL_OK) return st;                                                                             \
+  } break;
+  switch (kwt) {
+    SLCL_CB(2) SLCL_CB(3) SLCL_CB(4) SLCL_CB(5) SLCL_CB(6) SLCL_CB(8) SLCL_CB(10) SLCL_CB(12) SLCL_CB(16)
+    default: return SLCL_ERR_INVALID_ARGUMENT;
+  }
+#undef SLCL_CB
+  return SLCL_OK;
+}
+}  // namespace
+}  // namespace slcl
+
 extern "C" size_t slcl_centroid_bwd_workspace_bytes(int64_t channels, int n_cols) {
   if (channels <= 0 || n_cols < 1) return 0;
   return align_up((size_t)n_cols * (channels + 1) * sizeof(float), 256);
@@ -2011,42 +2079,319 @@ extern "C" int slcl_centroid_bwd(const float* feat, int64_t batch, int64_t chann
   a.s.part_id = part_id; a.s.n_part = n_partitions; a.s.n_class = n_class;
   a.s.n_cols = n_partitions * n_class;
   a.gc = gc; a.mu_dot_gc = mu_dot_gc; a.dfeat = dfeat; a.dprobs = dprobs;
-  const int kwt = pick_kwt(a.s.n_cols);
   const bool vec4 = nchw_vec4(feat, channels, pixels, {feat, labels, probs, part_id, dfeat, dprobs});
-  const int vec = vec4 ? 4 : 1;
-  size_t smem = (size_t)channels * ((kwt + 3) / 4 * 4) * sizeof(float);
-  if (vec4) {      // centroid_bwd4_kernel: {g, g} pairs [C][KP] + per-thread scratch [KWT][threads] float4 (+ the cp.async ring)
-    smem = (size_t)channels * ((kwt + 1) / 2 * 2) * 8 + (size_t)kwt * kThreads * 16;
-    if (dprobs) smem += (size_t)kCenRing * kThreads * 16;
-  }
-  if (smem > 200 * 1024) return SLCL_ERR_UNSUPPORTED;
-  const int blocks = (int)ceil_div<int64_t>(batch * pixels / vec, kThreads);
-  cudaStream_t stream = (cudaStream_t)stream_;
-#define SLCL_CB(KW_)                                                                                          \
-  case KW_: {                                                                                                 \
-    auto launch = [&](auto kern) -> int {                                                                     \
-      if (smem > 48 * 1024) {                                                                                 \
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   \
-        if (e != cudaSuccess) { set_cuda_error(e, "cudaFuncSetAttribute"); return SLCL_ERR_CUDA; }            \
-      }                                                                                                       \
-      kern<<<blocks, kThreads, smem, stream>>>(a);                                                            \
-      return SLCL_OK;                                                                                         \
-    };                                                                                                        \
-    int st;                                                                                                   \
-    if (logits) {                                                                                             \
-      if (dprobs) st = vec4 ? launch(centroid_bwd4_kernel<KW_, true, true>) : launch(centroid_bwd_kernel<KW_, 1, true, true>); \
-      else st = vec4 ? launch(centroid_bwd4_kernel<KW_, false, true>) : launch(centroid_bwd_kernel<KW_, 1, false, true>); \
-    } else if (dprobs) {                                                                                      \
-      st = vec4 ? launch(centroid_bwd4_kernel<KW_, true, false>) : launch(centroid_bwd_kernel<KW_, 1, true, false>); \
-    } else {                                                                                                  \
-      st = vec4 ? launch(centroid_bwd4_kernel<KW_, false, false>) : launch(centroid_bwd_kernel<KW_, 1, false, false>); \
-    }                                                                                                         \
-    if (st != SLCL_OK) return st;                                                                             \
-  } break;
-  switch (kwt) {
-    SLCL_CB(2) SLCL_CB(3) SLCL_CB(4) SLCL_CB(5) SLCL_CB(6) SLCL_CB(8) SLCL_CB(10) SLCL_CB(12) SLCL_CB(16)
-    default: return SLCL_ERR_INVALID_ARGUMENT;
-  }
-#undef SLCL_CB
+  const int st = launch_centroid_bwd(a, vec4, logits, (cudaStream_t)stream_);
+  if (st != SLCL_OK) return st;
   return check_launch("slcl_centroid_bwd");
+}
+
+// ===========================================================================
+// The MCCL loss section as one call (trainer/Trainer_MCCL.py:275-326):
+//   cs = cal_centroid(ft_s, labels_s, previous_centroid_s)              hard labels, EMA'd; detached (:277)
+//   ct = cal_centroid(ft_t, pred_t, pseudo_label, partition = P)        soft labels (probabilities or logits)
+//   ca = cal_centroid(ft_t_aug, pred_t_aug, pseudo_label)               P = 1, optional
+//   total, terms = mccl_centroid_losses(cs, ct, ca, ...)
+// Forward: the existing class-sum sweep once per set, each into its own region of one workspace, then ONE tail kernel
+// that reduces every set's partials in block order into one sums matrix
+//   rows [0, K) source | [K, (P+1)K) target partitions | [(P+1)K, (P+2)K) augmented target
+// (bit-identical to the separate calls' reduce), exchanges the whole matrix in one mailbox epoch, and in its last block
+// finalises the centroids and evaluates every centroid <-> centroid term and its gradient dL/dC (centroid_pair.cuh).
+// Backward: one coefficient kernel (grad_out * dL/dC scaled as centroid_bwd_prep_kernel does), then the existing
+// centroid backward sweep for the target set and for the augmented set.
+// ===========================================================================
+namespace slcl {
+namespace {
+
+constexpr int kStepMaxSets = 3;
+
+struct StepTail {
+  const float* partial[kStepMaxSets];
+  int n_blocks[kStepMaxSets], kwt[kStepMaxSets];
+  int row_end[kStepMaxSets];        // set s holds sums rows [row_end[s-1], row_end[s])
+  int rows, K, C;
+  double* sums;                     // [rows, C+1]
+  unsigned int* ticket;
+  const float* prev_s;              // previous source centroids [K, C] or null
+  float momentum;
+  float* cen;                       // [rows, C]
+  float* inv_w;                     // [rows] (scratch)
+  cpair::McclArgs loss;             // S, T, A = rows of cen; dS, dT, dA = rows of dL/dC
+};
+
+// One block: centroids from the complete sums, then every pair term and the weighted combination.
+__device__ __forceinline__ void mccl_step_finish_block(const StepTail& t) {
+  const FinArgs fs{kFinCentroid, t.prev_s, t.momentum, t.K, t.cen, t.inv_w};
+  finalize_rows(t.sums, fs, t.K, t.C, threadIdx.x, kThreads);
+  const FinArgs ft{kFinCentroid, nullptr, t.momentum, t.K, t.cen + (size_t)t.K * t.C, t.inv_w + t.K};
+  finalize_rows(t.sums + (size_t)t.K * (t.C + 1), ft, t.rows - t.K, t.C, threadIdx.x, kThreads);
+  __syncthreads();
+  for (int i = 0; i < 3 * t.loss.P; ++i) {
+    cpair::mccl_pair(t.loss, i);
+    __syncthreads();
+  }
+  cpair::mccl_combine<true>(t.loss);
+}
+
+// One warp per sums element, as class_sums_reduce_kernel; PEER: the element is all-reduced over the ranks in the same
+// epoch for every set.  `finish` = 0 leaves the (local) sums only: the NCCL route sums them and runs the finish kernel.
+template <bool PEER>
+__global__ void __launch_bounds__(kThreads) mccl_step_tail_kernel(const StepTail t, const PeerCtx pc, int finish) {
+  __shared__ int s_last;
+  const int lane = threadIdx.x & 31;
+  const int idx = blockIdx.x * kWarps + (threadIdx.x >> 5);
+  const int row = t.C + 1;
+  unsigned int e = 0u;
+  if constexpr (PEER) e = peer_epoch_begin(pc);
+  if (idx < t.rows * row) {
+    const int r = idx / row, c = idx % row;
+    int s = 0, r0 = 0;
+    while (r >= t.row_end[s]) { r0 = t.row_end[s]; ++s; }
+    const float* partial = t.partial[s];
+    const int kwt = t.kwt[s], n_blocks = t.n_blocks[s], col = r - r0;
+    double v = 0.0;                                   // the block order of class_sums_reduce_kernel: identical bits
+    for (int b = lane; b < n_blocks; b += 32) v += (double)partial[((int64_t)b * kwt + col) * row + c];
+    v = warp_sum(v);
+    if constexpr (PEER) v = peer_warp_allreduce(pc, e, idx, v);
+    if (lane == 0) t.sums[idx] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    bool last;
+    if constexpr (PEER) last = peer_epoch_end(pc, e, gridDim.x);
+    else {
+      __threadfence();
+      last = atomicAdd(t.ticket, 1u) == gridDim.x - 1;
+      if (last) *t.ticket = 0u;
+    }
+    s_last = last ? 1 : 0;
+  }
+  __syncthreads();
+  if (!s_last || !finish) return;
+  __threadfence();
+  mccl_step_finish_block(t);
+}
+
+__global__ void __launch_bounds__(kThreads) mccl_step_finish_kernel(const StepTail t) { mccl_step_finish_block(t); }
+
+// gc_j = (grad_out * dL/dC_j) / (W_j + 1e-7), mu_j . gc_j for the target and augmented rows (one block per row): the
+// arithmetic of the separate calls' backward, where autograd hands cal_centroid grad_out * dL/dC.
+__global__ void __launch_bounds__(kThreads) mccl_step_bwd_prep_kernel(const float* grad_out, const float* d_cen,
+                                                                      const double* sums, int C, float* gc,
+                                                                      float* mu_dot_gc) {
+  const float g = *grad_out;
+  centroid_bwd_prep_row([=](int64_t i) { return g * d_cen[i]; }, sums, 1.0f, C, blockIdx.x, gc, mu_dot_gc);
+}
+
+struct StepIn {
+  const float* feat_s; const int64_t* labels_s; int64_t batch_s;
+  const float* feat_t; const float* pred_t; const int32_t* part_id; int64_t batch_t;
+  const float* feat_a; const float* pred_a; int64_t batch_a;
+  int64_t channels, pixels;
+  int P, K, flags;
+  float threshold;
+};
+
+bool step_shape_ok(int64_t batch_s, int64_t batch_t, int64_t batch_a, int64_t channels, int64_t pixels, int P, int K) {
+  return batch_s > 0 && batch_t > 0 && batch_a >= 0 && channels > 0 && pixels > 0 && K >= 2 && K <= kMaxK && P >= 1 &&
+         P * K <= SLCL_MAX_WEIGHT_COLS && (int64_t)(P + 2) * K * (channels + 1) <= INT_MAX;
+}
+
+bool step_in_ok(const StepIn& in) {
+  if (!step_shape_ok(in.batch_s, in.batch_t, in.batch_a, in.channels, in.pixels, in.P, in.K)) return false;
+  if (!in.feat_s || !in.labels_s || !in.feat_t || !in.pred_t) return false;
+  if ((in.feat_a == nullptr) != (in.pred_a == nullptr) || (in.feat_a == nullptr) != (in.batch_a == 0)) return false;
+  if (in.P > 1 && in.part_id == nullptr) return false;
+  return (in.flags & ~(SLCL_SOFT_WEIGHTED | SLCL_SOFT_LOGITS)) == 0;
+}
+
+int step_rows(int P, int K, bool aug) { return (P + 1 + (aug ? 1 : 0)) * K; }
+
+size_t step_scratch_bytes(int rows, int P, int K, int64_t C) {
+  return align_up((size_t)rows * sizeof(float), 256) + slcl_mccl_losses_workspace_bytes(P, K, C);
+}
+
+size_t step_ws_bytes(int64_t batch_s, int64_t batch_t, int64_t batch_a, int64_t C, int64_t HW, int P, int K) {
+  size_t b = step_scratch_bytes(step_rows(P, K, batch_a > 0), P, K, C) + kTicketBytes;
+  b += class_sums_ws_bytes(batch_s, C, HW, K) - kTicketBytes;
+  b += class_sums_ws_bytes(batch_t, C, HW, P * K) - kTicketBytes;
+  if (batch_a > 0) b += class_sums_ws_bytes(batch_a, C, HW, K) - kTicketBytes;
+  return b;
+}
+
+// The loss half of the tail's arguments: centroids, dL/dC and the pair scratch.
+void step_loss_args(StepTail& t, int P, bool aug, int split, int bg, int norm, float inter_w, float intra_w, float cnr_w,
+                    float* losses, float* d_cen, void* scratch) {
+  const size_t kc = (size_t)t.K * t.C;
+  t.inv_w = reinterpret_cast<float*>(scratch);
+  cpair::McclArgs& a = t.loss;
+  a.S = t.cen; a.T = t.cen + kc; a.A = aug ? t.cen + (size_t)(P + 1) * kc : nullptr;
+  a.P = P; a.K = t.K; a.C = t.C; a.split = split; a.first = bg ? 0 : 1; a.norm = norm;
+  a.inter_w = inter_w; a.intra_w = intra_w; a.cnr_w = cnr_w;
+  a.scratch = reinterpret_cast<float*>(reinterpret_cast<char*>(scratch) + align_up((size_t)t.rows * sizeof(float), 256));
+  a.loss = losses; a.dS = d_cen; a.dT = d_cen + kc; a.dA = aug ? d_cen + (size_t)(P + 1) * kc : nullptr;
+}
+
+// One class-sum sweep per set, each into its own region of `workspace`; fills the reduce half of `t`.
+int step_sweeps(const StepIn& in, double* sums, void* workspace, size_t workspace_bytes, cudaStream_t stream, StepTail& t) {
+  const bool aug = in.feat_a != nullptr;
+  if (workspace_bytes < step_ws_bytes(in.batch_s, in.batch_t, in.batch_a, in.channels, in.pixels, in.P, in.K) ||
+      !aligned16(workspace))
+    return SLCL_ERR_WORKSPACE;
+  t.K = in.K; t.C = (int)in.channels; t.rows = step_rows(in.P, in.K, aug); t.sums = sums;
+  char* base = reinterpret_cast<char*>(workspace);
+  size_t off = step_scratch_bytes(t.rows, in.P, in.K, in.channels);
+  t.ticket = reinterpret_cast<unsigned int*>(base + off);
+  off += kTicketBytes;
+  const bool logits = (in.flags & SLCL_SOFT_LOGITS) != 0;
+  int row = 0;
+  for (int s = 0; s < (aug ? 3 : 2); ++s) {
+    SumArgs a{};
+    a.batch = s == 0 ? in.batch_s : s == 1 ? in.batch_t : in.batch_a;
+    a.feat = s == 0 ? in.feat_s : s == 1 ? in.feat_t : in.feat_a;
+    a.channels = in.channels; a.pixels = in.pixels;
+    a.sb = in.channels * in.pixels; a.sc = in.pixels; a.sp = 1;
+    a.n_class = in.K; a.n_part = s == 1 ? in.P : 1; a.n_cols = a.n_part * in.K;
+    if (s == 0) {
+      a.mode = kHard; a.labels = in.labels_s;
+    } else {
+      a.mode = kSoft; a.probs = s == 1 ? in.pred_t : in.pred_a;
+      a.weighted = in.flags & SLCL_SOFT_WEIGHTED; a.threshold = in.threshold;
+      a.part_id = (s == 1 && in.P > 1) ? in.part_id : nullptr;
+    }
+    a.ticket = t.ticket;
+    const bool vec4 = nchw_vec4(a.feat, a.channels, a.pixels, {a.feat, a.labels, a.probs, a.part_id});
+    const size_t region = class_sums_ws_bytes(a.batch, in.channels, in.pixels, a.n_cols) - kTicketBytes;
+    const int st = launch_sweep(a, vec4, base + off, region, stream, s > 0 && logits, t.n_blocks[s], t.kwt[s]);
+    if (st != SLCL_OK) return st;
+    t.partial[s] = a.partial;
+    row += a.n_cols;
+    t.row_end[s] = row;
+    off += region;
+  }
+  for (int s = aug ? 3 : 2; s < kStepMaxSets; ++s) t.row_end[s] = INT_MAX;
+  return SLCL_OK;
+}
+
+void launch_step_tail(const StepTail& t, const slcl_peer_t* peer, int finish, cudaStream_t stream) {
+  const dim3 grid(ceil_div(t.rows * (t.C + 1), kWarps));
+  if (peer != nullptr && peer->world > 1)
+    mccl_step_tail_kernel<true><<<grid, kThreads, 0, stream>>>(t, peer_ctx(peer), finish);
+  else
+    mccl_step_tail_kernel<false><<<grid, kThreads, 0, stream>>>(t, PeerCtx{}, finish);
+}
+
+}  // namespace
+}  // namespace slcl
+
+extern "C" size_t slcl_mccl_step_workspace_bytes(int64_t batch_s, int64_t batch_t, int64_t batch_a, int64_t channels,
+                                                 int64_t pixels, int n_partitions, int n_class) {
+  if (!step_shape_ok(batch_s, batch_t, batch_a, channels, pixels, n_partitions, n_class)) return 0;
+  return step_ws_bytes(batch_s, batch_t, batch_a, channels, pixels, n_partitions, n_class);
+}
+
+extern "C" size_t slcl_mccl_step_finish_workspace_bytes(int has_aug, int64_t channels, int n_partitions, int n_class) {
+  if (!step_shape_ok(1, 1, has_aug ? 1 : 0, channels, 1, n_partitions, n_class)) return 0;
+  return step_scratch_bytes(step_rows(n_partitions, n_class, has_aug != 0), n_partitions, n_class, channels);
+}
+
+extern "C" int slcl_mccl_step_fwd(const float* feat_s, const int64_t* labels_s, int64_t batch_s, const float* feat_t,
+                                  const float* pred_t, const int32_t* part_id, int64_t batch_t, const float* feat_a,
+                                  const float* pred_a, int64_t batch_a, int64_t channels, int64_t pixels, int n_partitions,
+                                  int n_class, int flags, float threshold, const float* previous_s, float momentum,
+                                  int split, int bg, int norm, float inter_w, float intra_w, float cnr_w, double* sums,
+                                  float* centroids, float* losses, float* d_centroids, const slcl_peer_t* peer,
+                                  void* workspace, size_t workspace_bytes, slcl_stream_t stream_) {
+  const StepIn in{feat_s, labels_s, batch_s, feat_t, pred_t, part_id, batch_t, feat_a, pred_a, batch_a, channels, pixels,
+                  n_partitions, n_class, flags, threshold};
+  if (!step_in_ok(in) || !sums || !centroids || !losses || !d_centroids || !workspace) return SLCL_ERR_INVALID_ARGUMENT;
+  const int rows = step_rows(n_partitions, n_class, feat_a != nullptr);
+  if (peer != nullptr) {
+    if (!peer_valid(peer)) return SLCL_ERR_INVALID_ARGUMENT;
+    if (2 * (int64_t)rows * (channels + 1) > peer->capacity_words) return SLCL_ERR_INVALID_ARGUMENT;
+  }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  StepTail t{};
+  int st = step_sweeps(in, sums, workspace, workspace_bytes, stream, t);
+  if (st != SLCL_OK) return st;
+  t.prev_s = previous_s; t.momentum = momentum; t.cen = centroids;
+  step_loss_args(t, n_partitions, feat_a != nullptr, split, bg, norm, inter_w, intra_w, cnr_w, losses, d_centroids, workspace);
+  launch_step_tail(t, peer, 1, stream);
+  return check_launch("slcl_mccl_step_fwd");
+}
+
+extern "C" int slcl_mccl_step_fwd_local(const float* feat_s, const int64_t* labels_s, int64_t batch_s, const float* feat_t,
+                                        const float* pred_t, const int32_t* part_id, int64_t batch_t, const float* feat_a,
+                                        const float* pred_a, int64_t batch_a, int64_t channels, int64_t pixels,
+                                        int n_partitions, int n_class, int flags, float threshold, double* sums,
+                                        void* workspace, size_t workspace_bytes, slcl_stream_t stream_) {
+  const StepIn in{feat_s, labels_s, batch_s, feat_t, pred_t, part_id, batch_t, feat_a, pred_a, batch_a, channels, pixels,
+                  n_partitions, n_class, flags, threshold};
+  if (!step_in_ok(in) || !sums || !workspace) return SLCL_ERR_INVALID_ARGUMENT;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  StepTail t{};
+  int st = step_sweeps(in, sums, workspace, workspace_bytes, stream, t);
+  if (st != SLCL_OK) return st;
+  launch_step_tail(t, nullptr, 0, stream);
+  return check_launch("slcl_mccl_step_fwd_local");
+}
+
+extern "C" int slcl_mccl_step_finish(const double* sums, int has_aug, int64_t channels, int n_partitions, int n_class,
+                                     const float* previous_s, float momentum, int split, int bg, int norm, float inter_w,
+                                     float intra_w, float cnr_w, float* centroids, float* losses, float* d_centroids,
+                                     void* workspace, size_t workspace_bytes, slcl_stream_t stream_) {
+  if (!step_shape_ok(1, 1, has_aug ? 1 : 0, channels, 1, n_partitions, n_class)) return SLCL_ERR_INVALID_ARGUMENT;
+  if (!sums || !centroids || !losses || !d_centroids || !workspace) return SLCL_ERR_INVALID_ARGUMENT;
+  if (workspace_bytes < slcl_mccl_step_finish_workspace_bytes(has_aug, channels, n_partitions, n_class) ||
+      !aligned16(workspace))
+    return SLCL_ERR_WORKSPACE;
+  StepTail t{};
+  t.K = n_class; t.C = (int)channels; t.rows = step_rows(n_partitions, n_class, has_aug != 0);
+  t.sums = const_cast<double*>(sums);
+  t.prev_s = previous_s; t.momentum = momentum; t.cen = centroids;
+  step_loss_args(t, n_partitions, has_aug != 0, split, bg, norm, inter_w, intra_w, cnr_w, losses, d_centroids, workspace);
+  mccl_step_finish_kernel<<<1, kThreads, 0, (cudaStream_t)stream_>>>(t);
+  return check_launch("slcl_mccl_step_finish");
+}
+
+extern "C" int slcl_mccl_step_bwd(const float* feat_t, const float* pred_t, const int32_t* part_id, int64_t batch_t,
+                                  const float* feat_a, const float* pred_a, int64_t batch_a, int64_t channels,
+                                  int64_t pixels, int n_partitions, int n_class, int flags, float threshold,
+                                  const double* sums, const float* d_centroids, const float* grad_out, float* dfeat_t,
+                                  float* dpred_t, float* dfeat_a, float* dpred_a, void* workspace, size_t workspace_bytes,
+                                  slcl_stream_t stream_) {
+  if (!step_shape_ok(1, batch_t, batch_a, channels, pixels, n_partitions, n_class) || !feat_t || !pred_t)
+    return SLCL_ERR_INVALID_ARGUMENT;
+  if ((feat_a == nullptr) != (pred_a == nullptr) || (feat_a == nullptr) != (batch_a == 0)) return SLCL_ERR_INVALID_ARGUMENT;
+  if ((flags & ~(SLCL_SOFT_WEIGHTED | SLCL_SOFT_LOGITS)) != 0 || (n_partitions > 1 && part_id == nullptr))
+    return SLCL_ERR_INVALID_ARGUMENT;
+  if (!sums || !d_centroids || !grad_out || !dfeat_t || (feat_a != nullptr && !dfeat_a)) return SLCL_ERR_INVALID_ARGUMENT;
+  if ((dpred_t != nullptr || dpred_a != nullptr) && !(flags & SLCL_SOFT_WEIGHTED)) return SLCL_ERR_INVALID_ARGUMENT;
+  const bool aug = feat_a != nullptr;
+  const int K = n_class, C = (int)channels;
+  const int g_rows = step_rows(n_partitions, K, aug) - K;            // target partitions + augmented target
+  if (workspace_bytes < slcl_centroid_bwd_workspace_bytes(channels, g_rows) || !aligned16(workspace))
+    return SLCL_ERR_WORKSPACE;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  float* gc = reinterpret_cast<float*>(workspace);
+  float* mu_dot_gc = gc + (size_t)g_rows * C;
+  mccl_step_bwd_prep_kernel<<<g_rows, kThreads, 0, stream>>>(grad_out, d_centroids + (size_t)K * C, sums + (size_t)K * (C + 1),
+                                                             C, gc, mu_dot_gc);
+  const bool logits = (flags & SLCL_SOFT_LOGITS) != 0;
+  for (int s = 1; s <= (aug ? 2 : 1); ++s) {
+    CenBwdArgs a{};
+    a.s.feat = s == 1 ? feat_t : feat_a;
+    a.s.batch = s == 1 ? batch_t : batch_a; a.s.channels = channels; a.s.pixels = pixels;
+    a.s.sb = channels * pixels; a.s.sc = pixels; a.s.sp = 1;
+    a.s.mode = kSoft; a.s.probs = s == 1 ? pred_t : pred_a;
+    a.s.weighted = flags & SLCL_SOFT_WEIGHTED; a.s.threshold = threshold;
+    a.s.part_id = (s == 1 && n_partitions > 1) ? part_id : nullptr;
+    a.s.n_part = s == 1 ? n_partitions : 1; a.s.n_class = K; a.s.n_cols = a.s.n_part * K;
+    const size_t row0 = s == 1 ? 0 : (size_t)n_partitions * K;
+    a.gc = gc + row0 * C; a.mu_dot_gc = mu_dot_gc + row0;
+    a.dfeat = s == 1 ? dfeat_t : dfeat_a; a.dprobs = s == 1 ? dpred_t : dpred_a;
+    const bool vec4 = nchw_vec4(a.s.feat, channels, pixels, {a.s.feat, a.s.probs, a.s.part_id, a.dfeat, a.dprobs});
+    const int st = launch_centroid_bwd(a, vec4, logits, stream);
+    if (st != SLCL_OK) return st;
+  }
+  return check_launch("slcl_mccl_step_bwd");
 }

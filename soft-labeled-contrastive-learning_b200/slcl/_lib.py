@@ -88,6 +88,18 @@ SIGNATURES = {
     "slcl_mccl_losses_workspace_bytes": (_SZ, [C.c_int, C.c_int, _I64]),
     "slcl_mccl_losses": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _I64, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float,
                                    _P, _P, _P, _P, _P, _SZ, _P]),
+    # the MCCL loss section in one call (trainer/Trainer_MCCL.py:275-326)
+    "slcl_mccl_step_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64, _I64, C.c_int, C.c_int]),
+    "slcl_mccl_step_finish_workspace_bytes": (_SZ, [C.c_int, _I64, C.c_int, C.c_int]),
+    "slcl_mccl_step_fwd": (C.c_int, [_P, _P, _I64, _P, _P, _P, _I64, _P, _P, _I64, _I64, _I64, C.c_int, C.c_int, C.c_int,
+                                     C.c_float, _P, C.c_float, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float,
+                                     _P, _P, _P, _P, C.POINTER(PeerT), _P, _SZ, _P]),
+    "slcl_mccl_step_fwd_local": (C.c_int, [_P, _P, _I64, _P, _P, _P, _I64, _P, _P, _I64, _I64, _I64, C.c_int, C.c_int, C.c_int,
+                                           C.c_float, _P, _P, _SZ, _P]),
+    "slcl_mccl_step_finish": (C.c_int, [_P, C.c_int, _I64, C.c_int, C.c_int, _P, C.c_float, C.c_int, C.c_int, C.c_int,
+                                        C.c_float, C.c_float, C.c_float, _P, _P, _P, _P, _SZ, _P]),
+    "slcl_mccl_step_bwd": (C.c_int, [_P, _P, _P, _I64, _P, _P, _I64, _I64, _I64, C.c_int, C.c_int, C.c_int, C.c_float, _P, _P,
+                                     _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "slcl_compact_workspace_bytes": (_SZ, [_I64, C.c_int]),
     "slcl_compact_by_class": (C.c_int, [_P, _I64, C.c_int, _P, _P, _P, _P, _SZ, _P]),
     "slcl_sample_balanced_workspace_bytes": (_SZ, [_I64, C.c_int]),

@@ -275,3 +275,58 @@ def mccl_losses(cs: Tensor, ct_parts: Tensor, ct_aug: Optional[Tensor], *, n_par
                 inter_w: float, intra_w: float, cnr_w: float):
     return _McclLosses.apply(cs, ct_parts, ct_aug, int(n_partitions), bool(split), bool(bg), bool(norm), float(inter_w),
                              float(intra_w), float(cnr_w))
+
+
+class _McclStep(torch.autograd.Function):
+    """The MCCL loss section (trainer/Trainer_MCCL.py:275-326) as one node: source, target and augmented-target centroids
+    and every centroid term in one forward call, the target maps' gradients in one backward call.  The source map gets no
+    gradient (the trainer detaches the source centroids, :277)."""
+
+    @staticmethod
+    def forward(ctx, feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, previous_s, n_partitions, n_class, weighted,
+                threshold, from_logits, momentum, split, bg, norm, inter_w, intra_w, cnr_w, group):
+        from .peer import PeerMailbox
+        d = lambda t: None if t is None else t.detach()
+        sets = (feat_s.detach(), labels_s, feat_t.detach(), pred_t.detach(), part_id, d(feat_a), d(pred_a))
+        loss_cfg = (momentum, split, bg, norm, inter_w, intra_w, cnr_w)
+        if group is None or isinstance(group, PeerMailbox):
+            peer = group.args() if group is not None else ()
+            losses, cen, sums, dcen = _ops.mccl_step_fwd(*sets, d(previous_s), n_partitions, n_class, weighted, threshold,
+                                                         from_logits, *loss_cfg, *peer)
+        else:       # NCCL: local sums -> one all-reduce -> the tail without the reduce
+            from .distributed import all_reduce_sums
+            sums = all_reduce_sums(_ops.mccl_step_fwd_local(*sets, n_partitions, n_class, weighted, threshold, from_logits),
+                                   group)
+            losses, cen, dcen = _ops.mccl_step_finish(sums, feat_a is not None, d(previous_s), n_partitions, n_class,
+                                                      *loss_cfg)
+        ctx.save_for_backward(feat_t, pred_t, part_id, feat_a, pred_a, sums, dcen)
+        ctx.cfg = (n_partitions, n_class, weighted, threshold, from_logits)
+        terms = losses[1:]
+        ctx.mark_non_differentiable(terms, cen, sums)
+        # the outputs other than `total` get no gradient: no zero tensors (one fill launch each) for their slots
+        ctx.set_materialize_grads(False)
+        return losses[0], terms, cen, sums
+
+    @staticmethod
+    def backward(ctx, g, _g_terms, _g_cen, _g_sums):
+        feat_t, pred_t, part_id, feat_a, pred_a, sums, dcen = ctx.saved_tensors
+        n_partitions, n_class, weighted, threshold, from_logits = ctx.cfg
+        need = ctx.needs_input_grad
+        if g is None or not (need[2] or need[3] or need[5] or need[6]):
+            return (None,) * 21
+        d = lambda t: None if t is None else t.detach()
+        df_t, dp_t, df_a, dp_a = _ops.mccl_step_bwd(feat_t.detach(), pred_t.detach(), part_id, d(feat_a), d(pred_a),
+                                                    n_partitions, n_class, weighted, threshold, from_logits, sums, dcen,
+                                                    g.reshape(1), bool(need[3] or need[6]))
+        pick = lambda t, i: t if (need[i] and t.numel()) else None
+        return (None, None, pick(df_t, 2), pick(dp_t, 3), None, pick(df_a, 5), pick(dp_a, 6)) + (None,) * 14
+
+
+def mccl_step(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, pred_t: Tensor, part_id: Optional[Tensor],
+              feat_a: Optional[Tensor], pred_a: Optional[Tensor], previous_s: Optional[Tensor], *, n_partitions: int,
+              n_class: int, weighted: bool, threshold: float, from_logits: bool, momentum: float, split: bool, bg: bool,
+              norm: bool, inter_w: float, intra_w: float, cnr_w: float, group=None):
+    """-> (total, terms [3], centroids [rows, C] (source | target partitions | aug), sums [rows, C+1] fp64)."""
+    return _McclStep.apply(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, previous_s, int(n_partitions),
+                           int(n_class), bool(weighted), float(threshold), bool(from_logits), float(momentum), bool(split),
+                           bool(bg), bool(norm), float(inter_w), float(intra_w), float(cnr_w), group)

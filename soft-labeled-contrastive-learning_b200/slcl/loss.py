@@ -186,6 +186,90 @@ def mccl_centroid_losses(centroid_s, centroid_t, centroid_t_aug=None, inter_w=1.
                           inter_w=inter_w, intra_w=intra_w, cnr_w=cnr_w)
 
 
+def mccl_step(ft_s, labels_s, ft_t, pred_t, ft_t_aug=None, pred_t_aug=None, *, n_class=4, partition=2, part_id=None,
+              generator=None, threshold=None, weighted_ave=True, from_logits=True, previous_centroid_s=None, momentum=0.95,
+              inter_w=1.0, intra_w=1.0, cnr_w=4e-5, split=False, bg=False, norm=True, group=None):
+    """The MCCL loss section of trainer/Trainer_MCCL.py:275-326, from the decoder outputs to the loss, as ONE forward and
+    ONE backward call (an addition).  It is defined as this composition of the drop-in calls::
+
+        cs, _, _ = cal_centroid(ft_s, labels_s, previous_centroid=previous_centroid_s, momentum=momentum, n_class=n_class)
+        cs = cs.detach()
+        ct, _, _ = cal_centroid(ft_t, pred_t, pseudo_label=True, partition=partition, threshold=threshold,
+                                weighted_ave=weighted_ave, n_class=n_class, part_id=part_id, generator=generator,
+                                from_logits=from_logits)
+        ct_aug, _, _ = cal_centroid(ft_t_aug, pred_t_aug, pseudo_label=True, threshold=threshold,
+                                    weighted_ave=weighted_ave, n_class=n_class, from_logits=from_logits)
+        total, terms = mccl_centroid_losses(cs, ct, ct_aug, inter_w, intra_w, cnr_w, split=split, bg=bg, norm=norm)
+
+    and returns ``(total, terms, cs, ct, ct_aug)``: ``total`` differentiable w.r.t. ``ft_t``, ``ft_t_aug``, ``pred_t`` and
+    ``pred_t_aug`` (dL/dlogits with ``from_logits``, dL/dprobs otherwise); ``ft_s`` gets no gradient.  ``terms`` =
+    ``[inter, intra, cnr]`` and the centroids are detached; ``ct`` is a list of ``partition`` tensors when
+    ``partition > 1``; ``ct_aug`` is None without the augmented view (and there is then no intra term).
+
+    The class sums of every set come from the same sweeps as ``cal_centroid``'s, reduced in the same order, and one tail
+    kernel finalises the centroids and evaluates every centroid term: four launches forward when ``part_id`` is given,
+    three backward, no host synchronisation.  ``group``: as ``cal_centroid`` / ``seg_losses`` -- the centroids and losses
+    of the ranks' batches concatenated, with ONE exchange of all the sets' sums per step (inside the tail kernel for a
+    ``slcl.peer.PeerMailbox``, one NCCL all-reduce for ``True`` / a ProcessGroup).
+
+    Raises ``ValueError``, before any launch or exchange, for maps that are not contiguous float32 NCHW, channel counts
+    that differ, ``n_class`` outside [2, 8] or ``partition * n_class > 16``, labels or ``pred`` not at the feature
+    map's resolution, or a mailbox too small for the sums; the separate calls remain the route for those."""
+    from .seg import _resolve_group
+    from .utils_ import rmc_partition_ids
+    from ._lib import MAX_CLASSES, MAX_WEIGHT_COLS
+    from .peer import PeerMailbox
+    k, parts = int(n_class), int(partition)
+    if not (2 <= k <= MAX_CLASSES):
+        raise ValueError(f"mccl_step: n_class must be in [2, {MAX_CLASSES}], got {k}")
+    if parts < 1 or parts * k > MAX_WEIGHT_COLS:
+        raise ValueError(f"mccl_step: partition * n_class must be at most {MAX_WEIGHT_COLS}, got {parts} * {k}")
+    if (ft_t_aug is None) != (pred_t_aug is None):
+        raise ValueError("mccl_step: ft_t_aug and pred_t_aug go together")
+    maps = [("ft_s", ft_s), ("ft_t", ft_t)] + ([("ft_t_aug", ft_t_aug)] if ft_t_aug is not None else [])
+    for name, m in maps:
+        if not isinstance(m, torch.Tensor) or m.dim() != 4 or m.dtype != torch.float32 or not m.is_contiguous():
+            raise ValueError(f"mccl_step: {name} must be a contiguous float32 [B, C, h, w] map")
+    c, h, w = ft_s.shape[1:]
+    for name, m in maps[1:]:
+        if m.shape[1] != c:
+            raise ValueError(f"mccl_step: {name} has {m.shape[1]} channels, ft_s has {c}")
+        if tuple(m.shape[2:]) != (h, w):
+            raise ValueError(f"mccl_step: {name} is {tuple(m.shape[2:])}, ft_s is {(h, w)}: the maps share one resolution")
+    b_s, b_t = ft_s.shape[0], ft_t.shape[0]
+    if labels_s.shape[-2:] != (h, w) or labels_s.numel() != b_s * h * w:
+        raise ValueError(f"mccl_step: labels_s must be [B, h, w] = {(b_s, h, w)} at the feature map's resolution, "
+                         f"got {tuple(labels_s.shape)}")
+    for name, p, b in [("pred_t", pred_t, b_t)] + ([("pred_t_aug", pred_t_aug, ft_t_aug.shape[0])] if ft_t_aug is not None
+                                                      else []):
+        if tuple(p.shape) != (b, k, h, w) or p.dtype != torch.float32:
+            raise ValueError(f"mccl_step: {name} must be float32 [B, K, h, w] = {(b, k, h, w)} at the feature map's "
+                             f"resolution, got {tuple(p.shape)} {p.dtype}")
+    if previous_centroid_s is not None and tuple(previous_centroid_s.shape) != (k, c):
+        raise ValueError(f"mccl_step: previous_centroid_s must be [K, C] = {(k, c)}, got {tuple(previous_centroid_s.shape)}")
+    if parts > 1 and part_id is not None and part_id.numel() != b_t * h * w:
+        raise ValueError(f"mccl_step: part_id must hold B_t*h*w = {b_t * h * w} ids, got {part_id.numel()}")
+    group = _resolve_group(group)
+    rows = (parts + 1 + (ft_t_aug is not None)) * k
+    if isinstance(group, PeerMailbox) and group.capacity_words < 2 * rows * (c + 1):
+        raise ValueError(f"mccl_step: the sums of one step are {rows} x {c + 1} doubles; the mailbox needs capacity_words >= "
+                         f"{2 * rows * (c + 1)}, this one has {group.capacity_words}")
+    pid = None
+    if parts > 1:
+        pid = part_id if part_id is not None else rmc_partition_ids(b_t * h * w, parts, generator, ft_t.device)
+        pid = pid.to(device=ft_t.device, dtype=torch.int32).reshape(-1)
+    thr = float(threshold) if threshold is not None else 0.0
+    total, terms, cen, _sums = SF.mccl_step(ft_s, labels_s.to(ft_s.device), ft_t, pred_t, pid, ft_t_aug, pred_t_aug,
+                                            previous_centroid_s, n_partitions=parts, n_class=k, weighted=bool(weighted_ave),
+                                            threshold=thr, from_logits=bool(from_logits), momentum=float(momentum),
+                                            split=split, bg=bg, norm=norm, inter_w=inter_w, intra_w=intra_w, cnr_w=cnr_w,
+                                            group=group)
+    cs = cen[:k]
+    ct = [cen[(p + 1) * k:(p + 2) * k] for p in range(parts)] if parts > 1 else cen[k:2 * k]
+    ct_aug = cen[(parts + 1) * k:] if ft_t_aug is not None else None
+    return total, terms, cs, ct, ct_aug
+
+
 SupConLoss = p2p.SupConLoss
 LocalConLoss = p2p.LocalConLoss
 BlockConLoss = p2p.BlockConLoss

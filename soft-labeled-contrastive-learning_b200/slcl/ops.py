@@ -676,6 +676,174 @@ def _(centroid_s, centroid_t_parts, centroid_t_aug, n_partitions, split, bg, nor
 
 
 # ----------------------------------------------------------------------------
+# the MCCL loss section in one call (trainer/Trainer_MCCL.py:275-326)
+# ----------------------------------------------------------------------------
+def mccl_step_rows(n_partitions: int, n_class: int, has_aug: bool) -> int:
+    """Rows of the step's sums / centroids: source K | target P*K | augmented target K (when given)."""
+    return (int(n_partitions) + 1 + (1 if has_aug else 0)) * int(n_class)
+
+
+def _mccl_step_inputs(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, n_partitions, n_class):
+    """(pointers and sizes) of the sets; the caller (slcl.loss.mccl_step) has validated shapes and dtypes."""
+    b_s, c, h, w = feat_s.shape
+    b_t = feat_t.shape[0]
+    b_a = 0 if feat_a is None else feat_a.shape[0]
+    labels_s = labels_s.reshape(-1).long().contiguous()
+    if part_id is not None:
+        part_id = part_id.reshape(-1).to(torch.int32).contiguous()
+    if n_partitions > 1 and (part_id is None or part_id.numel() != b_t * h * w):
+        raise ValueError("n_partitions > 1 needs part_id with B_t*h*w elements")
+    keep = (feat_s.contiguous(), labels_s, feat_t.contiguous(), pred_t.contiguous(), part_id,
+            None if feat_a is None else feat_a.contiguous(), None if pred_a is None else pred_a.contiguous())
+    return keep, (b_s, b_t, b_a, c, h * w)
+
+
+def _mccl_step_args(keep, sizes, n_partitions, n_class, weighted, threshold, from_logits):
+    f_s, l_s, f_t, p_t, pid, f_a, p_a = keep
+    b_s, b_t, b_a, c, hw = sizes
+    return (ptr(f_s), ptr(l_s), b_s, ptr(f_t), ptr(p_t), ptr(pid), b_t, ptr(f_a), ptr(p_a), b_a, c, hw, int(n_partitions),
+            int(n_class), _soft_flags(weighted, from_logits), float(threshold))
+
+
+@torch.library.custom_op("slcl::mccl_step_fwd", mutates_args=(), device_types="cuda")
+def mccl_step_fwd(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, pred_t: Tensor, part_id: Optional[Tensor],
+                  feat_a: Optional[Tensor], pred_a: Optional[Tensor], previous_s: Optional[Tensor], n_partitions: int,
+                  n_class: int, weighted: bool, threshold: float, from_logits: bool, momentum: float, split: bool, bg: bool,
+                  norm: bool, inter_w: float, intra_w: float, cnr_w: float, peer_ptrs: int = 0, rank: int = 0, world: int = 1,
+                  capacity_words: int = 0, timeout_s: float = 0.0) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """One class-sum sweep per set + one tail kernel [+ one peer exchange of every set's sums].
+    -> (losses[4] = {total, inter, intra, cnr}, centroids [rows, C], sums [rows, C+1] fp64, d total / d centroids [rows, C])."""
+    dev = require_cuda(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, previous_s)
+    lib = _lib.load()
+    keep, sizes = _mccl_step_inputs(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, n_partitions, n_class)
+    b_s, b_t, b_a, c, hw = sizes
+    rows = mccl_step_rows(n_partitions, n_class, feat_a is not None)
+    prev = None if previous_s is None else previous_s.to(_F32).contiguous()
+    losses = torch.empty(4, dtype=_F32, device=dev)
+    cen = torch.empty((rows, c), dtype=_F32, device=dev)
+    sums = torch.empty((rows, c + 1), dtype=torch.float64, device=dev)
+    dcen = torch.empty((rows, c), dtype=_F32, device=dev)
+    ws = _ws(lib.slcl_mccl_step_workspace_bytes(b_s, b_t, b_a, c, hw, n_partitions, n_class), dev)
+    peer = _peer(peer_ptrs, rank, world, capacity_words, timeout_s)
+    with _guard(dev):
+        st = lib.slcl_mccl_step_fwd(*_mccl_step_args(keep, sizes, n_partitions, n_class, weighted, threshold, from_logits),
+                                    ptr(prev), float(momentum), int(split), int(bg), int(norm), float(inter_w),
+                                    float(intra_w), float(cnr_w), ptr(sums), ptr(cen), ptr(losses), ptr(dcen),
+                                    C.byref(peer) if peer is not None else None, ptr(ws), ws.numel(), stream_ptr(dev))
+    check(st, "slcl_mccl_step_fwd")
+    return losses, cen, sums, dcen
+
+
+@mccl_step_fwd.register_fake
+def _(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, previous_s, n_partitions, n_class, weighted, threshold,
+      from_logits, momentum, split, bg, norm, inter_w, intra_w, cnr_w, peer_ptrs=0, rank=0, world=1, capacity_words=0,
+      timeout_s=0.0):
+    rows, c = mccl_step_rows(n_partitions, n_class, feat_a is not None), feat_s.shape[1]
+    return (feat_s.new_empty(4), feat_s.new_empty((rows, c)), feat_s.new_empty((rows, c + 1), dtype=torch.float64),
+            feat_s.new_empty((rows, c)))
+
+
+@torch.library.custom_op("slcl::mccl_step_fwd_local", mutates_args=(), device_types="cuda")
+def mccl_step_fwd_local(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, pred_t: Tensor, part_id: Optional[Tensor],
+                        feat_a: Optional[Tensor], pred_a: Optional[Tensor], n_partitions: int, n_class: int, weighted: bool,
+                        threshold: float, from_logits: bool) -> Tensor:
+    """-> this rank's sums [rows, C+1] fp64; sum them over the ranks, then mccl_step_finish."""
+    dev = require_cuda(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a)
+    lib = _lib.load()
+    keep, sizes = _mccl_step_inputs(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, n_partitions, n_class)
+    b_s, b_t, b_a, c, hw = sizes
+    sums = torch.empty((mccl_step_rows(n_partitions, n_class, feat_a is not None), c + 1), dtype=torch.float64, device=dev)
+    ws = _ws(lib.slcl_mccl_step_workspace_bytes(b_s, b_t, b_a, c, hw, n_partitions, n_class), dev)
+    with _guard(dev):
+        st = lib.slcl_mccl_step_fwd_local(*_mccl_step_args(keep, sizes, n_partitions, n_class, weighted, threshold,
+                                                           from_logits), ptr(sums), ptr(ws), ws.numel(), stream_ptr(dev))
+    check(st, "slcl_mccl_step_fwd_local")
+    return sums
+
+
+@mccl_step_fwd_local.register_fake
+def _(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, n_partitions, n_class, weighted, threshold, from_logits):
+    rows = mccl_step_rows(n_partitions, n_class, feat_a is not None)
+    return feat_s.new_empty((rows, feat_s.shape[1] + 1), dtype=torch.float64)
+
+
+@torch.library.custom_op("slcl::mccl_step_finish", mutates_args=(), device_types="cuda")
+def mccl_step_finish(sums: Tensor, has_aug: bool, previous_s: Optional[Tensor], n_partitions: int, n_class: int,
+                     momentum: float, split: bool, bg: bool, norm: bool, inter_w: float, intra_w: float,
+                     cnr_w: float) -> Tuple[Tensor, Tensor, Tensor]:
+    """The tail's work after the reduce, from sums summed over the ranks.  -> (losses[4], centroids, d total / d centroids)."""
+    dev = require_cuda(sums, previous_s)
+    lib = _lib.load()
+    rows = mccl_step_rows(n_partitions, n_class, has_aug)
+    if sums.dtype != torch.float64 or sums.dim() != 2 or sums.shape[0] != rows:
+        raise ValueError(f"sums must be float64 [{rows}, C+1]")
+    sums = sums.contiguous()
+    c = sums.shape[1] - 1
+    prev = None if previous_s is None else previous_s.to(_F32).contiguous()
+    losses = torch.empty(4, dtype=_F32, device=dev)
+    cen = torch.empty((rows, c), dtype=_F32, device=dev)
+    dcen = torch.empty((rows, c), dtype=_F32, device=dev)
+    ws = _ws(lib.slcl_mccl_step_finish_workspace_bytes(int(has_aug), c, n_partitions, n_class), dev)
+    with _guard(dev):
+        st = lib.slcl_mccl_step_finish(ptr(sums), int(has_aug), c, int(n_partitions), int(n_class), ptr(prev), float(momentum),
+                                       int(split), int(bg), int(norm), float(inter_w), float(intra_w), float(cnr_w), ptr(cen),
+                                       ptr(losses), ptr(dcen), ptr(ws), ws.numel(), stream_ptr(dev))
+    check(st, "slcl_mccl_step_finish")
+    return losses, cen, dcen
+
+
+@mccl_step_finish.register_fake
+def _(sums, has_aug, previous_s, n_partitions, n_class, momentum, split, bg, norm, inter_w, intra_w, cnr_w):
+    rows, c = sums.shape[0], sums.shape[1] - 1
+    return sums.new_empty(4, dtype=_F32), sums.new_empty((rows, c), dtype=_F32), sums.new_empty((rows, c), dtype=_F32)
+
+
+@torch.library.custom_op("slcl::mccl_step_bwd", mutates_args=(), device_types="cuda")
+def mccl_step_bwd(feat_t: Tensor, pred_t: Tensor, part_id: Optional[Tensor], feat_a: Optional[Tensor], pred_a: Optional[Tensor],
+                  n_partitions: int, n_class: int, weighted: bool, threshold: float, from_logits: bool, sums: Tensor,
+                  d_centroids: Tensor, grad_out: Tensor, need_dpred: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (dfeat_t, dpred_t, dfeat_a, dpred_a) of grad_out * total; empty tensors for what is not computed (dpred without
+    ``need_dpred`` or ``weighted``; the aug set when it is absent)."""
+    dev = require_cuda(feat_t, pred_t, part_id, feat_a, pred_a, sums, d_centroids, grad_out)
+    lib = _lib.load()
+    feat_t, pred_t = feat_t.contiguous(), pred_t.contiguous()
+    if part_id is not None:
+        part_id = part_id.reshape(-1).to(torch.int32).contiguous()
+    b_t, c, h, w = feat_t.shape
+    aug = feat_a is not None
+    if aug:
+        feat_a, pred_a = feat_a.contiguous(), pred_a.contiguous()
+    b_a = feat_a.shape[0] if aug else 0
+    g = grad_out.to(_F32).reshape(1).contiguous()
+    want_dp = bool(need_dpred and weighted)
+    empty = torch.empty(0, dtype=_F32, device=dev)
+    dfeat_t = torch.empty_like(feat_t)
+    dpred_t = torch.empty_like(pred_t) if want_dp else empty
+    dfeat_a = torch.empty_like(feat_a) if aug else empty
+    dpred_a = torch.empty_like(pred_a) if (aug and want_dp) else empty
+    rows = mccl_step_rows(n_partitions, n_class, aug)
+    ws = _ws(lib.slcl_centroid_bwd_workspace_bytes(c, rows - n_class), dev)
+    with _guard(dev):
+        st = lib.slcl_mccl_step_bwd(ptr(feat_t), ptr(pred_t), ptr(part_id), b_t, ptr(feat_a), ptr(pred_a), b_a, c, h * w,
+                                    int(n_partitions), int(n_class), _soft_flags(weighted, from_logits), float(threshold),
+                                    ptr(sums.contiguous()), ptr(d_centroids.contiguous()), ptr(g), ptr(dfeat_t),
+                                    ptr(dpred_t) if want_dp else None, ptr(dfeat_a) if aug else None,
+                                    ptr(dpred_a) if (aug and want_dp) else None, ptr(ws), ws.numel(), stream_ptr(dev))
+    check(st, "slcl_mccl_step_bwd")
+    return dfeat_t, dpred_t, dfeat_a, dpred_a
+
+
+@mccl_step_bwd.register_fake
+def _(feat_t, pred_t, part_id, feat_a, pred_a, n_partitions, n_class, weighted, threshold, from_logits, sums, d_centroids,
+      grad_out, need_dpred):
+    want_dp = bool(need_dpred and weighted)
+    empty = feat_t.new_empty(0)
+    return (torch.empty_like(feat_t), torch.empty_like(pred_t) if want_dp else empty,
+            torch.empty_like(feat_a) if feat_a is not None else empty,
+            torch.empty_like(pred_a) if (feat_a is not None and want_dp) else empty)
+
+
+# ----------------------------------------------------------------------------
 # sampler
 # ----------------------------------------------------------------------------
 @torch.library.custom_op("slcl::compact_by_class", mutates_args=(), device_types="cuda")
