@@ -347,6 +347,41 @@ int slcl_mccl_step_bwd(const float* feat_t, const float* pred_t, const int32_t* 
                        slcl_stream_t stream);
 
 /* ---------------------------------------------------------------------------
+ * The MPSCL loss section (trainer/Trainer_MPSCL.py:133-147) in one call:
+ *   centres = update_class_center_iter(feat_s, labels_s, old_centres, momentum)
+ *   hard, mask = generate_pseudo_label(feat_t, centres, sel_threshold)
+ *   loss_s = mpcl_loss_calc(feat_s, labels_s, centres, mpcl_src)
+ *   loss_t = mpcl_loss_calc(feat_t, hard, centres, mpcl_trg, pixel_sel_loc=mask)
+ * Both maps are dense NCHW with the same channels and pixels (batches may differ); params_s / params_t carry each
+ * loss's constants, the same n_class in [2, 8], and normalize = 1.  scal_s / scal_t are the quadruples of
+ * slcl_proto_fwd (loss, coefficient, weight sum, weighted row-loss sum); label_t / sel_t are the pseudo labels and mask.
+ * slcl_mpscl_step_fwd: the class-sum sweep and reduce [+ exchange through `peer`, capacity_words >= 2 K (C+1)] + EMA of
+ * slcl_class_centres_update, the unit centres, ONE prototype forward over both maps and ONE finaliser that exchanges
+ * both loss pairs in one mailbox epoch: 5 launches; peer may be null.
+ * slcl_mpscl_step_fwd_local (NCCL route, after the caller has the global centres): the same forward without the
+ * exchange; pairs[4] = this rank's {w_s, l_s, w_t, l_t}.  Sum pairs over the ranks, then slcl_mpscl_step_finish.
+ * slcl_mpscl_step_bwd: dfeat_s = grad_s[0] d loss_s / d feat_s and dfeat_t likewise, one launch over both maps; a null
+ * grad_s or grad_t skips that map.  Each map's load width follows its own alignment; maps of different widths take
+ * one launch each. */
+size_t slcl_mpscl_step_workspace_bytes(const slcl_map_t* map_s, const slcl_map_t* map_t, int n_class);
+int slcl_mpscl_step_fwd(const float* feat_s, const slcl_map_t* map_s, const int64_t* labels_s, const float* feat_t,
+                        const slcl_map_t* map_t, const float* old_centres, float momentum,
+                        const slcl_proto_params_t* params_s, const slcl_proto_params_t* params_t, float sel_threshold,
+                        float* centres, float* cstate, float* stash_s, float* stash_t, int64_t* label_t, float* sel_t,
+                        float* scal_s, float* scal_t, const slcl_peer_t* peer, void* workspace, size_t workspace_bytes,
+                        slcl_stream_t stream);
+int slcl_mpscl_step_fwd_local(const float* feat_s, const slcl_map_t* map_s, const int64_t* labels_s, const float* feat_t,
+                              const slcl_map_t* map_t, const float* centres, const slcl_proto_params_t* params_s,
+                              const slcl_proto_params_t* params_t, float sel_threshold, float* cstate, float* stash_s,
+                              float* stash_t, int64_t* label_t, float* sel_t, float* pairs, void* workspace,
+                              size_t workspace_bytes, slcl_stream_t stream);
+int slcl_mpscl_step_finish(const float* pairs, float* scal_s, float* scal_t, slcl_stream_t stream);
+int slcl_mpscl_step_bwd(const float* feat_s, const slcl_map_t* map_s, const float* feat_t, const slcl_map_t* map_t,
+                        const float* stash_s, const float* stash_t, const float* cstate, const float* scal_s,
+                        const float* scal_t, const float* grad_s, const float* grad_t, const slcl_proto_params_t* params_s,
+                        const slcl_proto_params_t* params_t, float* dfeat_s, float* dfeat_t, slcl_stream_t stream);
+
+/* ---------------------------------------------------------------------------
  * Sampler: per-class compaction + gather (north_star item 1).
  * slcl_compact_by_class: stable compaction of pixel indices by label, order
  * bit-identical to torch.nonzero(labels == k) for every k.  counts [K] int64,

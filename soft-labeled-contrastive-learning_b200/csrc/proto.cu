@@ -40,6 +40,9 @@ constexpr int kThreads = SLCL_PROTO_THREADS;
 #ifndef SLCL_BWD_MINBLK
 #define SLCL_BWD_MINBLK 3
 #endif
+#ifndef SLCL_MPSCL_L2_BOTH
+#define SLCL_MPSCL_L2_BOTH 0      // 1: the MPSCL step keeps both maps in L2 when only each one alone fits (slower, DESIGN §3)
+#endif
 constexpr int kUnroll = SLCL_FWD_UNROLL;      // channel planes in flight per thread (8 x 16 B)
 constexpr int kUnrollBwd = SLCL_BWD_UNROLL;
 
@@ -114,10 +117,10 @@ __device__ __forceinline__ void centre_row(const float* sC, int c, float (&ck)[K
   for (int k = 0; k < K; ++k) ck[k] = tmp[k];
 }
 
-// Pixel-group addressing shared by every kernel in this file.
+// Pixel-group addressing shared by every kernel in this file: `bid` is the block's index within its map (the
+// two-map kernels of the MPSCL step run one map per segment of their grid).
 template <int VEC>
-__device__ __forceinline__ bool locate(const ProtoArgs& a, int64_t& pix, int64_t& offset) {
-  const int64_t bid = a.reverse ? (int64_t)(gridDim.x - 1 - blockIdx.x) : (int64_t)blockIdx.x;
+__device__ __forceinline__ bool locate_at(const ProtoArgs& a, int64_t bid, int64_t& pix, int64_t& offset) {
   int64_t g = bid * blockDim.x + threadIdx.x;
   int64_t groups_per_image = a.pixels / VEC;
   if (g >= a.batch * groups_per_image) { pix = 0; offset = 0; return false; }
@@ -127,6 +130,29 @@ __device__ __forceinline__ bool locate(const ProtoArgs& a, int64_t& pix, int64_t
   offset = b * a.sb + p * a.sp;
   return true;
 }
+template <int VEC>
+__device__ __forceinline__ bool locate(const ProtoArgs& a, int64_t& pix, int64_t& offset) {
+  const int64_t bid = a.reverse ? (int64_t)(gridDim.x - 1 - blockIdx.x) : (int64_t)blockIdx.x;
+  return locate_at<VEC>(a, bid, pix, offset);
+}
+
+// Which block of its map this block is, evaluated where the kernel needs it.  WholeGrid: the grid is the map
+// (walked back to front with a.reverse); Segment: blocks [first, first + n) of the grid are the map.
+struct WholeGrid {
+  __device__ __forceinline__ int64_t bid(const ProtoArgs& a) const {
+    return a.reverse ? (int64_t)(gridDim.x - 1 - blockIdx.x) : (int64_t)blockIdx.x;
+  }
+  __device__ __forceinline__ unsigned int slot(const ProtoArgs& a) const {
+    return a.reverse ? gridDim.x - 1 - blockIdx.x : blockIdx.x;
+  }
+};
+struct Segment {
+  unsigned int first, n;
+  __device__ __forceinline__ unsigned int slot(const ProtoArgs& a) const {
+    return a.reverse ? first + n - 1 - blockIdx.x : blockIdx.x - first;
+  }
+  __device__ __forceinline__ int64_t bid(const ProtoArgs& a) const { return (int64_t)slot(a); }
+};
 
 // Accumulate squared norm and K dot products over all channels.
 template <int K, int VEC>
@@ -172,18 +198,13 @@ __device__ __forceinline__ void channel_pass(const float* base, int64_t sc, int 
 // ---------------------------------------------------------------------------
 // forward: loss rows + stash
 // ---------------------------------------------------------------------------
-template <int K, int VEC>
-__global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_FWD_MINBLK : 1) proto_fwd_kernel(const ProtoArgs a) {
-  pdl_trigger();
-  pdl_wait();
-  extern __shared__ __align__(16) float sC[];
-  __shared__ double red[2][kThreads / 32];
-  const int C = (int)a.channels;
-  load_centres_smem<K>(sC, a.cstate, C);
-  __syncthreads();
-
+// One block's pixels of one map (the centres already in sC): loss rows, stash, and the block's partial, indexed by its
+// pixel range.
+template <int K, int VEC, class Blk>
+__device__ __forceinline__ void proto_fwd_block(const ProtoArgs& a, const float* sC, double (*red)[kThreads / 32], int C,
+                                                Blk blk) {
   int64_t pix, off;
-  const bool active = locate<VEC>(a, pix, off);
+  const bool active = locate_at<VEC>(a, blk.bid(a), pix, off);
   double loss_acc = 0.0, sel_acc = 0.0;
   if (active) {
     float nrm[VEC], dot[K][VEC];
@@ -256,7 +277,7 @@ __global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_FWD_MINB
 #pragma unroll
       for (int k = 0; k < K; ++k) {
         cosv[k] = dot[k][v] * inv_n;
-        if (a.labels != nullptr || a.fused_target) M[k] = (lab[v] == (long long)k) ? 1.0f : 0.0f;      // :513
+        if (!(a.labels == nullptr && !a.fused_target)) M[k] = (lab[v] == (long long)k) ? 1.0f : 0.0f;   // :513
         else M[k] = msoft[v * K + k];                                                  // :517
       }
       float row = margin_row<K>(cosv, M, selv[v], inv_n, a.mc, coef);
@@ -278,8 +299,44 @@ __global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_FWD_MINB
     double l = 0.0, s = 0.0;
 #pragma unroll
     for (int w = 0; w < kThreads / 32; ++w) { l += red[0][w]; s += red[1][w]; }
-    a.partial[a.reverse ? gridDim.x - 1 - blockIdx.x : blockIdx.x] = make_double2(l, s);      // indexed by pixel range
+    a.partial[blk.slot(a)] = make_double2(l, s);      // indexed by pixel range
   }
+}
+
+template <int K, int VEC>
+__global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_FWD_MINBLK : 1) proto_fwd_kernel(const ProtoArgs a) {
+  pdl_trigger();
+  pdl_wait();
+  extern __shared__ __align__(16) float sC[];
+  __shared__ double red[2][kThreads / 32];
+  const int C = (int)a.channels;
+  load_centres_smem<K>(sC, a.cstate, C);
+  __syncthreads();
+  proto_fwd_block<K, VEC>(a, sC, red, C, WholeGrid{});
+}
+
+// Blocks per SM of the two-map kernels: the single-map kernels' 3 where both bodies fit the 80 registers that leaves
+// without spilling (ptxas -v), else 2.
+constexpr int mpscl_fwd_minblk(int K, int VEC) { return VEC == 4 && K <= 5 ? ((K == 2 || K == 4) ? SLCL_FWD_MINBLK : 2) : 1; }
+constexpr int mpscl_bwd_minblk(int K, int VEC) { return VEC == 4 && K <= 5 ? (K == 4 ? 2 : SLCL_BWD_MINBLK) : 1; }
+
+// The MPSCL step's prototype forward over BOTH maps in one launch: blocks [0, nb_s) run the source map `s` (hard labels,
+// source margin constants), blocks [nb_s, nb_s + nb_t) the fused target map `t` (pseudo label and mask written out,
+// target constants).  Each map keeps the block decomposition, partial indexing and walk direction proto_fwd_kernel gives
+// it, so each map's sums are the single-map launch's.  Both maps share the centres (one cstate).
+
+template <int K, int VEC>
+__global__ void __launch_bounds__(kThreads, mpscl_fwd_minblk(K, VEC))
+    mpscl_fwd_kernel(const ProtoArgs s, const ProtoArgs t, int nb_s, int nb_t) {
+  pdl_trigger();
+  pdl_wait();
+  extern __shared__ __align__(16) float sC[];
+  __shared__ double red[2][kThreads / 32];
+  const int C = (int)s.channels;
+  load_centres_smem<K>(sC, s.cstate, C);
+  __syncthreads();
+  if (blockIdx.x < (unsigned int)nb_s) proto_fwd_block<K, VEC>(s, sC, red, C, Segment{0u, (unsigned int)nb_s});
+  else proto_fwd_block<K, VEC>(t, sC, red, C, Segment{(unsigned int)nb_s, (unsigned int)nb_t});
 }
 
 // Sums the block partials in index order (deterministic) and writes
@@ -289,15 +346,10 @@ __global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_FWD_MINB
 // same rank order -- so the forward needs no extra launch (and no collective) to return the GLOBAL loss.
 // split != 0: SEND only -- scal[2..3] keep the LOCAL pair, the epoch goes to mailbox word 4, and proto_bwd_kernel
 // (launched with the same mailboxes) receives, adds and publishes: the exchange latency hides behind its launch + prologue.
-__global__ void __launch_bounds__(kThreads) proto_finalize_kernel(const double2* partial, int n_blocks, int64_t n_total,
-                                                                   int has_sel, float* scal, const PeerCtx pc, int split) {
-  pdl_trigger();
-  pdl_wait();
-  __shared__ double red[2][kThreads / 32];
-  __shared__ float s_pair[2];
-  __shared__ float s_vals[2 * kMaxPeers];
-  __shared__ int s_bad;
-  double l = 0.0, s = 0.0;
+// The block partials of one map summed in index order (deterministic); the totals are valid on thread 0.
+__device__ __forceinline__ void sum_partials(const double2* partial, int n_blocks, double (*red)[kThreads / 32], double& l,
+                                             double& s) {
+  l = 0.0; s = 0.0;
   for (int i = threadIdx.x; i < n_blocks; i += kThreads) { double2 p = partial[i]; l += p.x; s += p.y; }
   l = warp_sum(l); s = warp_sum(s);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -306,6 +358,30 @@ __global__ void __launch_bounds__(kThreads) proto_finalize_kernel(const double2*
   if (threadIdx.x == 0) {
     l = 0.0; s = 0.0;
     for (int w = 0; w < kThreads / 32; ++w) { l += red[0][w]; s += red[1][w]; }
+  }
+}
+
+// scal = {loss, coefficient, weight sum, weighted row-loss sum} from the (global) pair.
+__device__ __forceinline__ void write_scal(float* scal, int has_sel, float wsum, float lsum) {
+  // with pixel_sel_loc: sum / (sum(sel) + 1e-4) (:565); else mean over N (:571)
+  const float coef = has_sel ? 1.0f / (wsum + 1e-4f) : 1.0f / wsum;
+  scal[0] = lsum * coef;
+  scal[1] = coef;
+  scal[2] = wsum;
+  scal[3] = lsum;
+}
+
+__global__ void __launch_bounds__(kThreads) proto_finalize_kernel(const double2* partial, int n_blocks, int64_t n_total,
+                                                                   int has_sel, float* scal, const PeerCtx pc, int split) {
+  pdl_trigger();
+  pdl_wait();
+  __shared__ double red[2][kThreads / 32];
+  __shared__ float s_pair[2];
+  __shared__ float s_vals[2 * kMaxPeers];
+  __shared__ int s_bad;
+  double l, s;
+  sum_partials(partial, n_blocks, red, l, s);
+  if (threadIdx.x == 0) {
     s_pair[0] = has_sel ? (float)s : (float)n_total;
     s_pair[1] = (float)l;
     s_bad = 0;
@@ -334,13 +410,66 @@ __global__ void __launch_bounds__(kThreads) proto_finalize_kernel(const double2*
       peer_epoch_end(pc, e, 1u);
     }
   }
+  if (threadIdx.x == 0) write_scal(scal, has_sel, wsum, lsum);
+}
+
+// The MPSCL step's finaliser: both maps' partials summed as proto_finalize_kernel sums them, then ONE exchange of both
+// pairs (thread 4p+v sends word v of {source weight sum, source row-loss sum, target weight sum, target row-loss sum}
+// to rank p), added in rank order as proto_finalize_kernel adds them.  The source has no pixel selection (its weight sum
+// is its pixel count), the target is weighted by its mask.  pairs != null (the NCCL route): the LOCAL quadruple goes
+// there for the caller's all-reduce and mpscl_finish_kernel, and scal is left alone.
+__global__ void __launch_bounds__(kThreads) mpscl_finalize_kernel(const double2* part_s, int nb_s, int64_t n_s,
+                                                                   const double2* part_t, int nb_t, float* scal_s,
+                                                                   float* scal_t, float* pairs, const PeerCtx pc) {
+  pdl_trigger();
+  pdl_wait();
+  __shared__ double red_s[2][kThreads / 32], red_t[2][kThreads / 32];
+  __shared__ float s_q[4];
+  __shared__ float s_vals[4 * kMaxPeers];
+  __shared__ int s_bad;
+  double l, s;
+  sum_partials(part_s, nb_s, red_s, l, s);
+  if (threadIdx.x == 0) { s_q[0] = (float)n_s; s_q[1] = (float)l; }
+  sum_partials(part_t, nb_t, red_t, l, s);
+  if (threadIdx.x == 0) { s_q[2] = (float)s; s_q[3] = (float)l; s_bad = 0; }
+  __syncthreads();
+  float q[4] = {s_q[0], s_q[1], s_q[2], s_q[3]};
+  if (pc.world > 1) {
+    const unsigned int e = peer_epoch_begin(pc);
+    const int t = threadIdx.x;
+    if (t < 4 * pc.world) {
+      bool ok;
+      const unsigned int got = peer_send_recv(pc, e, t >> 2, t & 3, __float_as_uint(s_q[t & 3]), ok);
+      s_vals[t] = __uint_as_float(got);
+      if (!ok) s_bad = 1;
+    }
+    __syncthreads();
+    if (t == 0) {
+      for (int v = 0; v < 4; ++v) q[v] = 0.f;
+      for (int r = 0; r < pc.world; ++r)
+        for (int v = 0; v < 4; ++v) q[v] += s_vals[4 * r + v];
+      if (s_bad)       // a peer never arrived: poison, do not hang
+        for (int v = 0; v < 4; ++v) q[v] = __uint_as_float(0x7FC00000u);
+      peer_epoch_end(pc, e, 1u);
+    }
+  }
   if (threadIdx.x == 0) {
-    // with pixel_sel_loc: sum / (sum(sel) + 1e-4) (:565); else mean over N (:571)
-    const float coef = has_sel ? 1.0f / (wsum + 1e-4f) : 1.0f / wsum;
-    scal[0] = lsum * coef;
-    scal[1] = coef;
-    scal[2] = wsum;
-    scal[3] = lsum;
+    if (pairs != nullptr) {
+      for (int v = 0; v < 4; ++v) pairs[v] = q[v];
+    } else {
+      write_scal(scal_s, 0, q[0], q[1]);
+      write_scal(scal_t, 1, q[2], q[3]);
+    }
+  }
+}
+
+// NCCL route: after the caller's all-reduce of the four pair words, the two global quadruples.
+__global__ void mpscl_finish_kernel(const float* pairs, float* scal_s, float* scal_t) {
+  pdl_trigger();
+  pdl_wait();
+  if (threadIdx.x == 0 && blockIdx.x == 0) {
+    write_scal(scal_s, 0, pairs[0], pairs[1]);
+    write_scal(scal_t, 1, pairs[2], pairs[3]);
   }
 }
 
@@ -404,50 +533,14 @@ __global__ void __launch_bounds__(256) peer_allreduce_f64_kernel(double* buf, lo
 // ---------------------------------------------------------------------------
 // backward: dF = gamma * ( sum_k a_k chat_k - b x )
 // ---------------------------------------------------------------------------
-template <int K, int VEC>
-__global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_BWD_MINBLK : 1) proto_bwd_kernel(const ProtoArgs a, float* scal, const float* grad_out,
-                                                             float* dfeat, const PeerCtx pc, int has_sel) {
-  pdl_trigger();
-  pdl_wait();
-  extern __shared__ __align__(16) float sC[];
-  __shared__ float s_coef;
-  __shared__ float s_vals[2 * kMaxPeers];
-  const int C = (int)a.channels;
-  load_centres_smem<K>(sC, a.cstate, C);
-  if (pc.world > 1) {
-    // second half of a split-phase exchange (proto_finalize_kernel sent this rank's pair and left the epoch in word 4):
-    // block 0 receives every rank's pair, adds in rank order, rewrites scal and publishes the epoch in word 3; the other
-    // blocks wait for that word.  By now the wire latency has been overlapped with this kernel's launch and prologue.
-    unsigned long long* mine = pc.boxes[pc.rank];
-    const unsigned int e = (unsigned int)(*reinterpret_cast<volatile unsigned long long*>(mine + 4));
-    const int t = threadIdx.x;
-    if (blockIdx.x == 0) {
-      bool ok = true;
-      if (t < 2 * pc.world) s_vals[t] = __uint_as_float(peer_recv(pc, e, t >> 1, t & 1, ok));
-      const int bad = __syncthreads_or(!ok);
-      if (t == 0) {
-        float wsum = 0.f, lsum = 0.f;
-        for (int r = 0; r < pc.world; ++r) { wsum += s_vals[2 * r]; lsum += s_vals[2 * r + 1]; }
-        if (bad) { wsum = __uint_as_float(0x7FC00000u); lsum = wsum; }
-        const float coef = has_sel ? 1.0f / (wsum + 1e-4f) : 1.0f / wsum;
-        scal[0] = lsum * coef; scal[1] = coef; scal[2] = wsum; scal[3] = lsum;
-        s_coef = coef;
-        __threadfence();
-        *reinterpret_cast<volatile unsigned long long*>(mine + 3) = (unsigned long long)e;       // ready
-        peer_epoch_end(pc, e, 1u);
-      }
-    } else if (t == 0) {
-      while ((unsigned int)(*reinterpret_cast<volatile unsigned long long*>(mine + 3)) != e) { }
-      __threadfence();
-      s_coef = *reinterpret_cast<volatile float*>(scal + 1);
-    }
-  } else if (threadIdx.x == 0) {
-    s_coef = scal[1];
-  }
-  __syncthreads();
+// One block's pixels of one map (block `bid` of that map; the centres already in sC), a_k and b from the stash.
+// gamma = grad_out[0] * (*coef), coef in shared memory.
+template <int K, int VEC, class Blk>
+__device__ __forceinline__ void proto_bwd_block(const ProtoArgs& a, const float* sC, int C, Blk blk, const float* grad_out,
+                                                const float* coef_, float* dfeat) {
   int64_t pix, off;
-  if (!locate<VEC>(a, pix, off)) return;
-  const float gamma = grad_out[0] * s_coef;
+  if (!locate_at<VEC>(a, blk.bid(a), pix, off)) return;
+  const float gamma = grad_out[0] * *coef_;
   float coef[K + 1][VEC];
 #pragma unroll
   for (int k = 0; k <= K; ++k) {
@@ -490,6 +583,70 @@ __global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_BWD_MINB
     }
     Vec<VEC>::store(dst + (int64_t)c * a.sc, o);
   }
+}
+
+template <int K, int VEC>
+__global__ void __launch_bounds__(kThreads, (K <= 5 && VEC == 4) ? SLCL_BWD_MINBLK : 1) proto_bwd_kernel(const ProtoArgs a, float* scal, const float* grad_out,
+                                                             float* dfeat, const PeerCtx pc, int has_sel) {
+  pdl_trigger();
+  pdl_wait();
+  extern __shared__ __align__(16) float sC[];
+  __shared__ float s_coef;
+  __shared__ float s_vals[2 * kMaxPeers];
+  const int C = (int)a.channels;
+  load_centres_smem<K>(sC, a.cstate, C);
+  if (pc.world > 1) {
+    // second half of a split-phase exchange (proto_finalize_kernel sent this rank's pair and left the epoch in word 4):
+    // block 0 receives every rank's pair, adds in rank order, rewrites scal and publishes the epoch in word 3; the other
+    // blocks wait for that word.  By now the wire latency has been overlapped with this kernel's launch and prologue.
+    unsigned long long* mine = pc.boxes[pc.rank];
+    const unsigned int e = (unsigned int)(*reinterpret_cast<volatile unsigned long long*>(mine + 4));
+    const int t = threadIdx.x;
+    if (blockIdx.x == 0) {
+      bool ok = true;
+      if (t < 2 * pc.world) s_vals[t] = __uint_as_float(peer_recv(pc, e, t >> 1, t & 1, ok));
+      const int bad = __syncthreads_or(!ok);
+      if (t == 0) {
+        float wsum = 0.f, lsum = 0.f;
+        for (int r = 0; r < pc.world; ++r) { wsum += s_vals[2 * r]; lsum += s_vals[2 * r + 1]; }
+        if (bad) { wsum = __uint_as_float(0x7FC00000u); lsum = wsum; }
+        const float coef = has_sel ? 1.0f / (wsum + 1e-4f) : 1.0f / wsum;
+        scal[0] = lsum * coef; scal[1] = coef; scal[2] = wsum; scal[3] = lsum;
+        s_coef = coef;
+        __threadfence();
+        *reinterpret_cast<volatile unsigned long long*>(mine + 3) = (unsigned long long)e;       // ready
+        peer_epoch_end(pc, e, 1u);
+      }
+    } else if (t == 0) {
+      while ((unsigned int)(*reinterpret_cast<volatile unsigned long long*>(mine + 3)) != e) { }
+      __threadfence();
+      s_coef = *reinterpret_cast<volatile float*>(scal + 1);
+    }
+  } else if (threadIdx.x == 0) {
+    s_coef = scal[1];
+  }
+  __syncthreads();
+  proto_bwd_block<K, VEC>(a, sC, C, WholeGrid{}, grad_out, &s_coef, dfeat);
+}
+
+// The MPSCL step's backward over both maps in one launch: blocks [0, nb_s) write dF_s from the source stash and scal_s,
+// blocks [nb_s, nb_s + nb_t) dF_t from the target's; both maps share the centres.  A map whose loss got no gradient is
+// launched with no blocks.
+template <int K, int VEC>
+__global__ void __launch_bounds__(kThreads, mpscl_bwd_minblk(K, VEC))
+    mpscl_bwd_kernel(const ProtoArgs s, const ProtoArgs t, int nb_s, int nb_t, const float* scal_s, const float* scal_t,
+                     const float* grad_s, const float* grad_t, float* dfeat_s, float* dfeat_t) {
+  pdl_trigger();
+  pdl_wait();
+  extern __shared__ __align__(16) float sC[];
+  __shared__ float s_coef;
+  const int C = (int)s.channels;
+  load_centres_smem<K>(sC, s.cstate, C);
+  const bool src = blockIdx.x < (unsigned int)nb_s;
+  if (threadIdx.x == 0) s_coef = src ? scal_s[1] : scal_t[1];
+  __syncthreads();
+  if (src) proto_bwd_block<K, VEC>(s, sC, C, Segment{0u, (unsigned int)nb_s}, grad_s, &s_coef, dfeat_s);
+  else proto_bwd_block<K, VEC>(t, sC, C, Segment{(unsigned int)nb_s, (unsigned int)nb_t}, grad_t, &s_coef, dfeat_t);
 }
 
 // ---------------------------------------------------------------------------
@@ -907,4 +1064,205 @@ extern "C" int slcl_proto_bwd_centres(const float* feat, const slcl_map_t* map, 
   centre_grad_kernel<<<K, kThreads, 0, stream>>>(sums, cstate, scal, grad_out, (int)map->channels, K,
                                                   params->normalize, dcentres);
   return check_launch("slcl_proto_bwd_centres");
+}
+
+// ---------------------------------------------------------------------------
+// The MPSCL loss section (trainer/Trainer_MPSCL.py:133-147) in one forward and one backward call:
+//   centres = update_class_center_iter(F_s, labels_s, old, m)          class-sum sweep + reduce/exchange/EMA (class_sums.cu)
+//   hard, mask = generate_pseudo_label(F_t, centres, th)                \  prep_centres_kernel, then mpscl_fwd_kernel over
+//   loss_s = mpcl_loss_calc(F_s, labels_s, centres, mpcl_src)           |  both maps and mpscl_finalize_kernel (one
+//   loss_t = mpcl_loss_calc(F_t, hard, centres, mpcl_trg, mask)        /   exchange of both loss pairs)
+// Workspace: [class sums K x (C+1) fp64 | source block partials | target block partials | class-sum sweep workspace].
+// ---------------------------------------------------------------------------
+namespace slcl {
+namespace {
+
+struct MpsclWs {
+  double* sums;
+  double2* part_s;
+  double2* part_t;
+  void* cs;
+  size_t cs_bytes;
+};
+
+bool dense_nchw(const slcl_map_t* m) {
+  return validate_map(m) && m->stride_p == 1 && m->stride_c == m->pixels && m->stride_b == m->channels * m->pixels;
+}
+
+size_t mpscl_cs_bytes(const slcl_map_t* s, int K) { return class_sums_ws_bytes(s->batch, s->channels, s->pixels, K); }
+
+size_t mpscl_ws_layout(const slcl_map_t* s, const slcl_map_t* t, int K, void* base, MpsclWs* ws) {
+  const size_t sums = align_up((size_t)K * (s->channels + 1) * sizeof(double), 256);
+  const size_t ps = align_up(slcl_proto_workspace_bytes(s->batch * s->pixels), 256);
+  const size_t pt = align_up(slcl_proto_workspace_bytes(t->batch * t->pixels), 256);
+  const size_t cs = mpscl_cs_bytes(s, K);
+  if (ws != nullptr) {
+    char* b = reinterpret_cast<char*>(base);
+    ws->sums = reinterpret_cast<double*>(b);
+    ws->part_s = reinterpret_cast<double2*>(b + sums);
+    ws->part_t = reinterpret_cast<double2*>(b + sums + ps);
+    ws->cs = b + sums + ps + pt;
+    ws->cs_bytes = cs;
+  }
+  return sums + ps + pt + cs;
+}
+
+// The checks every entry point makes before anything is launched.
+int mpscl_check_maps(const float* feat_s, const slcl_map_t* map_s, const float* feat_t, const slcl_map_t* map_t,
+                     const slcl_proto_params_t* ps, const slcl_proto_params_t* pt) {
+  if (!feat_s || !feat_t || !ps || !pt || !dense_nchw(map_s) || !dense_nchw(map_t)) return SLCL_ERR_INVALID_ARGUMENT;
+  if (map_s->channels != map_t->channels || map_s->pixels != map_t->pixels) return SLCL_ERR_INVALID_ARGUMENT;
+  const int K = ps->n_class;
+  if (K < 2 || K > kMaxK || pt->n_class != K) return SLCL_ERR_INVALID_ARGUMENT;
+  return SLCL_OK;
+}
+
+int mpscl_check_params(const slcl_proto_params_t* p) {
+  return (p->temperature > 0.f && p->base_temperature > 0.f && p->normalize) ? SLCL_OK : SLCL_ERR_INVALID_ARGUMENT;
+}
+
+// Prototype forward of both maps (mpscl_fwd_kernel; one launch per map when their load widths differ) and the finaliser.
+int mpscl_proto_fwd(const float* feat_s, const slcl_map_t* map_s, const int64_t* labels_s, const float* feat_t,
+                    const slcl_map_t* map_t, const float* centres, const slcl_proto_params_t* ps,
+                    const slcl_proto_params_t* pt, float sel_threshold, float* cstate, float* stash_s, float* stash_t,
+                    int64_t* label_t, float* sel_t, float* scal_s, float* scal_t, float* pairs, const slcl_peer_t* peer,
+                    const MpsclWs& ws, cudaStream_t stream) {
+  const int K = ps->n_class;
+  const int C = (int)map_s->channels;
+  // the plans, walk directions and L2 policies of the single-map calls (slcl_proto_fwd, slcl_proto_fwd_target)
+  const Plan plan_s = make_plan(map_s, K, {feat_s, labels_s, nullptr, stash_s, nullptr});
+  const Plan plan_t = make_plan(map_t, K, {feat_t, label_t, sel_t, stash_t});
+  ProtoArgs s = base_args(feat_s, map_s, cstate);
+  s.labels = labels_s; s.stash = stash_s; s.partial = ws.part_s; s.mc = make_const(ps);
+  s.reverse = s.keep_l2;
+  ProtoArgs t = base_args(feat_t, map_t, cstate);
+  t.stash = stash_t; t.partial = ws.part_t; t.mc = make_const(pt);
+  t.fused_target = 1; t.sel_threshold = sel_threshold; t.out_label = label_t; t.out_sel = sel_t;
+  // Both maps together larger than L2 (the cfg4 8-GPU shard: 2 x 98 MiB): only the source map, which the backward reads
+  // first, is loaded with evict_last -- measured faster than keeping both (DESIGN §3); building with
+  // -DSLCL_MPSCL_L2_BOTH=1 keeps the single-map policy for both maps instead.
+  const size_t bytes_s = (size_t)s.n_total * C * sizeof(float), bytes_t = (size_t)t.n_total * C * sizeof(float);
+  if (!SLCL_MPSCL_L2_BOTH && s.keep_l2 && t.keep_l2 && bytes_s + bytes_t > kL2KeepBytes) t.keep_l2 = 0;
+  t.reverse = 0;             // the target segment follows the source segment's last block (the start of F_s)
+  launch_pdl(prep_centres_kernel, dim3(K), dim3(kThreads), 0, stream, centres, C, K, 1, cstate);
+  SLCL_DISPATCH_K(K, plan_s.vec, {
+    int st = ensure_smem(mpscl_fwd_kernel<KK, VV>, plan_s.smem);
+    if (st != SLCL_OK) return st;
+    if (plan_t.vec == VV) {
+      launch_pdl(mpscl_fwd_kernel<KK, VV>, dim3(plan_s.n_blocks + plan_t.n_blocks), dim3(kThreads), plan_s.smem, stream, s, t,
+                 plan_s.n_blocks, plan_t.n_blocks);
+    } else {
+      launch_pdl(mpscl_fwd_kernel<KK, VV>, dim3(plan_s.n_blocks), dim3(kThreads), plan_s.smem, stream, s, t, plan_s.n_blocks, 0);
+      constexpr int VT = VV == 4 ? 1 : 4;
+      st = ensure_smem(mpscl_fwd_kernel<KK, VT>, plan_t.smem);
+      if (st != SLCL_OK) return st;
+      launch_pdl(mpscl_fwd_kernel<KK, VT>, dim3(plan_t.n_blocks), dim3(kThreads), plan_t.smem, stream, s, t, 0, plan_t.n_blocks);
+    }
+  })
+  launch_pdl(mpscl_finalize_kernel, dim3(1), dim3(kThreads), 0, stream, (const double2*)ws.part_s, plan_s.n_blocks,
+             plan_s.n_total, (const double2*)ws.part_t, plan_t.n_blocks, scal_s, scal_t, pairs, peer_ctx(peer));
+  return SLCL_OK;
+}
+
+}  // namespace
+}  // namespace slcl
+
+extern "C" size_t slcl_mpscl_step_workspace_bytes(const slcl_map_t* map_s, const slcl_map_t* map_t, int n_class) {
+  if (!validate_map(map_s) || !validate_map(map_t) || n_class < 2 || n_class > kMaxK) return 0;
+  return mpscl_ws_layout(map_s, map_t, n_class, nullptr, nullptr);
+}
+
+extern "C" int slcl_mpscl_step_fwd(const float* feat_s, const slcl_map_t* map_s, const int64_t* labels_s, const float* feat_t,
+                                   const slcl_map_t* map_t, const float* old_centres, float momentum,
+                                   const slcl_proto_params_t* params_s, const slcl_proto_params_t* params_t,
+                                   float sel_threshold, float* centres, float* cstate, float* stash_s, float* stash_t,
+                                   int64_t* label_t, float* sel_t, float* scal_s, float* scal_t, const slcl_peer_t* peer,
+                                   void* workspace, size_t workspace_bytes, slcl_stream_t stream_) {
+  int st = mpscl_check_maps(feat_s, map_s, feat_t, map_t, params_s, params_t);
+  if (st != SLCL_OK) return st;
+  if (mpscl_check_params(params_s) != SLCL_OK || mpscl_check_params(params_t) != SLCL_OK) return SLCL_ERR_INVALID_ARGUMENT;
+  if (!labels_s || !old_centres || !centres || !cstate || !stash_s || !stash_t || !label_t || !sel_t || !scal_s || !scal_t ||
+      !workspace)
+    return SLCL_ERR_INVALID_ARGUMENT;
+  const int K = params_s->n_class;
+  if (peer != nullptr && (!peer_valid(peer) || 2 * (int64_t)K * (map_s->channels + 1) > peer->capacity_words))
+    return SLCL_ERR_INVALID_ARGUMENT;
+  MpsclWs ws;
+  if (workspace_bytes < mpscl_ws_layout(map_s, map_t, K, workspace, &ws)) return SLCL_ERR_WORKSPACE;
+  if (!aligned16(workspace)) return SLCL_ERR_INVALID_ARGUMENT;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  // update_class_center_iter: the sweep and the reduce [+ exchange] + EMA kernels of slcl_class_centres_update, unchanged
+  st = slcl_class_centres_update(feat_s, map_s->batch, map_s->channels, map_s->pixels, labels_s, K, old_centres, momentum,
+                                 centres, ws.sums, peer, ws.cs, ws.cs_bytes, stream_);
+  if (st != SLCL_OK) return st;
+  st = mpscl_proto_fwd(feat_s, map_s, labels_s, feat_t, map_t, centres, params_s, params_t, sel_threshold, cstate, stash_s,
+                       stash_t, label_t, sel_t, scal_s, scal_t, nullptr, peer, ws, stream);
+  if (st != SLCL_OK) return st;
+  return check_launch("slcl_mpscl_step_fwd");
+}
+
+extern "C" int slcl_mpscl_step_fwd_local(const float* feat_s, const slcl_map_t* map_s, const int64_t* labels_s,
+                                         const float* feat_t, const slcl_map_t* map_t, const float* centres,
+                                         const slcl_proto_params_t* params_s, const slcl_proto_params_t* params_t,
+                                         float sel_threshold, float* cstate, float* stash_s, float* stash_t, int64_t* label_t,
+                                         float* sel_t, float* pairs, void* workspace, size_t workspace_bytes,
+                                         slcl_stream_t stream_) {
+  int st = mpscl_check_maps(feat_s, map_s, feat_t, map_t, params_s, params_t);
+  if (st != SLCL_OK) return st;
+  if (mpscl_check_params(params_s) != SLCL_OK || mpscl_check_params(params_t) != SLCL_OK) return SLCL_ERR_INVALID_ARGUMENT;
+  if (!labels_s || !centres || !cstate || !stash_s || !stash_t || !label_t || !sel_t || !pairs || !workspace)
+    return SLCL_ERR_INVALID_ARGUMENT;
+  MpsclWs ws;
+  if (workspace_bytes < mpscl_ws_layout(map_s, map_t, params_s->n_class, workspace, &ws)) return SLCL_ERR_WORKSPACE;
+  if (!aligned16(workspace)) return SLCL_ERR_INVALID_ARGUMENT;
+  st = mpscl_proto_fwd(feat_s, map_s, labels_s, feat_t, map_t, centres, params_s, params_t, sel_threshold, cstate, stash_s,
+                       stash_t, label_t, sel_t, nullptr, nullptr, pairs, nullptr, ws, (cudaStream_t)stream_);
+  if (st != SLCL_OK) return st;
+  return check_launch("slcl_mpscl_step_fwd_local");
+}
+
+extern "C" int slcl_mpscl_step_finish(const float* pairs, float* scal_s, float* scal_t, slcl_stream_t stream_) {
+  if (!pairs || !scal_s || !scal_t) return SLCL_ERR_INVALID_ARGUMENT;
+  launch_pdl(mpscl_finish_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream_, pairs, scal_s, scal_t);
+  return check_launch("slcl_mpscl_step_finish");
+}
+
+extern "C" int slcl_mpscl_step_bwd(const float* feat_s, const slcl_map_t* map_s, const float* feat_t, const slcl_map_t* map_t,
+                                   const float* stash_s, const float* stash_t, const float* cstate, const float* scal_s,
+                                   const float* scal_t, const float* grad_s, const float* grad_t,
+                                   const slcl_proto_params_t* params_s, const slcl_proto_params_t* params_t, float* dfeat_s,
+                                   float* dfeat_t, slcl_stream_t stream_) {
+  int st = mpscl_check_maps(feat_s, map_s, feat_t, map_t, params_s, params_t);
+  if (st != SLCL_OK) return st;
+  if (!cstate || (!grad_s && !grad_t)) return SLCL_ERR_INVALID_ARGUMENT;
+  if (grad_s && (!stash_s || !scal_s || !dfeat_s)) return SLCL_ERR_INVALID_ARGUMENT;
+  if (grad_t && (!stash_t || !scal_t || !dfeat_t)) return SLCL_ERR_INVALID_ARGUMENT;
+  const int K = params_s->n_class;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  // the plans of slcl_proto_bwd for each map; a map without an upstream gradient gets no blocks
+  const Plan plan_s = make_plan(map_s, K, {feat_s, stash_s, dfeat_s});
+  const Plan plan_t = make_plan(map_t, K, {feat_t, stash_t, dfeat_t});
+  const int nb_s = grad_s ? plan_s.n_blocks : 0, nb_t = grad_t ? plan_t.n_blocks : 0;
+  ProtoArgs s = base_args(feat_s, map_s, cstate);
+  s.stash = const_cast<float*>(stash_s);
+  ProtoArgs t = base_args(feat_t, map_t, cstate);
+  t.stash = const_cast<float*>(stash_t);
+  s.reverse = t.reverse = 0;
+  SLCL_DISPATCH_K(K, (nb_s ? plan_s.vec : plan_t.vec), {
+    st = ensure_smem(mpscl_bwd_kernel<KK, VV>, plan_s.smem);
+    if (st != SLCL_OK) return st;
+    if (nb_s == 0 || nb_t == 0 || plan_t.vec == plan_s.vec) {
+      launch_pdl(mpscl_bwd_kernel<KK, VV>, dim3(nb_s + nb_t), dim3(kThreads), plan_s.smem, stream, s, t, nb_s, nb_t, scal_s,
+                 scal_t, grad_s, grad_t, dfeat_s, dfeat_t);
+    } else {
+      launch_pdl(mpscl_bwd_kernel<KK, VV>, dim3(nb_s), dim3(kThreads), plan_s.smem, stream, s, t, nb_s, 0, scal_s, scal_t,
+                 grad_s, grad_t, dfeat_s, dfeat_t);
+      constexpr int VT = VV == 4 ? 1 : 4;
+      st = ensure_smem(mpscl_bwd_kernel<KK, VT>, plan_t.smem);
+      if (st != SLCL_OK) return st;
+      launch_pdl(mpscl_bwd_kernel<KK, VT>, dim3(nb_t), dim3(kThreads), plan_t.smem, stream, s, t, 0, nb_t, scal_s, scal_t,
+                 grad_s, grad_t, dfeat_s, dfeat_t);
+    }
+  })
+  return check_launch("slcl_mpscl_step_bwd");
 }

@@ -100,6 +100,16 @@ SIGNATURES = {
                                         C.c_float, C.c_float, C.c_float, _P, _P, _P, _P, _SZ, _P]),
     "slcl_mccl_step_bwd": (C.c_int, [_P, _P, _P, _I64, _P, _P, _I64, _I64, _I64, C.c_int, C.c_int, C.c_int, C.c_float, _P, _P,
                                      _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    # the MPSCL loss section in one call (trainer/Trainer_MPSCL.py:133-147)
+    "slcl_mpscl_step_workspace_bytes": (_SZ, [C.POINTER(MapT), C.POINTER(MapT), C.c_int]),
+    "slcl_mpscl_step_fwd": (C.c_int, [_P, C.POINTER(MapT), _P, _P, C.POINTER(MapT), _P, C.c_float, C.POINTER(ProtoParamsT),
+                                      C.POINTER(ProtoParamsT), C.c_float, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(PeerT),
+                                      _P, _SZ, _P]),
+    "slcl_mpscl_step_fwd_local": (C.c_int, [_P, C.POINTER(MapT), _P, _P, C.POINTER(MapT), _P, C.POINTER(ProtoParamsT),
+                                            C.POINTER(ProtoParamsT), C.c_float, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "slcl_mpscl_step_finish": (C.c_int, [_P, _P, _P, _P]),
+    "slcl_mpscl_step_bwd": (C.c_int, [_P, C.POINTER(MapT), _P, C.POINTER(MapT), _P, _P, _P, _P, _P, _P, _P,
+                                      C.POINTER(ProtoParamsT), C.POINTER(ProtoParamsT), _P, _P, _P]),
     "slcl_compact_workspace_bytes": (_SZ, [_I64, C.c_int]),
     "slcl_compact_by_class": (C.c_int, [_P, _I64, C.c_int, _P, _P, _P, _P, _SZ, _P]),
     "slcl_sample_balanced_workspace_bytes": (_SZ, [_I64, C.c_int]),

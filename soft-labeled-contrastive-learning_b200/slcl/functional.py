@@ -330,3 +330,53 @@ def mccl_step(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, pred_t: Tensor, 
     return _McclStep.apply(feat_s, labels_s, feat_t, pred_t, part_id, feat_a, pred_a, previous_s, int(n_partitions),
                            int(n_class), bool(weighted), float(threshold), bool(from_logits), float(momentum), bool(split),
                            bool(bg), bool(norm), float(inter_w), float(intra_w), float(cnr_w), group)
+
+
+class _MpsclStep(torch.autograd.Function):
+    """The MPSCL loss section (trainer/Trainer_MPSCL.py:133-147) as one node: EMA class centres from the source map, pseudo
+    labels of the target map and both prototype losses in one forward call; dF_s and dF_t in one backward launch.  The
+    centres, pseudo labels and mask get no gradient (the trainer detaches the centres, :138 / :144)."""
+
+    @staticmethod
+    def forward(ctx, feat_s, labels_s, feat_t, old_centres, m, sel_threshold, n_class, const_s, const_t, group):
+        from .peer import PeerMailbox
+        fs, ft = feat_s.detach(), feat_t.detach()
+        if group is None or isinstance(group, PeerMailbox):
+            peer = group.args() if group is not None else ()
+            scal, centres, cstate, stash_s, stash_t, label, sel = _ops.mpscl_step_fwd(
+                fs, labels_s, ft, old_centres.detach(), m, sel_threshold, n_class, *const_s, *const_t, *peer)
+        else:       # NCCL: class sums -> all-reduce -> EMA, the local forward, one all-reduce of both pairs, the finish
+            import torch.distributed as dist
+            from .distributed import all_reduce_sums
+            sums = all_reduce_sums(_ops.class_sums(fs, labels_s, None, False, 0.0, None, 1, n_class), group)
+            centres = _ops.ema_finalize(sums, old_centres.detach(), m)
+            pairs, cstate, stash_s, stash_t, label, sel = _ops.mpscl_step_fwd_local(fs, labels_s, ft, centres, sel_threshold,
+                                                                                    n_class, *const_s, *const_t)
+            dist.all_reduce(pairs, op=dist.ReduceOp.SUM, group=None if group is True else group)
+            scal = _ops.mpscl_step_finish(pairs)
+        ctx.save_for_backward(feat_s, feat_t, stash_s, stash_t, cstate, scal)
+        ctx.n_class = n_class
+        ctx.mark_non_differentiable(centres, label, sel)
+        # only the losses carry gradients, and one of them may get none: no zero tensors for the other slots
+        ctx.set_materialize_grads(False)
+        return scal[0], scal[4], centres, label, sel
+
+    @staticmethod
+    def backward(ctx, g_s, g_t, _gc, _gl, _gm):
+        feat_s, feat_t, stash_s, stash_t, cstate, scal = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        g_s = g_s.reshape(1) if (g_s is not None and need[0]) else None
+        g_t = g_t.reshape(1) if (g_t is not None and need[2]) else None
+        if g_s is None and g_t is None:
+            return (None,) * 10
+        d_s, d_t = _ops.mpscl_step_bwd(feat_s.detach(), feat_t.detach(), stash_s, stash_t, cstate, scal, g_s, g_t,
+                                       ctx.n_class)
+        return (d_s if g_s is not None else None, None, d_t if g_t is not None else None) + (None,) * 7
+
+
+def mpscl_step(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, old_centres: Tensor, *, m: float, sel_threshold: float,
+               n_class: int, const_s: Sequence, const_t: Sequence, group=None):
+    """-> (loss_s, loss_t, centres [K, C], hard [N_t] int64, mask [N_t]).  ``const_s`` / ``const_t``: (temperature,
+    base_temperature, margin, easy_margin) of each loss."""
+    return _MpsclStep.apply(feat_s, labels_s, feat_t, old_centres, float(m), float(sel_threshold), int(n_class),
+                            tuple(const_s), tuple(const_t), group)

@@ -270,6 +270,69 @@ def mccl_step(ft_s, labels_s, ft_t, pred_t, ft_t_aug=None, pred_t_aug=None, *, n
     return total, terms, cs, ct, ct_aug
 
 
+def mpscl_step(ft_s, labels_s, ft_t, class_center_feas, mpcl_src, mpcl_trg, *, m=0.9, num_class=4, pixel_sel_th=0.25,
+               group=None):
+    """The MPSCL loss section of trainer/Trainer_MPSCL.py:133-147 as ONE forward and ONE backward call (an addition).  It is
+    defined as this composition of the drop-in calls::
+
+        centres = update_class_center_iter(ft_s, labels_s, class_center_feas, m=m, num_class=num_class, group=group)
+        hard, mask = generate_pseudo_label(ft_t, centres, pixel_sel_th)
+        loss_s = mpcl_loss_calc(ft_s, labels_s, centres.detach(), mpcl_src, tag='source', group=group)
+        loss_t = mpcl_loss_calc(ft_t, hard, centres.detach(), mpcl_trg, pixel_sel_loc=mask, tag='target', group=group)
+
+    and returns ``(loss_s, loss_t, centres, hard, mask)`` with the same values.  ``loss_s`` is differentiable w.r.t.
+    ``ft_s`` only, ``loss_t`` w.r.t. ``ft_t`` only; ``centres``, ``hard`` and ``mask`` are not differentiable.  The two
+    ``MPCL`` modules may differ in margin, temperature, base temperature and ``easy_margin``.
+
+    Five launches forward (class-sum sweep, reduce + EMA, unit centres, one prototype forward over both maps, one
+    finaliser) and one backward (both maps; only the map whose loss receives a gradient), no host synchronisation.
+    ``group``: as ``update_class_center_iter`` / ``mpcl_loss_calc`` -- two exchanges per step: the class sums, then both
+    loss pairs at once (inside the reduce kernel and the finaliser for a ``slcl.peer.PeerMailbox``; two NCCL all-reduces
+    for ``True`` / a ProcessGroup).  The backward exchanges nothing.
+
+    Raises ``ValueError``, before any launch or exchange, for maps that are not contiguous float32 ``[B, C, h, w]``,
+    channel counts or resolutions that differ between the maps (the batch sizes may differ), ``labels_s`` not at the
+    feature resolution, ``class_center_feas`` not ``[num_class, C]`` or requiring grad, an ``MPCL`` whose ``num_class``
+    is not ``num_class``, ``num_class`` outside [2, 8], or a mailbox too small for ``2 K (C+1)`` words; the separate
+    calls remain the route for those."""
+    from .seg import _resolve_group
+    from ._lib import MAX_CLASSES
+    from .peer import PeerMailbox
+    k = int(num_class)
+    if not (2 <= k <= MAX_CLASSES):
+        raise ValueError(f"mpscl_step: num_class must be in [2, {MAX_CLASSES}], got {k}")
+    for name, mod in (("mpcl_src", mpcl_src), ("mpcl_trg", mpcl_trg)):
+        if not isinstance(mod, MPCL):
+            raise TypeError(f"mpscl_step: {name} must be an slcl.loss.MPCL")
+        if mod.num_class != k:
+            raise ValueError(f"mpscl_step: {name}.num_class is {mod.num_class}, num_class is {k}")
+    for name, t in (("ft_s", ft_s), ("ft_t", ft_t)):
+        if not isinstance(t, torch.Tensor) or t.dim() != 4 or t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError(f"mpscl_step: {name} must be a contiguous float32 [B, C, h, w] map")
+    b_s, c, h, w = ft_s.shape
+    if ft_t.shape[1] != c:
+        raise ValueError(f"mpscl_step: ft_t has {ft_t.shape[1]} channels, ft_s has {c}")
+    if tuple(ft_t.shape[2:]) != (h, w):
+        raise ValueError(f"mpscl_step: ft_t is {tuple(ft_t.shape[2:])}, ft_s is {(h, w)}: the maps share one resolution")
+    if tuple(labels_s.shape[-2:]) != (h, w) or labels_s.numel() != b_s * h * w:
+        raise ValueError(f"mpscl_step: labels_s must be [B, h, w] = {(b_s, h, w)} at the feature resolution "
+                         f"(update_class_center_iter, utils/utils_.py:575-577), got {tuple(labels_s.shape)}")
+    if not isinstance(class_center_feas, torch.Tensor) or tuple(class_center_feas.shape) != (k, c):
+        raise ValueError(f"mpscl_step: class_center_feas must be [num_class, C] = {(k, c)}, "
+                         f"got {tuple(getattr(class_center_feas, 'shape', ()))}")
+    if class_center_feas.requires_grad:
+        raise ValueError("mpscl_step: class_center_feas requires grad; the step's centres are a plain tensor (the "
+                         "separate calls keep the graph through m * class_center_feas)")
+    group = _resolve_group(group)
+    if isinstance(group, PeerMailbox) and group.capacity_words < 2 * k * (c + 1):
+        raise ValueError(f"mpscl_step: the class sums are {k} x {c + 1} doubles; the mailbox needs capacity_words >= "
+                         f"{2 * k * (c + 1)}, this one has {group.capacity_words}")
+    labels = labels_s.to(ft_s.device).reshape(-1).long()
+    const = lambda mod: (float(mod.temperature), float(mod.base_temperature), float(mod.m), bool(mod.easy_margin))
+    return SF.mpscl_step(ft_s, labels, ft_t, class_center_feas, m=m, sel_threshold=pixel_sel_th, n_class=k,
+                         const_s=const(mpcl_src), const_t=const(mpcl_trg), group=group)
+
+
 SupConLoss = p2p.SupConLoss
 LocalConLoss = p2p.LocalConLoss
 BlockConLoss = p2p.BlockConLoss

@@ -846,6 +846,149 @@ def _(feat_t, pred_t, part_id, feat_a, pred_a, n_partitions, n_class, weighted, 
 # ----------------------------------------------------------------------------
 # sampler
 # ----------------------------------------------------------------------------
+# ----------------------------------------------------------------------------
+# the MPSCL loss section in one call (trainer/Trainer_MPSCL.py:133-147)
+# ----------------------------------------------------------------------------
+def _mpscl_maps(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, n_class: int):
+    feat_s, map_s = _map_nchw(_nchw_contig(feat_s))
+    feat_t, map_t = _map_nchw(_nchw_contig(feat_t))
+    labels_s = labels_s.contiguous()
+    if labels_s.dtype != torch.int64 or labels_s.numel() != map_s.batch * map_s.pixels:
+        raise ValueError("labels_s must be int64 with B_s*h*w elements")
+    return feat_s, map_s, labels_s, feat_t, map_t
+
+
+def _mpscl_outputs(map_s: MapT, map_t: MapT, n_class: int, dev):
+    n_s, n_t = map_s.batch * map_s.pixels, map_t.batch * map_t.pixels
+    return (torch.empty(n_class * map_s.channels + n_class, dtype=_F32, device=dev),
+            torch.empty((n_class + 1, n_s), dtype=_F32, device=dev), torch.empty((n_class + 1, n_t), dtype=_F32, device=dev),
+            torch.empty(n_t, dtype=torch.int64, device=dev), torch.empty(n_t, dtype=_F32, device=dev))
+
+
+@torch.library.custom_op("slcl::mpscl_step_fwd", mutates_args=(), device_types="cuda")
+def mpscl_step_fwd(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, old_centres: Tensor, m: float, sel_threshold: float,
+                   n_class: int, temperature_s: float, base_temperature_s: float, margin_s: float, easy_margin_s: bool,
+                   temperature_t: float, base_temperature_t: float, margin_t: float, easy_margin_t: bool, peer_ptrs: int = 0,
+                   rank: int = 0, world: int = 1, capacity_words: int = 0,
+                   timeout_s: float = 0.0) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """-> (scal[8] = source quadruple | target quadruple, new centres [K,C], cstate, stash_s, stash_t, label_t [N_t] int64,
+    sel_t [N_t]).  With a peer mailbox the class sums and both loss pairs are GLOBAL (two exchanges)."""
+    dev = require_cuda(feat_s, labels_s, feat_t, old_centres)
+    lib = _lib.load()
+    feat_s, map_s, labels_s, feat_t, map_t = _mpscl_maps(feat_s, labels_s, feat_t, n_class)
+    old = old_centres.to(_F32).contiguous()
+    scal = torch.empty(8, dtype=_F32, device=dev)
+    centres = torch.empty_like(old)
+    cstate, stash_s, stash_t, label_t, sel_t = _mpscl_outputs(map_s, map_t, n_class, dev)
+    ws = _ws(lib.slcl_mpscl_step_workspace_bytes(C.byref(map_s), C.byref(map_t), n_class), dev)
+    ps = _params(n_class, temperature_s, base_temperature_s, margin_s, easy_margin_s, True)
+    pt = _params(n_class, temperature_t, base_temperature_t, margin_t, easy_margin_t, True)
+    peer = _peer(peer_ptrs, rank, world, capacity_words, timeout_s)
+    with _guard(dev):
+        st = lib.slcl_mpscl_step_fwd(ptr(feat_s), C.byref(map_s), ptr(labels_s), ptr(feat_t), C.byref(map_t), ptr(old),
+                                     float(m), C.byref(ps), C.byref(pt), float(sel_threshold), ptr(centres), ptr(cstate),
+                                     ptr(stash_s), ptr(stash_t), ptr(label_t), ptr(sel_t), ptr(scal), ptr(scal) + 16,
+                                     C.byref(peer) if peer is not None else None, ptr(ws), ws.numel(), stream_ptr(dev))
+    check(st, "slcl_mpscl_step_fwd")
+    return scal, centres, cstate, stash_s, stash_t, label_t, sel_t
+
+
+@mpscl_step_fwd.register_fake
+def _(feat_s, labels_s, feat_t, old_centres, m, sel_threshold, n_class, temperature_s, base_temperature_s, margin_s,
+      easy_margin_s, temperature_t, base_temperature_t, margin_t, easy_margin_t, peer_ptrs=0, rank=0, world=1,
+      capacity_words=0, timeout_s=0.0):
+    c = feat_s.shape[1]
+    n_s, n_t = feat_s.shape[0] * feat_s.shape[2] * feat_s.shape[3], feat_t.shape[0] * feat_t.shape[2] * feat_t.shape[3]
+    return (feat_s.new_empty(8), feat_s.new_empty((n_class, c)), feat_s.new_empty(n_class * c + n_class),
+            feat_s.new_empty((n_class + 1, n_s)), feat_s.new_empty((n_class + 1, n_t)),
+            torch.empty(n_t, dtype=torch.int64, device=feat_s.device), feat_s.new_empty(n_t))
+
+
+@torch.library.custom_op("slcl::mpscl_step_fwd_local", mutates_args=(), device_types="cuda")
+def mpscl_step_fwd_local(feat_s: Tensor, labels_s: Tensor, feat_t: Tensor, centres: Tensor, sel_threshold: float,
+                         n_class: int, temperature_s: float, base_temperature_s: float, margin_s: float, easy_margin_s: bool,
+                         temperature_t: float, base_temperature_t: float, margin_t: float,
+                         easy_margin_t: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """NCCL route, from the global centres: -> (pairs[4] = this rank's {w_s, l_s, w_t, l_t}, cstate, stash_s, stash_t,
+    label_t, sel_t).  All-reduce ``pairs``, then ``mpscl_step_finish``."""
+    dev = require_cuda(feat_s, labels_s, feat_t, centres)
+    lib = _lib.load()
+    feat_s, map_s, labels_s, feat_t, map_t = _mpscl_maps(feat_s, labels_s, feat_t, n_class)
+    centres = centres.to(_F32).contiguous()
+    pairs = torch.empty(4, dtype=_F32, device=dev)
+    cstate, stash_s, stash_t, label_t, sel_t = _mpscl_outputs(map_s, map_t, n_class, dev)
+    ws = _ws(lib.slcl_mpscl_step_workspace_bytes(C.byref(map_s), C.byref(map_t), n_class), dev)
+    ps = _params(n_class, temperature_s, base_temperature_s, margin_s, easy_margin_s, True)
+    pt = _params(n_class, temperature_t, base_temperature_t, margin_t, easy_margin_t, True)
+    with _guard(dev):
+        st = lib.slcl_mpscl_step_fwd_local(ptr(feat_s), C.byref(map_s), ptr(labels_s), ptr(feat_t), C.byref(map_t),
+                                           ptr(centres), C.byref(ps), C.byref(pt), float(sel_threshold), ptr(cstate),
+                                           ptr(stash_s), ptr(stash_t), ptr(label_t), ptr(sel_t), ptr(pairs), ptr(ws),
+                                           ws.numel(), stream_ptr(dev))
+    check(st, "slcl_mpscl_step_fwd_local")
+    return pairs, cstate, stash_s, stash_t, label_t, sel_t
+
+
+@mpscl_step_fwd_local.register_fake
+def _(feat_s, labels_s, feat_t, centres, sel_threshold, n_class, temperature_s, base_temperature_s, margin_s, easy_margin_s,
+      temperature_t, base_temperature_t, margin_t, easy_margin_t):
+    c = feat_s.shape[1]
+    n_s, n_t = feat_s.shape[0] * feat_s.shape[2] * feat_s.shape[3], feat_t.shape[0] * feat_t.shape[2] * feat_t.shape[3]
+    return (feat_s.new_empty(4), feat_s.new_empty(n_class * c + n_class), feat_s.new_empty((n_class + 1, n_s)),
+            feat_s.new_empty((n_class + 1, n_t)), torch.empty(n_t, dtype=torch.int64, device=feat_s.device),
+            feat_s.new_empty(n_t))
+
+
+@torch.library.custom_op("slcl::mpscl_step_finish", mutates_args=(), device_types="cuda")
+def mpscl_step_finish(pairs: Tensor) -> Tensor:
+    """-> scal[8] (source quadruple | target quadruple) from the all-reduced pairs[4]: one launch."""
+    dev = require_cuda(pairs)
+    if pairs.dtype != _F32 or pairs.numel() != 4:
+        raise ValueError("pairs must be float32 [4]")
+    pairs = pairs.contiguous()
+    scal = torch.empty(8, dtype=_F32, device=dev)
+    with _guard(dev):
+        st = _lib.load().slcl_mpscl_step_finish(ptr(pairs), ptr(scal), ptr(scal) + 16, stream_ptr(dev))
+    check(st, "slcl_mpscl_step_finish")
+    return scal
+
+
+@mpscl_step_finish.register_fake
+def _(pairs):
+    return pairs.new_empty(8)
+
+
+@torch.library.custom_op("slcl::mpscl_step_bwd", mutates_args=(), device_types="cuda")
+def mpscl_step_bwd(feat_s: Tensor, feat_t: Tensor, stash_s: Tensor, stash_t: Tensor, cstate: Tensor, scal: Tensor,
+                   grad_s: Optional[Tensor], grad_t: Optional[Tensor], n_class: int) -> Tuple[Tensor, Tensor]:
+    """-> (dfeat_s, dfeat_t) of grad_s * loss_s + grad_t * loss_t, one launch; the map of a missing gradient comes back
+    empty (numel 0) and is not launched."""
+    dev = require_cuda(feat_s, feat_t, stash_s, stash_t, cstate, scal, grad_s, grad_t)
+    if grad_s is None and grad_t is None:
+        raise ValueError("mpscl_step_bwd needs grad_s or grad_t")
+    lib = _lib.load()
+    feat_s, map_s = _map_nchw(_nchw_contig(feat_s))
+    feat_t, map_t = _map_nchw(_nchw_contig(feat_t))
+    g_s = None if grad_s is None else grad_s.to(_F32).contiguous()
+    g_t = None if grad_t is None else grad_t.to(_F32).contiguous()
+    d_s = torch.empty_like(feat_s) if g_s is not None else feat_s.new_empty(0)
+    d_t = torch.empty_like(feat_t) if g_t is not None else feat_t.new_empty(0)
+    p = _params(n_class, 1.0, 1.0, 0.0, False, True)
+    with _guard(dev):
+        st = lib.slcl_mpscl_step_bwd(ptr(feat_s), C.byref(map_s), ptr(feat_t), C.byref(map_t), ptr(stash_s), ptr(stash_t),
+                                     ptr(cstate), ptr(scal), ptr(scal) + 16, ptr(g_s), ptr(g_t), C.byref(p), C.byref(p),
+                                     ptr(d_s) if g_s is not None else None, ptr(d_t) if g_t is not None else None,
+                                     stream_ptr(dev))
+    check(st, "slcl_mpscl_step_bwd")
+    return d_s, d_t
+
+
+@mpscl_step_bwd.register_fake
+def _(feat_s, feat_t, stash_s, stash_t, cstate, scal, grad_s, grad_t, n_class):
+    return (torch.empty_like(feat_s) if grad_s is not None else feat_s.new_empty(0),
+            torch.empty_like(feat_t) if grad_t is not None else feat_t.new_empty(0))
+
+
 @torch.library.custom_op("slcl::compact_by_class", mutates_args=(), device_types="cuda")
 def compact_by_class(labels: Tensor, n_class: int) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (counts[K], offsets[K+1], index[N]) int64; index[offsets[k]:offsets[k+1]] == nonzero(labels == k)."""
